@@ -11,6 +11,9 @@ Metric (BASELINE.json): channel-MS/s = wideband input MS/s x concurrent client c
                                                      (STRONG scaling: the total is fixed), the IQ block crossing NVLink every step,
                                                      plus the north-star load paced at real time as a sub-object.
   python bench.py --impl reference ...              the CPU chain (oracle port; pycsdr cannot be built here) on the host cores
+  python bench.py --gpus 1 ... --dump-outputs DIR   also writes DIR/audio.npy: the float32 audio [channels, samples] of the last
+                                                     timed step, as a caller of the device path receives it; the input is seeded,
+                                                     so two builds run with the same arguments can be compared output for output
 
 A step = one pass of the hot path (Shift -> FirDecimate -> [FractionalDecimator] -> Bandpass -> Squelch -> demodulator -> Agc for
 every channel) over one synthetic IQ block.  Prints ONE JSON line (rank 0): `value` = device-resident throughput (CUDA events,
@@ -368,6 +371,17 @@ def time_bank_device(torch, bank, blocks, n, stream, steps, warmup):
     return ms, stages, (N.lib.owrx_launch_count() - l0) / steps
 
 
+def dump_audio(path, bank, chans):
+    """the outputs of the last process_device step: owrx_bank_drain moves them to the host queues, one read pops every channel's
+    audio; written as float32 [channels, samples] (every channel of the workload has the same output rate)"""
+    bank.drain()
+    buf = np.empty((len(chans), 1 << 15), np.float32)
+    counts = bank.read_audio_all(chans, buf)
+    assert len(set(counts)) == 1 and counts[0] > 0, counts
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "audio.npy"), buf[:, :counts[0]])
+
+
 def bench_selector_config(torch, dev, cfg, n_ch, hbm_peak, peak_src, f_mhz, steps=5, warmup=3, cpu_seconds=1.5):
     """one selector config on this GPU, device-resident, with its SURVEY 8(d) roofline and the CPU port beside it"""
     m = selector_model(cfg, n_ch)
@@ -480,6 +494,8 @@ def run_single(args, torch, local, dev):
     ms_step, stages, launches = time_bank_device(torch, bank, blocks, BLOCK, stream, args.steps, 0)
     fir_form = bank.fir_form()
     value = n_ch * consumed / (ms_step * 1e-3) / 1e6
+    if args.dump_outputs:
+        dump_audio(args.dump_outputs, bank, chans)
 
     # ---- e2e: public host API, pinned host input, H2D + audio D2H inside the timed region
     h_iq = torch.empty(BLOCK, 2, dtype=torch.float32).pin_memory()
@@ -917,7 +933,12 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--headline-only", action="store_true", help="skip the per-config sub-benchmarks (C1, C3, C4, C5 / the paced north-star run)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the audio of the last timed step to DIR/audio.npy (--gpus 1)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1):
+        ap.error("--dump-outputs covers the one-GPU workload of --impl ours (--gpus 1)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     # stdout carries exactly ONE JSON line: anything a library prints on fd 1 meanwhile (NCCL's version banner under
     # NCCL_DEBUG=VERSION, ...) is sent to stderr, and the line is written to the real stdout at the end

@@ -10,13 +10,9 @@ if ROOT not in sys.path:
 
 def _ensure_built():
     """A fresh checkout has no libowrx_b200.so / oracle .so (git-ignored) and an edited source leaves a stale one: (re)compile
-    (nvcc cross-compiles without a GPU)."""
-    so = os.path.join(ROOT, "openwebrx_b200", "libowrx_b200.so")
-    # on the GPU box the prebuilt library travels with the snapshot: build only if it is missing; in the development
-    # container (where /root/reference exists) also refresh a stale one (incremental, mtime-based)
-    if not os.path.exists(so) or os.path.isdir("/root/reference"):
-        import __graft_entry__
-        __graft_entry__.build()
+    (nvcc cross-compiles without a GPU).  The build is incremental (mtime-based): an up-to-date tree compiles nothing."""
+    import __graft_entry__
+    __graft_entry__.build()
 
 
 def pytest_configure(config):

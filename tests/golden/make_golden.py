@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Generates the committed golden fixtures.  Runs ONLY in the build container (needs /root/reference).
+"""Generates the committed golden fixtures.  Needs an OpenWebRX source tree: OWRX_REFERENCE=<path>.
 
 1. params_reference.json — the exact constructor / setter arguments the reference's UNMODIFIED
    csdr.chain classes (FftChain, Selector, Decimator, NFm/Am/Ssb/WFm) hand to pycsdr, captured with a
@@ -18,7 +18,7 @@ import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REF = os.environ.get("OWRX_REFERENCE", "/root/reference")
+REF = os.environ["OWRX_REFERENCE"]        # an OpenWebRX source tree
 
 LOG = []
 

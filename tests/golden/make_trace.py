@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Records the pycsdr call sequences of the reference's own, UNMODIFIED callers of the hot path and commits them as
-fixtures (tests/golden/trace_*.json).  Runs ONLY in the build container (needs /root/reference); the GPU box replays the
+fixtures (tests/golden/trace_*.json).  Needs an OpenWebRX source tree: OWRX_REFERENCE=<path>.  A GPU run replays the
 fixtures (tests/test_gpu_trace_replay.py) with IQ flowing between the recorded steps.
 
   trace_spectrum.json  owrx/fft.py:13-109     SpectrumThread(sdrSource).start(), then the on-the-fly property changes
@@ -25,7 +25,7 @@ from enum import Enum
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REF = os.environ.get("OWRX_REFERENCE", "/root/reference")
+REF = os.environ["OWRX_REFERENCE"]        # an OpenWebRX source tree
 sys.path.insert(0, ROOT)
 sys.path.insert(0, REF)
 

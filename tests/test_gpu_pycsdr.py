@@ -1,7 +1,6 @@
 """GPU tests of the drop-in boundary: pycsdr module objects wired with the reference's Chain._connect
-pattern (csdr/chain/__init__.py:21-25, restated locally because /root/reference is absent on the GPU box;
-when it is present the reference's own unmodified FftChain / Selector / NFm are driven as well)."""
-import os
+pattern (csdr/chain/__init__.py:21-25, restated locally: the reference's own classes are not part of this
+repository)."""
 import sys
 import threading
 import time
@@ -17,8 +16,6 @@ from pycsdr.types import AgcProfile, Format
 from test_oracle import JsImaAdpcmCodec, browser_fft_decode
 
 pytestmark = pytest.mark.gpu
-REF = os.environ.get("OWRX_REFERENCE", "/root/reference")
-HAVE_REF = os.path.isdir(os.path.join(REF, "csdr", "chain"))
 
 
 def _connect(workers):
@@ -163,9 +160,9 @@ def test_audio_tail_convert_and_adpcm_bit_exact(gpu):
         assert len(dec) == 4500
 
 
-# (The reference's own FftChain / SpectrumThread / DspManager classes cannot be imported on the GPU box — /root/reference does not
-# travel.  Their recorded call traces are replayed with data in tests/test_gpu_trace_replay.py; the classes themselves run
-# unmodified on the shim, without a device, in tests/test_pycsdr_shim.py.)
+# (The reference's own FftChain / SpectrumThread / DspManager classes are not part of this repository.  Their recorded call
+# traces are replayed with data in tests/test_gpu_trace_replay.py; the classes themselves run unmodified on the shim, without a
+# device, in tests/test_pycsdr_shim.py when OWRX_REFERENCE names an OpenWebRX source tree.)
 
 
 def test_raw_ingress_formats_equal_cpu_side_convert(gpu):

@@ -1,6 +1,6 @@
 """CPU tests of the drop-in `pycsdr` package: Buffer/Reader semantics, the module API surface the
 reference uses (SURVEY 8b, Appendix C/D), and chain discovery on chains built by the reference's own
-UNMODIFIED classes when /root/reference is present (it is absent on the GPU box)."""
+UNMODIFIED classes when the environment variable OWRX_REFERENCE names an OpenWebRX source tree."""
 import os
 import sys
 import threading
@@ -13,8 +13,9 @@ import pytest
 import pycsdr.modules as M
 from pycsdr.types import AgcProfile, Format
 
-REF = os.environ.get("OWRX_REFERENCE", "/root/reference")
-HAVE_REF = os.path.isdir(os.path.join(REF, "csdr", "chain"))
+REF = os.environ.get("OWRX_REFERENCE", "")
+HAVE_REF = bool(REF) and os.path.isdir(os.path.join(REF, "csdr", "chain"))
+NO_REF = "needs an OpenWebRX source tree named by OWRX_REFERENCE"
 
 
 def test_buffer_multi_reader_and_stop():
@@ -125,7 +126,7 @@ def test_chain_discovery_without_gpu():
     assert len(M._WaterfallPlan.match(M._walk(wf[0])[0])) == 3
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree not present (GPU box)")
+@pytest.mark.skipif(not HAVE_REF, reason=NO_REF)
 def test_reference_classes_run_unmodified_on_the_shim():
     sys.path.insert(0, REF)
     try:
@@ -201,7 +202,7 @@ def test_source_side_convert_gain_forwards_raw_samples_tagged():
     conv.stop(); gain.stop()
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="needs the reference tree (build container only)")
+@pytest.mark.skipif(not HAVE_REF, reason=NO_REF)
 def test_reference_fifi_sdr_format_conversion_runs_on_the_shim():
     """the reference's UNMODIFIED FifiSdrSource.getFormatConversion() (owrx/source/fifi_sdr.py:27-28), wired the way
     DirectSource.getBuffer does (owrx/source/direct.py:59-71), hands raw int16 samples on with gain 5.0"""

@@ -1,5 +1,5 @@
-import sys, time, torch, numpy as np
-sys.path.insert(0, '/root/repo')
+import os, sys, time, torch, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from openwebrx_b200 import ChannelBank
 from openwebrx_b200.synth import BANDPASS, carrier_plan
 FS=10_000_000; BLOCK=1<<24
