@@ -10,7 +10,6 @@
 
 #include <algorithm>
 #include <cmath>
-#include <cstring>
 
 namespace owrx {
 
@@ -668,12 +667,9 @@ int launch_contract_nw(const FcShape& sh, const float4* F, const float2* tab, in
 
 }  // namespace
 
-int fc_pick_fft_size(int D, int P)
+int fc_pick_fft_size(int D, int P, int force_m)
 {
-    if (const char* m = getenv("OWRX_FC_M")) {
-        const int v = atoi(m);
-        if ((v == FC_M || v == FC_M_SMALL) && P <= v / 2) return v;
-    }
+    if ((force_m == FC_M || force_m == FC_M_SMALL) && P <= force_m / 2) return force_m;
     return (D >= 2048 && P <= FC_M_SMALL / 2) ? FC_M_SMALL : FC_M;
 }
 
@@ -702,12 +698,9 @@ int fc_launch_table_tc(const FcShape& sh, const float* d_h, const int* d_slot_li
     return OWRX_OK;
 }
 
-int fc_pick_tc_levels(int D)
+int fc_pick_tc_levels(int D, int force_levels)
 {
-    if (const char* f = getenv("OWRX_FC_TC_FMT")) {
-        if (!strcmp(f, "bf16x3")) return 3;
-        if (!strcmp(f, "f16x2")) return 2;
-    }
+    if (force_levels == 2 || force_levels == 3) return force_levels;
     // fp16 x 2 pays where the contraction is what a pass costs — large decimations: few outputs per table entry (C3: 2.83 ->
     // 2.05 ms per step).  With a short decimation (C2, C5) the contraction is a third of the FIR chain, the chain is not what
     // bounds the step, and the extra read of the input for max|x| costs the other streams what the smaller operands save.
@@ -781,10 +774,8 @@ int fc_launch_forward_tc(const FcShape& sh, const float2* iq, long long n_lim, i
 // the split (<= FC_MAXSPLIT) that wastes the least of the last wave
 void fc_contract_plan(const FcShape& sh, int B, int sm_count, int* nw_out, int* nsplit_out)
 {
-    static const int force_nw = getenv("OWRX_FC_NW") ? atoi(getenv("OWRX_FC_NW")) : 0;
-    static const int force_split = getenv("OWRX_FC_SPLIT") ? atoi(getenv("OWRX_FC_SPLIT")) : 0;
     const int nbt0 = (B + 95) / 96;
-    const int nw = force_nw ? std::max(1, std::min(6, force_nw)) : std::max(1, std::min(6, ((B + nbt0 - 1) / nbt0 + 15) / 16));
+    const int nw = std::max(1, std::min(6, ((B + nbt0 - 1) / nbt0 + 15) / 16));
     const int nbt = (B + 16 * nw - 1) / (16 * nw);
     const size_t smem = (size_t)FC_ST * (16 * nw * FC_KC * sizeof(float4) + FC_KC * FC_CG * sizeof(float2));
     const int per_sm = std::max(1, std::min((int)((size_t)(220 << 10) / smem), 2048 / (nw * 64 + 32)));
@@ -799,7 +790,7 @@ void fc_contract_plan(const FcShape& sh, int B, int sm_count, int* nw_out, int* 
         if (cost < best_cost * 0.97) { best_cost = cost; best = sp; }
     }
     *nw_out = nw;
-    *nsplit_out = force_split ? std::max(1, std::min(FC_MAXSPLIT, force_split)) : best;
+    *nsplit_out = best;
 }
 
 int fc_launch_contract(const FcShape& sh, const float4* d_F, const float2* d_tab, int B, float2* d_Z, int sm_count, int* nsplit_out, cudaStream_t st)

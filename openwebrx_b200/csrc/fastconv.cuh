@@ -35,8 +35,8 @@ struct FcShape {
 // read once per pass) against the branch spectra (written and read once, M / Kb times the input).  With D in the thousands
 // a pass holds few outputs n_k per channel slot S and the table dominates: 64-point FFTs (Kb = 38 at P = 27) cut the table
 // to a quarter for 1.5 times the spectra (C3, D = 5120, 2^25 samples: 16.4 -> 5.3 GB at 1024 slots, 2.9 -> 1.9 GB at 128).
-// Short decimations keep 256 points (C2, D = 833, 64 slots: 61 vs 90 k per unit).  OWRX_FC_M = 64 / 256 overrides.
-int fc_pick_fft_size(int D, int P);
+// Short decimations keep 256 points (C2, D = 833, 64 slots: 61 vs 90 k per unit).  force_m = 64 | 256 overrides (when P fits).
+int fc_pick_fft_size(int D, int P, int force_m);
 
 // rebuild the table columns of `n` slots: slot_list[i], rate_list[i] (device arrays)
 int fc_launch_table(const FcShape& sh, const float* d_h, const int* d_slot_list, const double* d_rate_list, int n, float2* d_tab,
@@ -62,8 +62,8 @@ int fc_launch_inverse(const FcShape& sh, const float2* d_Z, int nsplit, int B, c
 //     so the result does not depend on the scale and IF(x / 2) == IF(x) / 2 stays exact.
 constexpr int FC_TC_MAXPLANES = 6;
 inline int fc_tc_planes(const FcShape& sh) { return 2 * sh.tc_levels; }
-// operand split of a new group: fp16 x 2 for D >= 2048, else bf16 x 3; OWRX_FC_TC_FMT = bf16x3 | f16x2 overrides
-int fc_pick_tc_levels(int D);
+// operand split of a new group: fp16 x 2 for D >= 2048, else bf16 x 3; force_levels = 2 | 3 overrides
+int fc_pick_tc_levels(int D, int force_levels);
 // exact power of two 2^kt for the table of a group with these taps (1 for levels = 3)
 float fc_tab_scale(const FcShape& sh, const float* h_taps);
 size_t fc_tc_plane_elems_F(const FcShape& sh, int B);
@@ -74,8 +74,9 @@ int fc_launch_table_tc(const FcShape& sh, const float* d_h, const int* d_slot_li
 // d_work: 4 bytes of device scratch (the running maximum)
 int fc_launch_scale(const FcShape& sh, const float2* iq, long long n, float tab_scale, unsigned* d_work, float* d_scale, cudaStream_t st);
 int fc_launch_forward_tc(const FcShape& sh, const float2* iq, long long n_lim, int B, void* d_Fp, const float* d_scale, cudaStream_t st);
-int fc_launch_contract_tc(const FcShape& sh, const void* d_Fp, const void* d_tabp, int B, float2* d_Z, int sm_count, int* nsplit,
-                          cudaStream_t st);
+// force_form: 0 = blocks in the MMA's M, 1 = slots in M, < 0 = whichever the cycle model picks
+int fc_launch_contract_tc(const FcShape& sh, const void* d_Fp, const void* d_tabp, int B, float2* d_Z, int sm_count, int force_form,
+                          int* nsplit, cudaStream_t st);
 
 // ------------------------------------------------------------------------------------------------
 // K4F: Bandpass (csdr/chain/selector.py:115-117,159-166; per-channel complex taps at the selector output rate) as a

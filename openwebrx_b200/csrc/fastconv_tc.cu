@@ -34,6 +34,8 @@ namespace owrx {
 namespace {
 
 constexpr unsigned TC_COLS = 256;                           // TMEM columns: D1 | D2
+constexpr int TC_KC = 16;                                   // branches per ring stage: one K = 16 MMA step
+constexpr unsigned TC_ROWB = 2 * TC_KC;                     // bytes per operand row of a stage: one SWIZZLE_32B atom
 
 __device__ __forceinline__ void mbar_init(unsigned bar, unsigned count)
 {
@@ -89,13 +91,11 @@ __device__ __forceinline__ void umma_desc(unsigned tmem_d, unsigned long long da
         "}\n" ::"r"(tmem_d), "l"(da), "l"(db), "r"(idesc), "r"(accumulate)
         : "memory");
 }
-// K-major shared-memory matrix descriptor (cute::UMMA::SmemDescriptor) for operand rows of `rowb` bytes — one swizzle atom
-// along K (64: SWIZZLE_64B, layout type 4; 32: SWIZZLE_32B, type 6): start >> 4 in [0,14), LBO unused, SBO = 8 rows >> 4 in
-// [32,46), version 1 in [46,48), layout type in [61,64)
-__device__ __forceinline__ unsigned long long smem_desc_rows(unsigned addr, unsigned rowb)
+// K-major shared-memory matrix descriptor (cute::UMMA::SmemDescriptor) for operand rows of TC_ROWB = 32 bytes — one SWIZZLE_32B
+// atom along K: start >> 4 in [0,14), LBO unused, SBO = 8 rows >> 4 in [32,46), version 1 in [46,48), layout type 6 in [61,64)
+__device__ __forceinline__ unsigned long long smem_desc_rows(unsigned addr)
 {
-    const unsigned long long layout = rowb == 64 ? 4ull : 6ull;
-    return (unsigned long long)((addr & 0x3FFFFu) >> 4) | ((unsigned long long)((8u * rowb) >> 4) << 32) | (1ull << 46) | (layout << 61);
+    return (unsigned long long)((addr & 0x3FFFFu) >> 4) | ((unsigned long long)((8u * TC_ROWB) >> 4) << 32) | (1ull << 46) | (6ull << 61);
 }
 
 // the partial products (A level, B level), smallest first: three levels (bf16) keep the six of weight > 2^-24, two levels (fp16)
@@ -110,13 +110,11 @@ __device__ __forceinline__ unsigned tc_idesc(int levels, unsigned n)
     return (1u << 4) | (fmt << 7) | (fmt << 10) | ((n >> 3) << 17) | ((128u >> 4) << 24);
 }
 
-// kc = branches per ring stage: 32 (64-byte operand rows, SWIZZLE_64B, two K = 16 steps per stage: round 1's form, OWRX_FC_TC_KC=32)
-// or 16 (32-byte rows, SWIZZLE_32B, one step; default).  With 16-branch stages three stages of a 64-slot x 88-block tile are
-// 88 KB, so TWO CTAs share an SM (256 TMEM columns each): C2's 256 tiles are all resident at once — no second, 73 %-full wave —
-// and an SM keeps two operand streams in flight.
+// With 16-branch stages (TC_KC) three stages of a 64-slot x 88-block tile are 88 KB, so TWO CTAs share an SM (256 TMEM columns
+// each): C2's 256 tiles are all resident at once — no second, 73 %-full wave — and an SM keeps two operand streams in flight.
 __global__ void __launch_bounds__(192, 2)
 fc_contract_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB, float2* __restrict__ Z, int B, int Dp,
-                      int slots, int nbt, int mrows, int nsplit, int M, int kc, int nst, int levels)
+                      int slots, int nbt, int mrows, int nsplit, int M, int nst, int levels)
 {
     extern __shared__ unsigned char tc_smem_raw[];
     __shared__ unsigned long long bars[2 * TT_MAXST + 1];            // full[nst], empty[nst], accumulators ready
@@ -129,16 +127,15 @@ fc_contract_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_con
     const int q = (blockIdx.x / ngroups) / nbt, bt = (blockIdx.x / ngroups) % nbt;
     const int b0 = bt * mrows;
     const int rows = min(mrows, B - b0);
-    const int all_chunks = Dp / kc;
+    const int all_chunks = Dp / TC_KC;
     const int ch0 = (int)(((long long)all_chunks * blockIdx.z) / nsplit);
     const int nchunks = (int)(((long long)all_chunks * (blockIdx.z + 1)) / nsplit) - ch0;
     Z += (size_t)blockIdx.z * M * B * slots;
 
-    const unsigned rowb = (unsigned)kc * 2;                          // bytes per operand row of a stage
     const unsigned npl = 2u * (unsigned)levels;                      // operand planes: levels x (re, im)
-    const unsigned a_plane = (unsigned)mrows * rowb;                 // mrows is a multiple of 8: every plane starts on a swizzle atom
+    const unsigned a_plane = (unsigned)mrows * TC_ROWB;              // mrows is a multiple of 8: every plane starts on a swizzle atom
     const unsigned a_stage = npl * a_plane;
-    const unsigned b_plane = FC_CG * rowb;
+    const unsigned b_plane = FC_CG * TC_ROWB;
     const unsigned stage_bytes = a_stage + npl * b_plane;
     const unsigned smem0 = ((unsigned)__cvta_generic_to_shared(tc_smem_raw) + 1023u) & ~1023u;
     const unsigned bar0 = (unsigned)__cvta_generic_to_shared(bars);
@@ -174,15 +171,14 @@ fc_contract_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_con
                 const unsigned sa = smem0 + stage * stage_bytes;
                 // rows past the tile's last block come from the next bin (or are zero-filled past the tensor): they only
                 // feed accumulator rows that are never stored
-                tma_load_3d(sa, &mapA, (ch0 + ch) * kc, q * B + b0, 0, full);
-                tma_load_3d(sa + a_stage, &mapB, (ch0 + ch) * kc, q * slots + cg * FC_CG, 0, full);
+                tma_load_3d(sa, &mapA, (ch0 + ch) * TC_KC, q * B + b0, 0, full);
+                tma_load_3d(sa + a_stage, &mapB, (ch0 + ch) * TC_KC, q * slots + cg * FC_CG, 0, full);
                 if (++stage == nst) { stage = 0; phase ^= 1; }
             }
         }
         __syncwarp();
     } else if (wid == 1) {
         if (lane == 0) {
-            const int ksteps = kc / 16;
             const unsigned idesc = tc_idesc(levels, 128u);
             const int nprod = levels == 3 ? 6 : 3;
             int stage = 0;
@@ -191,16 +187,14 @@ fc_contract_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_con
                 mbar_wait(bar0 + 8 * stage, phase);                   // the stage's bytes have landed
                 asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory");
                 const unsigned sa = smem0 + stage * stage_bytes, sb = sa + a_stage;
-                for (int kk = 0; kk < ksteps; kk++) {
-                    for (int p = 0; p < nprod; p++) {
-                        const int la = levels == 3 ? kTcProd3[p][0] : kTcProd2[p][0], lb = levels == 3 ? kTcProd3[p][1] : kTcProd2[p][1];
-                        const unsigned long long d_re = smem_desc_rows(sa + (unsigned)(2 * la) * a_plane + kk * 32, rowb);
-                        const unsigned long long d_im = smem_desc_rows(sa + (unsigned)(2 * la + 1) * a_plane + kk * 32, rowb);
-                        const unsigned long long d_b = smem_desc_rows(sb + (unsigned)(2 * lb) * b_plane + kk * 32, rowb);
-                        const unsigned acc = (ch | kk | p) != 0;
-                        umma_desc(tmem, d_re, d_b, idesc, acc);       // D1 += F_re . [T_re | T_im]
-                        umma_desc(tmem + 128, d_im, d_b, idesc, acc); // D2 += F_im . [T_re | T_im]
-                    }
+                for (int p = 0; p < nprod; p++) {
+                    const int la = levels == 3 ? kTcProd3[p][0] : kTcProd2[p][0], lb = levels == 3 ? kTcProd3[p][1] : kTcProd2[p][1];
+                    const unsigned long long d_re = smem_desc_rows(sa + (unsigned)(2 * la) * a_plane);
+                    const unsigned long long d_im = smem_desc_rows(sa + (unsigned)(2 * la + 1) * a_plane);
+                    const unsigned long long d_b = smem_desc_rows(sb + (unsigned)(2 * lb) * b_plane);
+                    const unsigned acc = (ch | p) != 0;
+                    umma_desc(tmem, d_re, d_b, idesc, acc);           // D1 += F_re . [T_re | T_im]
+                    umma_desc(tmem + 128, d_im, d_b, idesc, acc);     // D2 += F_im . [T_re | T_im]
                 }
                 umma_commit(bar0 + 8 * (TT_MAXST + stage));           // slot free once these MMAs have read it
                 if (++stage == nst) { stage = 0; phase ^= 1; }
@@ -252,14 +246,13 @@ fc_contract_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_con
 // frees up: measured at C3, three 64-block tiles re-read most of the table from DRAM, not from L2).
 // ------------------------------------------------------------------------------------------------
 constexpr int TT_SLOTS = 128;                               // channel slots per CTA (the MMA's M)
-// kc = branches per ring stage: 32 (64-byte operand rows, two K = 16 steps per stage) or 16 (32-byte rows, one step).  What a
-// table-bound pass needs is bytes in flight: an SM streams (stages x stage bytes) per (load latency + MMA time of a stage).  With
-// 128-slot table tiles a 32-branch stage is 48 KB + 6 x 64 B per block row — only two fit beside 96 block rows, and the ring then
-// delivers 2 stages per (2.0 + 1.2) us: 52 GB/s per SM, below the SM's share of DRAM.  16-branch stages halve the granule: five of
-// 42 KB fit, 5 per (2.0 + 0.6) us.
+// Ring stages of 16 branches (TC_KC): what a table-bound pass needs is bytes in flight, and an SM streams (stages x stage bytes)
+// per (load latency + MMA time of a stage).  With 128-slot table tiles a 32-branch stage would be 48 KB + 6 x 64 B per block row —
+// only two fit beside 96 block rows, and the ring then delivers 2 stages per (2.0 + 1.2) us: 52 GB/s per SM, below the SM's share
+// of DRAM.  16-branch stages halve the granule: five of 42 KB fit, 5 per (2.0 + 0.6) us.
 __global__ void __launch_bounds__(192, 1)
 fc_contract_tct_kernel(const __grid_constant__ CUtensorMap mapF, const __grid_constant__ CUtensorMap mapT, float2* __restrict__ Z, int B, int Dp,
-                       int slots, int nbt, int mrows, int nsplit, int M, int kc, int nst, unsigned tmem_cols, int levels)
+                       int slots, int nbt, int mrows, int nsplit, int M, int nst, unsigned tmem_cols, int levels)
 {
     extern __shared__ unsigned char tc_smem_raw[];
     __shared__ unsigned long long bars[2 * TT_MAXST + 1];            // full[nst], empty[nst], accumulators ready
@@ -272,15 +265,14 @@ fc_contract_tct_kernel(const __grid_constant__ CUtensorMap mapF, const __grid_co
     const int q = (blockIdx.x / ngroups) / nbt, bt = (blockIdx.x / ngroups) % nbt;
     const int b0 = bt * mrows;
     const int rows = min(mrows, B - b0);
-    const int all_chunks = Dp / kc;
+    const int all_chunks = Dp / TC_KC;
     const int ch0 = (int)(((long long)all_chunks * blockIdx.z) / nsplit);
     const int nchunks = (int)(((long long)all_chunks * (blockIdx.z + 1)) / nsplit) - ch0;
     Z += (size_t)blockIdx.z * M * B * slots;
 
-    const unsigned rowb = (unsigned)kc * 2;                          // bytes per operand row of a stage
     const unsigned npl = 2u * (unsigned)levels;                      // operand planes: levels x (re, im)
-    const unsigned t_plane = TT_SLOTS * rowb, t_stage = npl * t_plane;
-    const unsigned f_plane = (unsigned)mrows * rowb;                 // mrows is a multiple of 8: every plane starts on a swizzle atom
+    const unsigned t_plane = TT_SLOTS * TC_ROWB, t_stage = npl * t_plane;
+    const unsigned f_plane = (unsigned)mrows * TC_ROWB;              // mrows is a multiple of 8: every plane starts on a swizzle atom
     const unsigned stage_bytes = t_stage + npl * f_plane;
     const unsigned smem0 = ((unsigned)__cvta_generic_to_shared(tc_smem_raw) + 1023u) & ~1023u;
     const unsigned bar0 = (unsigned)__cvta_generic_to_shared(bars);
@@ -317,8 +309,8 @@ fc_contract_tct_kernel(const __grid_constant__ CUtensorMap mapF, const __grid_co
                 const unsigned sa = smem0 + stage * stage_bytes;
                 // slot rows past the group's last slot / block rows past the tile's last block come from the next bin (or are
                 // zero-filled past the tensor): they only feed accumulator lanes / columns that are never stored
-                tma_load_3d(sa, &mapT, (ch0 + ch) * kc, q * slots + cg * TT_SLOTS, 0, full);
-                tma_load_3d(sa + t_stage, &mapF, (ch0 + ch) * kc, q * B + b0, 0, full);
+                tma_load_3d(sa, &mapT, (ch0 + ch) * TC_KC, q * slots + cg * TT_SLOTS, 0, full);
+                tma_load_3d(sa + t_stage, &mapF, (ch0 + ch) * TC_KC, q * B + b0, 0, full);
                 if (++stage == nst) { stage = 0; phase ^= 1; }
             }
         }
@@ -327,23 +319,20 @@ fc_contract_tct_kernel(const __grid_constant__ CUtensorMap mapF, const __grid_co
         if (lane == 0) {
             const unsigned idesc = tc_idesc(levels, ncols);          // N = 2 mrows, M = 128
             const int nprod = levels == 3 ? 6 : 3;
-            const int ksteps = kc / 16;
             int stage = 0;
             unsigned phase = 0;
             for (int ch = 0; ch < nchunks; ch++) {
                 mbar_wait(bar0 + 8 * stage, phase);
                 asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory");
                 const unsigned sa = smem0 + stage * stage_bytes, sf = sa + t_stage;
-                for (int kk = 0; kk < ksteps; kk++) {
-                    for (int p = 0; p < nprod; p++) {
-                        const int lt = levels == 3 ? kTcProd3[p][0] : kTcProd2[p][0], lf = levels == 3 ? kTcProd3[p][1] : kTcProd2[p][1];
-                        const unsigned long long d_re = smem_desc_rows(sa + (unsigned)(2 * lt) * t_plane + kk * 32, rowb);
-                        const unsigned long long d_im = smem_desc_rows(sa + (unsigned)(2 * lt + 1) * t_plane + kk * 32, rowb);
-                        const unsigned long long d_f = smem_desc_rows(sf + (unsigned)(2 * lf) * f_plane + kk * 32, rowb);   // [F_re ; F_im] of level lf
-                        const unsigned acc = (ch | kk | p) != 0;
-                        umma_desc(tmem, d_re, d_f, idesc, acc);           // D1 += T_re . [F_re | F_im]^T
-                        umma_desc(tmem + ncols, d_im, d_f, idesc, acc);   // D2 += T_im . [F_re | F_im]^T
-                    }
+                for (int p = 0; p < nprod; p++) {
+                    const int lt = levels == 3 ? kTcProd3[p][0] : kTcProd2[p][0], lf = levels == 3 ? kTcProd3[p][1] : kTcProd2[p][1];
+                    const unsigned long long d_re = smem_desc_rows(sa + (unsigned)(2 * lt) * t_plane);
+                    const unsigned long long d_im = smem_desc_rows(sa + (unsigned)(2 * lt + 1) * t_plane);
+                    const unsigned long long d_f = smem_desc_rows(sf + (unsigned)(2 * lf) * f_plane);   // [F_re ; F_im] of level lf
+                    const unsigned acc = (ch | p) != 0;
+                    umma_desc(tmem, d_re, d_f, idesc, acc);           // D1 += T_re . [F_re | F_im]^T
+                    umma_desc(tmem + ncols, d_im, d_f, idesc, acc);   // D2 += T_im . [F_re | F_im]^T
                 }
                 umma_commit(bar0 + 8 * (TT_MAXST + stage));
                 if (++stage == nst) { stage = 0; phase ^= 1; }
@@ -384,8 +373,8 @@ fc_contract_tct_kernel(const __grid_constant__ CUtensorMap mapF, const __grid_co
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
                                   const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
-// bf16 tensor [6 planes][rows][cols] (cols contiguous) with a (32 cols x box_rows x 6 planes) box, SWIZZLE_64B
-int make_plane_map(CUtensorMap* map, const void* base, size_t cols, size_t rows, unsigned box_rows, unsigned kc, int levels)
+// 16-bit tensor [2 levels planes][rows][cols] (cols contiguous) with a (TC_KC cols x box_rows x 2 levels planes) box, SWIZZLE_32B
+int make_plane_map(CUtensorMap* map, const void* base, size_t cols, size_t rows, unsigned box_rows, int levels)
 {
     static EncodeTiledFn encode = nullptr;
     if (!encode) {
@@ -397,10 +386,10 @@ int make_plane_map(CUtensorMap* map, const void* base, size_t cols, size_t rows,
     }
     const cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)rows, (cuuint64_t)(2 * levels)};
     const cuuint64_t strides[2] = {(cuuint64_t)cols * 2, (cuuint64_t)cols * rows * 2};
-    const cuuint32_t box[3] = {(cuuint32_t)kc, box_rows, (cuuint32_t)(2 * levels)};
+    const cuuint32_t box[3] = {(cuuint32_t)TC_KC, box_rows, (cuuint32_t)(2 * levels)};
     const cuuint32_t estr[3] = {1, 1, 1};
     const CUresult r = encode(map, levels == 3 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr,
-                              CU_TENSOR_MAP_INTERLEAVE_NONE, kc == 16 ? CU_TENSOR_MAP_SWIZZLE_32B : CU_TENSOR_MAP_SWIZZLE_64B,
+                              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_32B,
                               CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return fail(OWRX_E_CUDA, "cuTensorMapEncodeTiled (operand planes) failed (%d)", (int)r);
     return OWRX_OK;
@@ -424,13 +413,9 @@ int tc_plan_split(long long tiles, int chunks, int sm_count)
 size_t fc_tc_plane_elems_F(const FcShape& sh, int B) { return (size_t)sh.M * B * sh.Dp; }
 size_t fc_tc_plane_elems_tab(const FcShape& sh) { return (size_t)sh.M * sh.slots * sh.Dp; }
 
-int fc_launch_contract_tc(const FcShape& sh, const void* d_Fp, const void* d_tabp, int B, float2* d_Z, int sm_count, int* nsplit_out,
-                          cudaStream_t st)
+int fc_launch_contract_tc(const FcShape& sh, const void* d_Fp, const void* d_tabp, int B, float2* d_Z, int sm_count, int force_form,
+                          int* nsplit_out, cudaStream_t st)
 {
-    static const int force_split = getenv("OWRX_FC_SPLIT") ? atoi(getenv("OWRX_FC_SPLIT")) : 0;
-    // 0: blocks in M, 1: slots in M; read per launch (a host-side lookup) so that one process can exercise both forms
-    const char* ff = getenv("OWRX_FC_TC_FORM");
-    const int force_form = ff ? atoi(ff) : -1;
     CUtensorMap mapA, mapB;
     int rc;
     // ---- blocks in M: row tiles of <= 128 blocks, balanced, a multiple of 8 rows (the swizzle atom); 64 slots per CTA
@@ -447,48 +432,40 @@ int fc_launch_contract_tc(const FcShape& sh, const void* d_Fp, const void* d_tab
     const bool slots_in_m = force_form >= 0 ? (force_form == 1 && sh.slots >= FC_CG) : (sh.slots >= TT_SLOTS && cyc_t < cyc_m);
 
     if (slots_in_m) {
-        // OWRX_FC_TCT_KC = 32: the 64-byte-row stages of the first version (A/B runs)
-        const char* kce = getenv("OWRX_FC_TCT_KC");
-        const int kc = kce && atoi(kce) == 32 ? 32 : 16;
-        const int chunks_t = sh.Dp / kc;
+        const int chunks_t = sh.Dp / TC_KC;
         const int ngroups = (sh.slots + TT_SLOTS - 1) / TT_SLOTS;
-        const unsigned stage_bytes = npl * (unsigned)(TT_SLOTS + mrows_t) * (unsigned)kc * 2;
+        const unsigned stage_bytes = npl * (unsigned)(TT_SLOTS + mrows_t) * TC_ROWB;
         const int stages = std::max(2, std::min(TT_MAXST, (int)(((size_t)(220 << 10)) / stage_bytes)));
         const size_t smem = (size_t)stages * stage_bytes + 1024;
         const long long tiles = (long long)sh.M * nbt_t * ngroups;
-        if ((rc = make_plane_map(&mapA, d_Fp, (size_t)sh.Dp, (size_t)sh.M * B, (unsigned)mrows_t, (unsigned)kc, lv)) != OWRX_OK) return rc;
-        if ((rc = make_plane_map(&mapB, d_tabp, (size_t)sh.Dp, (size_t)sh.M * sh.slots, (unsigned)TT_SLOTS, (unsigned)kc, lv)) != OWRX_OK) return rc;
-        int nsplit = tc_plan_split(tiles, chunks_t, sm_count);
-        if (force_split) nsplit = std::max(1, std::min({FC_MAXSPLIT, force_split, chunks_t}));
+        if ((rc = make_plane_map(&mapA, d_Fp, (size_t)sh.Dp, (size_t)sh.M * B, (unsigned)mrows_t, lv)) != OWRX_OK) return rc;
+        if ((rc = make_plane_map(&mapB, d_tabp, (size_t)sh.Dp, (size_t)sh.M * sh.slots, (unsigned)TT_SLOTS, lv)) != OWRX_OK) return rc;
+        const int nsplit = tc_plan_split(tiles, chunks_t, sm_count);
         *nsplit_out = nsplit;
         // TMEM columns: D1 | D2, each 2 mrows wide; the allocation is a power of two >= 32
         unsigned cols = 32;
         while (cols < 4u * (unsigned)mrows_t) cols *= 2;
         OWRX_CUDA(cudaFuncSetAttribute(fc_contract_tct_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         fc_contract_tct_kernel<<<dim3((unsigned)tiles, 1, (unsigned)nsplit), 192, smem, st>>>(mapA, mapB, d_Z, B, sh.Dp, sh.slots, nbt_t, mrows_t,
-                                                                                               nsplit, sh.M, kc, stages, cols, lv);
+                                                                                               nsplit, sh.M, stages, cols, lv);
         OWRX_LAUNCH_CHECK();
         return OWRX_OK;
     }
 
-    // OWRX_FC_TC_KC = 32: round 1's 64-byte-row stages, three of them, one CTA per SM (A/B runs)
-    const char* kce = getenv("OWRX_FC_TC_KC");
-    const int kc = kce && atoi(kce) == 32 ? 32 : 16;
-    const int chunks_m = sh.Dp / kc;
-    const unsigned stage_bytes = npl * (unsigned)(mrows + FC_CG) * (unsigned)kc * 2;
-    // kc = 16: as many stages as leave room for two CTAs per SM (<= 110 KB each), at least three; kc = 32: three stages
-    const int stages = kc == 16 ? std::max(3, std::min(TT_MAXST, (int)(((size_t)(108 << 10)) / stage_bytes))) : 3;
+    const int chunks_m = sh.Dp / TC_KC;
+    const unsigned stage_bytes = npl * (unsigned)(mrows + FC_CG) * TC_ROWB;
+    // as many stages as leave room for two CTAs per SM (<= 110 KB each), at least three
+    const int stages = std::max(3, std::min(TT_MAXST, (int)(((size_t)(108 << 10)) / stage_bytes)));
     const size_t smem = (size_t)stages * stage_bytes + 1024;
     const long long tiles = (long long)sh.M * nbt * (sh.slots / FC_CG);
-    if ((rc = make_plane_map(&mapA, d_Fp, (size_t)sh.Dp, (size_t)sh.M * B, (unsigned)mrows, (unsigned)kc, lv)) != OWRX_OK) return rc;
-    if ((rc = make_plane_map(&mapB, d_tabp, (size_t)sh.Dp, (size_t)sh.M * sh.slots, (unsigned)FC_CG, (unsigned)kc, lv)) != OWRX_OK) return rc;
+    if ((rc = make_plane_map(&mapA, d_Fp, (size_t)sh.Dp, (size_t)sh.M * B, (unsigned)mrows, lv)) != OWRX_OK) return rc;
+    if ((rc = make_plane_map(&mapB, d_tabp, (size_t)sh.Dp, (size_t)sh.M * sh.slots, (unsigned)FC_CG, lv)) != OWRX_OK) return rc;
     const int per_sm = smem <= (size_t)(113 << 10) ? 2 : 1;
-    int nsplit = tc_plan_split(tiles, chunks_m, sm_count * per_sm);
-    if (force_split) nsplit = std::max(1, std::min({FC_MAXSPLIT, force_split, chunks_m}));
+    const int nsplit = tc_plan_split(tiles, chunks_m, sm_count * per_sm);
     *nsplit_out = nsplit;
     OWRX_CUDA(cudaFuncSetAttribute(fc_contract_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     fc_contract_tc_kernel<<<dim3((unsigned)tiles, 1, (unsigned)nsplit), 192, smem, st>>>(mapA, mapB, d_Z, B, sh.Dp, sh.slots, nbt, mrows, nsplit, sh.M,
-                                                                                          kc, stages, lv);
+                                                                                          stages, lv);
     OWRX_LAUNCH_CHECK();
     return OWRX_OK;
 }

@@ -12,6 +12,7 @@
 #include <cmath>
 #include <complex>
 #include <cstdlib>
+#include <cstring>
 #include <deque>
 #include <map>
 #include <memory>
@@ -356,12 +357,13 @@ struct owrx_bank {
     // deferred drain (owrx_bank_set_deferred_drain): a feed returns once its work is enqueued; its last outputs reach the
     // host queues at the start of the next feed — after that feed's uploads are under way — or in owrx_bank_flush
     bool deferred = false, pending_final = false;
-    cudaEvent_t carry_done = nullptr;
     int fir_form_used = 0;                           // form of the latest Shift + FirDecimate pass (owrx_bank_fir_form)
-    // evaluation variants kept for A/B runs and as second opinions in the tests (read from the environment at creation)
+    // forms the parity tests force at shapes where the cost models would not pick them (read from the environment at creation,
+    // like fir_mode)
     bool tail_fused = true;                          // OWRX_TAIL_FUSED=0: the seven-kernel low-rate tail
-    bool agc_cta = true;                             // OWRX_AGC_CTA=0: one warp per channel (agc_warp_kernel): 0.137 vs 0.219 ms alone,
-                                                     // but stretched to 0.51 ms by the other streams' CTAs on its SMs (C2 step 0.55 vs 0.29 ms)
+    int fc_m = 0;                                    // OWRX_FC_M = 64 | 256: branch FFT size of new groups (fc_pick_fft_size)
+    int fc_levels = 0;                               // OWRX_FC_TC_FMT = f16x2 | bf16x3: operand split of new groups (fc_pick_tc_levels)
+    int fc_tc_form = -1;                             // OWRX_FC_TC_FORM = 0 | 1: blocks | slots in the MMA's M (fc_launch_contract_tc)
     size_t last_consumed = 0;                        // device path: samples of the last block every group is done with
     // groups whose last client left: out of the feed loops at once, their device memory released by a later call once the
     // event (recorded behind everything issued while the group was live) has completed — no device synchronisation
@@ -471,8 +473,8 @@ int group_create(owrx_bank* bank, const owrx_chan_spec_t& sp, int* index)
     }
     g->fc_taps.resize((size_t)g->T);
     for (int t = 0; t < g->T; t++) g->fc_taps[(size_t)t] = (float)h[t];
-    const int fcM = fc_pick_fft_size(g->D, P);
-    g->fc = FcShape{g->D, g->T, P, fcM - P + 1, (g->D + FC_DPAD - 1) / FC_DPAD * FC_DPAD, g->slots, fcM, fc_pick_tc_levels(g->D)};
+    const int fcM = fc_pick_fft_size(g->D, P, bank->fc_m);
+    g->fc = FcShape{g->D, g->T, P, fcM - P + 1, (g->D + FC_DPAD - 1) / FC_DPAD * FC_DPAD, g->slots, fcM, fc_pick_tc_levels(g->D, bank->fc_levels)};
     g->fc_tab_scale = fc_tab_scale(g->fc, g->fc_taps.data());
     g->fc_ok = g->D >= 8 && P <= fcM / 2;
     int rc;
@@ -956,7 +958,7 @@ int group_fir_fastconv(owrx_bank* bank, Group* g, const float2* iq, size_t n_ava
         if ((rc = prof_mark(bank, OWRX_PROF_FC_FORWARD, st, false)) != OWRX_OK) return rc;
         if ((rc = prof_mark(bank, OWRX_PROF_FC_CONTRACT, st, true)) != OWRX_OK) return rc;
         int nsplit = 1;
-        rc = tc ? fc_launch_contract_tc(sh, g->d_fc_Fp, g->d_fc_tabp, B, g->d_fc_Z, bank->sm_count, &nsplit, st)
+        rc = tc ? fc_launch_contract_tc(sh, g->d_fc_Fp, g->d_fc_tabp, B, g->d_fc_Z, bank->sm_count, bank->fc_tc_form, &nsplit, st)
                 : fc_launch_contract(sh, g->d_fc_F, g->d_fc_tab, B, g->d_fc_Z, bank->sm_count, &nsplit, st);
         if (rc != OWRX_OK) return rc;
         if ((rc = prof_mark(bank, OWRX_PROF_FC_CONTRACT, st, false)) != OWRX_OK) return rc;
@@ -1307,18 +1309,9 @@ int group_tail_serial(owrx_bank* bank, Group* g, cudaStream_t st)
                 // a 66 KB FFT CTA can share their SM (measured inside the three-stream pipeline, C2, with a 100 KB claim while
                 // the contraction needed 177 KB: Agc stage 0.32 -> 0.26 ms, step 0.34 -> 0.32 ms).  OWRX_AGC_PAD_KB overrides.
                 static const int agc_pad = (getenv("OWRX_AGC_PAD_KB") ? atoi(getenv("OWRX_AGC_PAD_KB")) : 160) << 10;
-                // one warp per channel with no CTA barrier (agc_warp_kernel) unless OWRX_AGC_CTA=1 asks for the 8-channel CTAs
-                const bool agc_cta = bank->agc_cta;
-                static const int agcw_pad = (getenv("OWRX_AGCW_PAD_KB") ? atoi(getenv("OWRX_AGCW_PAD_KB")) : 0) << 10;
-                if (agc_cta) {
-                    if (agc_pad) OWRX_CUDA(cudaFuncSetAttribute(agc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, agc_pad));
-                    agc_kernel<<<S / AGC_CH, AGC_TL, agc_pad, st>>>(g->f2.rows(g->f2.fill - n_audio), S, (int)n_audio, g->d_cfg, g->d_state,
-                                                               g->f3.append_ptr());
-                } else {
-                    if (agcw_pad) OWRX_CUDA(cudaFuncSetAttribute(agc_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, agcw_pad));
-                    agc_warp_kernel<<<S, 32, agcw_pad, st>>>(g->f2.rows(g->f2.fill - n_audio), S, (int)n_audio, g->d_cfg, g->d_state,
+                if (agc_pad) OWRX_CUDA(cudaFuncSetAttribute(agc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, agc_pad));
+                agc_kernel<<<S / AGC_CH, AGC_TL, agc_pad, st>>>(g->f2.rows(g->f2.fill - n_audio), S, (int)n_audio, g->d_cfg, g->d_state,
                                                            g->f3.append_ptr());
-                }
                 OWRX_LAUNCH_CHECK();
             }
             if ((rc = prof_mark(bank, OWRX_PROF_AGC, st, false)) != OWRX_OK) return rc;
@@ -1512,8 +1505,9 @@ int owrx_bank_create(int device, double input_rate, owrx_bank_t** out)
     if (const char* m = getenv("OWRX_FIR_MODE")) b->fir_mode = std::max(OWRX_FIR_AUTO, std::min(OWRX_FIR_FASTCONV_TC, atoi(m)));
     b->bp_mode = std::min(b->fir_mode, OWRX_FIR_FASTCONV);
     if (const char* m = getenv("OWRX_TAIL_FUSED")) b->tail_fused = atoi(m) != 0;
-    if (const char* m = getenv("OWRX_AGC_CTA")) b->agc_cta = atoi(m) != 0;
-    if (const char* m = getenv("OWRX_BP_MODE")) b->bp_mode = std::max(OWRX_FIR_AUTO, std::min(OWRX_FIR_FASTCONV, atoi(m)));
+    if (const char* m = getenv("OWRX_FC_M")) b->fc_m = atoi(m);
+    if (const char* f = getenv("OWRX_FC_TC_FMT")) b->fc_levels = !strcmp(f, "bf16x3") ? 3 : !strcmp(f, "f16x2") ? 2 : 0;
+    if (const char* f = getenv("OWRX_FC_TC_FORM")) b->fc_tc_form = atoi(f);
     cudaError_t e = cudaStreamCreateWithFlags(&b->stream, cudaStreamNonBlocking);
     if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&b->copy_stream, cudaStreamNonBlocking);
     // The parallel low-rate stages are a chain of a dozen small dependent launches: on a high-priority stream their CTAs go
@@ -1534,7 +1528,6 @@ int owrx_bank_create(int device, double input_rate, owrx_bank_t** out)
     if (e == cudaSuccess) e = cudaEventCreate(&b->ev0);
     if (e == cudaSuccess) e = cudaEventCreate(&b->ev1);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&b->fir_done, cudaEventDisableTiming);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&b->carry_done, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&b->dev_done, cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&b->tail_done[0], cudaEventDisableTiming);
     if (e == cudaSuccess) e = cudaEventCreateWithFlags(&b->tail_done[1], cudaEventDisableTiming);
@@ -1552,7 +1545,6 @@ void owrx_bank_destroy(owrx_bank_t* bank)
     reap_groups(bank, true);
     if (bank->ctl_stream) cudaStreamDestroy(bank->ctl_stream);
     cudaFree(bank->d_iq[0]); cudaFree(bank->d_iq[1]); cudaFree(bank->d_xpose); cudaFree(bank->d_raw);
-    if (bank->carry_done) cudaEventDestroy(bank->carry_done);
     for (cudaEvent_t e : bank->chunk_events) cudaEventDestroy(e);
     for (cudaEvent_t e : bank->fir_events) cudaEventDestroy(e);
     for (cudaEvent_t e : bank->drain_events) cudaEventDestroy(e);
@@ -1960,8 +1952,6 @@ int owrx_bank_feed_fmt(owrx_bank_t* bank, const void* iq_raw, size_t n_samples, 
     // previous feed's carry copy (on `st`) fills [0, iq_fill) of the same buffer, and the last kernels that READ this buffer
     // belong to the feed before the previous one, which has been synchronised (finish_pending / the synchronous return) before
     // this call.  So this feed's chunks queue right behind the previous feed's on the copy stream: PCIe never idles.
-    static const bool wait_carry = getenv("OWRX_FEED_WAIT_CARRY") != nullptr;    // the conservative ordering, for A/B runs
-    if (wait_carry) OWRX_CUDA(cudaStreamWaitEvent(bank->copy_stream, bank->carry_done, 0));
     for (size_t c = 0; c < n_chunks; c++) {
         const size_t o = c * chunk, len = std::min(chunk, n_samples - o);
         if (len && format == OWRX_IQ_CF32) {
@@ -2058,7 +2048,6 @@ int owrx_bank_feed_fmt(owrx_bank_t* bank, const void* iq_raw, size_t n_samples, 
         bank->iq_fill = tail;
         for (auto& gp : bank->groups) if (gp) gp->in_off -= min_off;
     }
-    OWRX_CUDA(cudaEventRecord(bank->carry_done, st));
     if (overlap) {
         OWRX_CUDA(cudaEventRecord(bank->fir_done, tails));
         OWRX_CUDA(cudaStreamWaitEvent(st, bank->fir_done, 0));

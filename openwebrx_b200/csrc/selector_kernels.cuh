@@ -1056,62 +1056,6 @@ agc_kernel(const float* __restrict__ in, int slots, int n, const ChanCfg* __rest
     }
 }
 
-// agc_warp_kernel — the same recurrence, one WARP per CTA and channel, no CTA barrier anywhere.  The 8-channel CTA above stages
-// [256 samples][8 slots] tiles through shared memory behind two __syncthreads per tile: every warp of the CTA then moves at the
-// pace of its slowest channel (a third of the stall samples of the r1 capture sit behind those barriers) and two warps share
-// each scheduler.  Here a warp streams its own channel: the 128 samples of a step arrive through a 4-deep cp.async ring
-// (4-byte gathers `slots` floats apart: 32 sectors per request, all L2 hits — a C2 block of all 64 channels is 5 MB), outputs
-// leave as 4-byte scattered stores, and every channel gets a scheduler — with <= 148 channels an SM — of its own.
-constexpr int AGCW_STAGES = 4;
-__global__ void __launch_bounds__(32)
-agc_warp_kernel(const float* __restrict__ in, int slots, int n, const ChanCfg* __restrict__ cfg, ChanState* __restrict__ st,
-                float* __restrict__ out)
-{
-    __shared__ __align__(16) float ring[AGCW_STAGES][32 * AGC_E];
-    __shared__ __align__(16) float U[32 * AGC_E + 8];
-    if (n <= 0) return;
-    const int lane = threadIdx.x;
-    const int s = blockIdx.x;
-    const ChanCfg c = cfg[s];
-    const bool bypass = c.kind == OWRX_DEMOD_WFM || c.kind == OWRX_DEMOD_NONE;
-    AgcWarp a{st[s].agc_gain, 1.f - c.agc_attack, 1.f + c.agc_decay, c.agc_thr, c.agc_max, st[s].agc_hang, c.agc_hang_time};
-    a.gain = fmaxf(fminf(a.gain, a.gmax), 0.f);
-    constexpr int SL = 32 * AGC_E;                                   // samples per step
-    const int ns = (n + SL - 1) / SL;
-    const float* src = in + s;
-    auto issue = [&](int step) {
-        if (step < ns) {
-            const int i0 = step * SL + AGC_E * lane;
-#pragma unroll
-            for (int e = 0; e < AGC_E; e++) {
-                float* dst = &ring[step % AGCW_STAGES][AGC_E * lane + e];
-                if (i0 + e < n) cp_async4(dst, src + (size_t)(i0 + e) * slots);
-                else *dst = 0.f;                                     // zeros change neither state nor outputs
-            }
-        }
-        cp_async_commit();
-    };
-#pragma unroll
-    for (int k = 0; k < AGCW_STAGES - 1; k++) issue(k);
-    for (int step = 0; step < ns; step++) {
-        issue(step + AGCW_STAGES - 1);
-        cp_async_wait<AGCW_STAGES - 1>();
-        __syncwarp();
-        const float4 x4 = *reinterpret_cast<const float4*>(&ring[step % AGCW_STAGES][AGC_E * lane]);
-        float v[AGC_E] = {x4.x, x4.y, x4.z, x4.w};
-        if (!bypass) a.step(v, lane, U);
-        const int i0 = step * SL + AGC_E * lane;
-#pragma unroll
-        for (int e = 0; e < AGC_E; e++)
-            if (i0 + e < n) out[(size_t)(i0 + e) * slots + s] = v[e];
-        __syncwarp();                                                // the ring slot is rewritten by the next issue
-    }
-    if (lane == 0 && !bypass) {
-        st[s].agc_gain = a.gain;
-        st[s].agc_hang = a.hang;
-    }
-}
-
 // [n][slots] -> [slots][n] (output drain: one contiguous run per channel for the host)
 template <typename T>
 __global__ void __launch_bounds__(256) transpose_kernel(const T* __restrict__ in, int slots, size_t n, T* __restrict__ out)

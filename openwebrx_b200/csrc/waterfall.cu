@@ -6,11 +6,12 @@
 // Arithmetic spec: SURVEY.md Appendix A.2-A.5.
 //
 // Kernels (all hand-written, no cuFFT):
-//   wf_colpass_kernel<R0>   four-step column pass for N > 4096 (N = R0 x 4096): window, radix-R0
-//                           butterfly, W_N twiddle, writes the row-major scratch Y.
-//   wf_fft_kernel<LOG2M,..> shared-memory Stockham FFT of M <= 4096 points (radix 16,16,R3) with the
-//                           Hamming window fused into the load and |X|^2 accumulated in REGISTERS over
-//                           the avg frames of a line; one CTA per (line, row, frame-subset).
+//   wf_fft_kernel<LOG2M>    shared-memory Stockham FFT of M < 4096 points (radix 16,16,R3) with the
+//                           Hamming window fused into the load and |X|^2 accumulated over the avg
+//                           frames of a line; one CTA per (line, frame-subset).
+//   wf_fft2_kernel          the same for 4096 points on packed FP32, two frames per pass.
+//   wf_big_kernel<R0>       the four-step FFT of N = R0 x 4096 points (8192 ... 65536), one cluster
+//                           of R0 CTAs per frame pair.
 //   wf_finalize_kernel      sums the frame-subset partials, 10*log10 + add_db - 10*log10(avg),
 //                           half-swap on store, x100 -> int16 truncation + 10-sample pad.
 //   wf_adpcm_kernel         IMA-ADPCM, state reset per line, low nibble first.
@@ -30,23 +31,21 @@ namespace owrx {
 __device__ __forceinline__ int pad16(int i) { return i + (i >> 4); }
 
 struct WfFftParams {
-    const float2* src;       // FROM_IQ: wideband IQ;  else: scratch Y
-    const float* window;     // N floats (FROM_IQ only)
+    const float2* src;       // wideband IQ
+    const float* window;     // M floats
     const float2* tw2;       // [16][16]   exp(-2 pi i r k / 256)
     const float2* tw3;       // [R3][256]  exp(-2 pi i r k / M)
-    float* partial;          // [line][subset][N] partial power sums
-    int every_n;             // hop E between frames (FROM_IQ)
+    float* partial;          // [line][subset][M] partial power sums
+    int every_n;             // hop E between frames
     int frames_per_line;     // avg (or 1)
     int subsets;             // S frame-subsets per line
-    int r0;                  // four-step rows (1 when FROM_IQ)
-    int n;                   // full FFT size N = r0 * M
-    long long first_frame;   // FROM_IQ: global frame index of line 0 of this launch
-    int units;               // wf_fft2_kernel: (line, row, subset) units of this launch, handed out through `counter`
+    long long first_frame;   // global frame index of line 0 of this launch
+    int units;               // wf_fft2_kernel: (line, subset) units of this launch, handed out through `counter`
     int* counter;            // wf_fft2_kernel: zeroed before the launch
 };
 
-// One CTA per (line, row k1, frame subset).  M = 2^LOG2M points, T = M/16 threads.
-template <int LOG2M, bool FROM_IQ>
+// One CTA per (line, frame subset).  M = 2^LOG2M points, T = M/16 threads.
+template <int LOG2M>
 __global__ void __launch_bounds__((1 << LOG2M) / 16 < 32 ? 32 : (1 << LOG2M) / 16, LOG2M >= 11 ? 2 : 1)
 wf_fft_kernel(WfFftParams p)
 {
@@ -63,11 +62,8 @@ wf_fft_kernel(WfFftParams p)
 
     const int tid = threadIdx.x;
     const bool active = tid < T;
-    int unit = blockIdx.x;
-    const int subset = unit % p.subsets;
-    unit /= p.subsets;
-    const int k1 = unit % p.r0;
-    const int line = unit / p.r0;
+    const int subset = blockIdx.x % p.subsets;
+    const int line = blockIdx.x / p.subsets;
 
     const int per = (p.frames_per_line + p.subsets - 1) / p.subsets;
     const int a0 = subset * per;
@@ -80,7 +76,7 @@ wf_fft_kernel(WfFftParams p)
 
     // the Hamming window values of this thread's 16 points are the same for every frame of the line: keep them in registers
     float wreg[16];
-    if (FROM_IQ && active) {
+    if (active) {
 #pragma unroll
         for (int r = 0; r < 16; r++) wreg[r] = __ldg(p.window + tid + r * T);
     }
@@ -89,23 +85,17 @@ wf_fft_kernel(WfFftParams p)
         float2 v[16];
         const long long frame = (long long)line * p.frames_per_line + a;
         if (active) {
-            if (FROM_IQ) {
-                const float2* x = p.src + (p.first_frame + frame) * (long long)p.every_n;
-                if (a + 1 < a1) {
-                    // pull the next frame (M * 8 bytes = M/16 lines of 128 B: one per thread) towards the SM while this one is
-                    // transformed: its loads then find L2 instead of HBM
-                    const char* nx = reinterpret_cast<const char*>(x + p.every_n) + (size_t)tid * 128;
-                    asm volatile("prefetch.global.L2 [%0];" ::"l"(nx));
-                }
+            const float2* x = p.src + (p.first_frame + frame) * (long long)p.every_n;
+            if (a + 1 < a1) {
+                // pull the next frame (M * 8 bytes = M/16 lines of 128 B: one per thread) towards the SM while this one is
+                // transformed: its loads then find L2 instead of HBM
+                const char* nx = reinterpret_cast<const char*>(x + p.every_n) + (size_t)tid * 128;
+                asm volatile("prefetch.global.L2 [%0];" ::"l"(nx));
+            }
 #pragma unroll
-                for (int r = 0; r < 16; r++) {
-                    float2 s = __ldg(x + tid + r * T);
-                    v[r] = make_float2(s.x * wreg[r], s.y * wreg[r]);
-                }
-            } else {
-                const float2* x = p.src + (frame * p.r0 + k1) * (long long)M;
-#pragma unroll
-                for (int r = 0; r < 16; r++) v[r] = __ldg(x + tid + r * T);
+            for (int r = 0; r < 16; r++) {
+                float2 s = __ldg(x + tid + r * T);
+                v[r] = make_float2(s.x * wreg[r], s.y * wreg[r]);
             }
             // pass 1: radix 16, Ns = 1
             dft<16>(v);
@@ -149,7 +139,7 @@ wf_fft_kernel(WfFftParams p)
     }
 
     if (active) {
-        float* out = p.partial + ((size_t)line * p.subsets + subset) * (size_t)p.n;
+        float* out = p.partial + ((size_t)line * p.subsets + subset) * (size_t)M;
 #pragma unroll
         for (int q = 0; q < 16; q++) {
             int bin;
@@ -160,7 +150,7 @@ wf_fft_kernel(WfFftParams p)
             } else {
                 bin = tid + slot<16>(q) * 16;          // M == 256
             }
-            out[(size_t)k1 + (size_t)p.r0 * bin] = accS[q * T + tid];
+            out[bin] = accS[q * T + tid];
         }
     }
 }
@@ -225,8 +215,7 @@ __device__ __forceinline__ void c2dft16(C2* v)
     for (int m1 = 0; m1 < 4; m1++) c2dft4(v[4 * m1], v[4 * m1 + 1], v[4 * m1 + 2], v[4 * m1 + 3]);
 }
 
-// M = 4096 points: 256 threads x 16 points, radix 16 x 16 x 16; one CTA per (line, four-step row, frame subset).
-template <bool FROM_IQ>
+// M = 4096 points: 256 threads x 16 points, radix 16 x 16 x 16; one CTA per (line, frame subset).
 __global__ void __launch_bounds__(256, 2)
 wf_fft2_kernel(WfFftParams p)
 {
@@ -237,14 +226,11 @@ wf_fft2_kernel(WfFftParams p)
     const int k = tid & 15;
     const int base2 = (tid >> 4) * 256 + k;
     const int per = (p.frames_per_line + p.subsets - 1) / p.subsets;
-    // Persistent CTAs take (line, row, subset) units from a global counter: the grid is one resident wave, and an SM that is
-    // late (or held by the side-stream ADPCM encoder) simply takes fewer units — no wave quantisation.
+    // Persistent CTAs take (line, subset) units from a global counter: the grid is one resident wave, and an SM that is late
+    // (or held by the side-stream ADPCM encoder) simply takes fewer units — no wave quantisation.
     for (int cur = blockIdx.x; cur < p.units;) {
-    int unit = cur;
-    const int subset = unit % p.subsets;
-    unit /= p.subsets;
-    const int k1 = unit % p.r0;
-    const int line = unit / p.r0;
+    const int subset = cur % p.subsets;
+    const int line = cur / p.subsets;
     const int a0 = subset * per;
     const int a1 = min(p.frames_per_line, a0 + per);
     if (tid == 0) s_next = atomicAdd(p.counter, 1) + (int)gridDim.x;
@@ -257,33 +243,21 @@ wf_fft2_kernel(WfFftParams p)
         const bool two = a + 1 < a1;
         C2 v[16];
         const long long frame = (long long)line * p.frames_per_line + a;
-        if (FROM_IQ) {
-            const float2* x0 = p.src + (p.first_frame + frame) * (long long)p.every_n;
-            const float2* x1 = x0 + p.every_n;
-            if (a + 2 < a1) {
-                // pull the next pair of frames towards L2 while this one is transformed (one 128-byte line per thread and frame)
-                const char* nx = reinterpret_cast<const char*>(x1 + p.every_n) + (size_t)tid * 128;
-                asm volatile("prefetch.global.L2 [%0];" ::"l"(nx));
-                if (a + 3 < a1) asm volatile("prefetch.global.L2 [%0];" ::"l"(nx + (size_t)p.every_n * 8));
-            }
+        const float2* x0 = p.src + (p.first_frame + frame) * (long long)p.every_n;
+        const float2* x1 = x0 + p.every_n;
+        if (a + 2 < a1) {
+            // pull the next pair of frames towards L2 while this one is transformed (one 128-byte line per thread and frame)
+            const char* nx = reinterpret_cast<const char*>(x1 + p.every_n) + (size_t)tid * 128;
+            asm volatile("prefetch.global.L2 [%0];" ::"l"(nx));
+            if (a + 3 < a1) asm volatile("prefetch.global.L2 [%0];" ::"l"(nx + (size_t)p.every_n * 8));
+        }
 #pragma unroll
-            for (int r = 0; r < 16; r++) {
-                const float2 s0 = __ldg(x0 + tid + r * T);
-                const float2 s1 = two ? __ldg(x1 + tid + r * T) : make_float2(0.f, 0.f);
-                const float w = __ldg(p.window + tid + r * T);
-                v[r].re = __fmul2_rn(make_float2(s0.x, s1.x), OWRX_P2(w));
-                v[r].im = __fmul2_rn(make_float2(s0.y, s1.y), OWRX_P2(w));
-            }
-        } else {
-            const float2* x0 = p.src + (frame * p.r0 + k1) * (long long)M;
-            const float2* x1 = x0 + (long long)p.r0 * M;
-#pragma unroll
-            for (int r = 0; r < 16; r++) {
-                const float2 s0 = __ldg(x0 + tid + r * T);
-                const float2 s1 = two ? __ldg(x1 + tid + r * T) : make_float2(0.f, 0.f);
-                v[r].re = make_float2(s0.x, s1.x);
-                v[r].im = make_float2(s0.y, s1.y);
-            }
+        for (int r = 0; r < 16; r++) {
+            const float2 s0 = __ldg(x0 + tid + r * T);
+            const float2 s1 = two ? __ldg(x1 + tid + r * T) : make_float2(0.f, 0.f);
+            const float w = __ldg(p.window + tid + r * T);
+            v[r].re = __fmul2_rn(make_float2(s0.x, s1.x), OWRX_P2(w));
+            v[r].im = __fmul2_rn(make_float2(s0.y, s1.y), OWRX_P2(w));
         }
         // pass 1: radix 16, Ns = 1
         c2dft16(v);
@@ -327,9 +301,9 @@ wf_fft2_kernel(WfFftParams p)
             acc[q] += pw.x + pw.y;
         }
     }
-    float* out = p.partial + ((size_t)line * p.subsets + subset) * (size_t)p.n;
+    float* out = p.partial + ((size_t)line * p.subsets + subset) * (size_t)M;
 #pragma unroll
-    for (int q = 0; q < 16; q++) out[(size_t)k1 + (size_t)p.r0 * (tid + slot<16>(q) * 256)] = acc[q];
+    for (int q = 0; q < 16; q++) out[tid + slot<16>(q) * 256] = acc[q];
     __syncthreads();                                        // s_next is visible; every read of the shared buffer is done
     cur = s_next;
     }
@@ -513,40 +487,6 @@ wf_big_kernel(WfBigParams p)
     cluster_sync_all();                                     // no CTA of the cluster exits while another may still arrive
 }
 
-struct WfColParams {
-    const float2* iq;
-    const float* window;
-    const float2* twn;      // [R0][M] exp(-2 pi i k1 n2 / N)
-    float2* y;              // [frame][R0][M]
-    int every_n;
-    long long first_frame;
-};
-
-template <int R0>
-__global__ void __launch_bounds__(256) wf_colpass_kernel(WfColParams p)
-{
-    constexpr int M = 4096;
-    const int n2 = blockIdx.x * 256 + threadIdx.x;
-    const long long f = blockIdx.y;
-    const float2* x = p.iq + (p.first_frame + f) * (long long)p.every_n;
-    float2 v[R0];
-#pragma unroll
-    for (int n1 = 0; n1 < R0; n1++) {
-        float2 s = __ldg(x + n2 + M * n1);
-        float w = __ldg(p.window + n2 + M * n1);
-        v[n1] = make_float2(s.x * w, s.y * w);
-    }
-    dft<R0>(v);
-    float2* y = p.y + f * (long long)(R0 * M);
-#pragma unroll
-    for (int q = 0; q < R0; q++) {
-        const int k1 = slot<R0>(q);
-        float2 o = v[q];
-        if (k1 > 0) o = cmul(o, __ldg(p.twn + k1 * M + n2));
-        y[k1 * M + n2] = o;
-    }
-}
-
 // Spectral-subtraction noise filter (BASELINE config 4: "65536-pt high-zoom waterfall ... with spectral-subtraction noise
 // filter").  SPEC-DEFINED — the reference has no waterfall noise filter (SURVEY 8d C4); same arithmetic as the oracle's
 // oc_wf_noise_filter.  One thread per bin walks the lines of the batch in order (the floor estimate is a recurrence across
@@ -700,7 +640,6 @@ struct owrx_wf {
     int* d_counter = nullptr;                                  // work counter of the persistent FFT kernel
     float4* d_ybig = nullptr; size_t ybig_cap = 0;            // wf_big_kernel: per-cluster row scratch (L2-resident)
     int big_clusters = 0;                                      // clusters of the fused kernel the device keeps resident
-    float2* d_y = nullptr;      size_t y_cap = 0;
     int16_t* d_s16 = nullptr;   size_t s16_cap = 0;
     // pipelined mode: the (latency-bound, one warp per 32 lines) ADPCM pass of batch i runs on a high-priority side
     // stream beside the FFT pass of batch i+1; the int16 scratch is double-buffered
@@ -746,33 +685,26 @@ template <typename T> static int grow(T** ptr, size_t* cap, size_t need)
     return OWRX_OK;
 }
 
-template <int LOG2M, bool FROM_IQ> static int launch_fft(const WfFftParams& p, size_t units, cudaStream_t st)
+template <int LOG2M> static int launch_fft(const WfFftParams& p, size_t units, cudaStream_t st)
 {
     constexpr int M = 1 << LOG2M;
     constexpr int threads = M / 16 < 32 ? 32 : M / 16;
     const size_t smem = 2 * (size_t)(M + M / 16) * sizeof(float2) + (size_t)M * sizeof(float);
-    OWRX_CUDA(cudaFuncSetAttribute(wf_fft_kernel<LOG2M, FROM_IQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    wf_fft_kernel<LOG2M, FROM_IQ><<<(unsigned)units, threads, smem, st>>>(p);
+    OWRX_CUDA(cudaFuncSetAttribute(wf_fft_kernel<LOG2M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    wf_fft_kernel<LOG2M><<<(unsigned)units, threads, smem, st>>>(p);
     OWRX_LAUNCH_CHECK();
     return OWRX_OK;
 }
 
-template <bool FROM_IQ> static int launch_fft2(const WfFftParams& p, size_t units, int sm_count, cudaStream_t st)
+static int launch_fft2(const WfFftParams& p, size_t units, int sm_count, cudaStream_t st)
 {
     const size_t smem = (size_t)(4096 + 4096 / 16) * sizeof(float4);
-    OWRX_CUDA(cudaFuncSetAttribute(wf_fft2_kernel<FROM_IQ>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    OWRX_CUDA(cudaFuncSetAttribute(wf_fft2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     OWRX_CUDA(cudaMemsetAsync(p.counter, 0, sizeof(int), st));
     const unsigned grid = (unsigned)std::min<size_t>(units, (size_t)2 * sm_count);       // 2 CTAs per SM (128 registers, 70 KB)
-    wf_fft2_kernel<FROM_IQ><<<grid, 256, smem, st>>>(p);
+    wf_fft2_kernel<<<grid, 256, smem, st>>>(p);
     OWRX_LAUNCH_CHECK();
     return OWRX_OK;
-}
-
-// OWRX_WF_SCALAR=1 keeps the one-frame-per-pass scalar kernel for the 4096-point rows (A/B runs)
-static bool wf_use_packed()
-{
-    static const bool scalar = getenv("OWRX_WF_SCALAR") && atoi(getenv("OWRX_WF_SCALAR")) != 0;
-    return !scalar;
 }
 
 // the fused four-step kernel: clusters of R0 / 2 CTAs, as many clusters as the device keeps resident at once
@@ -811,59 +743,50 @@ template <int R0> static int launch_big(owrx_wf* wf, WfBigParams& p, cudaStream_
     return OWRX_OK;
 }
 
-// OWRX_WF_FUSED=0 keeps the two-kernel four-step path (column pass to an HBM scratch, then the row kernel) for A/B runs
-static bool wf_use_fused()
-{
-    static const bool off = getenv("OWRX_WF_FUSED") && atoi(getenv("OWRX_WF_FUSED")) == 0;
-    return !off && wf_use_packed();
-}
-
-static int wf_run_chunk(owrx_wf* wf, const float2* iq_dev, long long first_frame, size_t lines, uint8_t* out_dev,
-                        float* db_dev, int16_t* s16_dev, cudaStream_t st)
+static int wf_run_lines(owrx_wf* wf, const float2* iq_dev, size_t lines, uint8_t* out_dev, float* db_dev, int16_t* s16_dev,
+                        cudaStream_t st)
 {
     const int fpl = wf->avg > 0 ? wf->avg : 1;
     const int n = wf->n;
-    // frame subsets: enough CTAs to cover the SMs twice when few lines are in flight
     int subsets = 1;
-    const size_t base_units = lines * (size_t)wf->r0;
-    if (base_units < (size_t)2 * wf->sm_count)
-        subsets = (int)std::min<size_t>((size_t)std::min(fpl, 8), ((size_t)2 * wf->sm_count + base_units - 1) / base_units);
-    // the persistent packed kernel balances through its work counter: aim at ~8 units per resident CTA, each of at least
-    // 8 frame pairs (a subset costs one more partial-sum row for wf_finalize_kernel to add)
-    if (wf->m == 4096 && wf_use_packed() && base_units < (size_t)16 * wf->sm_count)
-        subsets = (int)std::max<size_t>(subsets, std::min<size_t>((size_t)std::max(1, std::min(fpl / 16, 8)),
-                                                                  ((size_t)16 * wf->sm_count + base_units - 1) / base_units));
-    if (wf->r0 > 1 && wf_use_fused()) {
+    if (wf->r0 > 1) {
         // fused four-step kernel: units are (line, subset), dealt round-robin to ~2 sm_count / r0 clusters
         const size_t clusters = std::max<size_t>(1, (size_t)2 * wf->sm_count / (size_t)wf->r0);
         subsets = (int)std::min<size_t>((size_t)std::max(1, std::min(fpl / 12, 8)), std::max<size_t>(1, (8 * clusters + lines - 1) / lines));
+    } else {
+        // frame subsets: enough CTAs to cover the SMs twice when few lines are in flight
+        if (lines < (size_t)2 * wf->sm_count)
+            subsets = (int)std::min<size_t>((size_t)std::min(fpl, 8), ((size_t)2 * wf->sm_count + lines - 1) / lines);
+        // the persistent packed kernel balances through its work counter: aim at ~8 units per resident CTA, each of at least
+        // 8 frame pairs (a subset costs one more partial-sum row for wf_finalize_kernel to add)
+        if (wf->m == 4096 && lines < (size_t)16 * wf->sm_count)
+            subsets = (int)std::max<size_t>(subsets, std::min<size_t>((size_t)std::max(1, std::min(fpl / 16, 8)),
+                                                                      ((size_t)16 * wf->sm_count + lines - 1) / lines));
     }
     int rc;
     if ((rc = grow(&wf->d_partial, &wf->partial_cap, lines * (size_t)subsets * (size_t)n)) != OWRX_OK) return rc;
-
-    WfFftParams p;
-    p.window = wf->d_window; p.tw2 = wf->d_tw2; p.tw3 = wf->d_tw3; p.partial = wf->d_partial;
-    p.every_n = wf->every_n; p.frames_per_line = fpl; p.subsets = subsets; p.r0 = wf->r0; p.n = n;
-    const size_t units = lines * (size_t)wf->r0 * (size_t)subsets;
+    const size_t units = lines * (size_t)subsets;
     if (units > (size_t)0x7fffffff) return fail(OWRX_E_INVALID, "batch too large");
-    p.units = (int)units; p.counter = wf->d_counter;
 
     if (wf->r0 == 1) {
-        p.src = iq_dev; p.first_frame = first_frame;
+        WfFftParams p;
+        p.src = iq_dev; p.window = wf->d_window; p.tw2 = wf->d_tw2; p.tw3 = wf->d_tw3; p.partial = wf->d_partial;
+        p.every_n = wf->every_n; p.frames_per_line = fpl; p.subsets = subsets; p.first_frame = 0;
+        p.units = (int)units; p.counter = wf->d_counter;
         switch (wf->log2m) {
-        case 8:  rc = launch_fft<8, true>(p, units, st); break;
-        case 9:  rc = launch_fft<9, true>(p, units, st); break;
-        case 10: rc = launch_fft<10, true>(p, units, st); break;
-        case 11: rc = launch_fft<11, true>(p, units, st); break;
-        case 12: rc = wf_use_packed() ? launch_fft2<true>(p, units, wf->sm_count, st) : launch_fft<12, true>(p, units, st); break;
+        case 8:  rc = launch_fft<8>(p, units, st); break;
+        case 9:  rc = launch_fft<9>(p, units, st); break;
+        case 10: rc = launch_fft<10>(p, units, st); break;
+        case 11: rc = launch_fft<11>(p, units, st); break;
+        case 12: rc = launch_fft2(p, units, wf->sm_count, st); break;
         default: return fail(OWRX_E_INVALID, "unsupported fft size");
         }
         if (rc != OWRX_OK) return rc;
-    } else if (wf_use_fused()) {
+    } else {
         WfBigParams b;
         b.iq = iq_dev; b.window = wf->d_window; b.twn = wf->d_twn; b.tw2 = wf->d_tw2; b.tw3 = wf->d_tw3; b.y = nullptr;
         b.partial = wf->d_partial; b.every_n = wf->every_n; b.frames_per_line = fpl; b.subsets = subsets; b.n = n;
-        b.units = (int)(lines * (size_t)subsets); b.first_frame = first_frame;
+        b.units = (int)units; b.first_frame = 0;
         switch (wf->r0) {
         case 2:  rc = launch_big<2>(wf, b, st); break;
         case 4:  rc = launch_big<4>(wf, b, st); break;
@@ -872,27 +795,10 @@ static int wf_run_chunk(owrx_wf* wf, const float2* iq_dev, long long first_frame
         default: return fail(OWRX_E_INVALID, "unsupported fft size");
         }
         if (rc != OWRX_OK) return rc;
-    } else {
-        const size_t frames = lines * (size_t)fpl;
-        if ((rc = grow(&wf->d_y, &wf->y_cap, frames * (size_t)n)) != OWRX_OK) return rc;
-        WfColParams c;
-        c.iq = iq_dev; c.window = wf->d_window; c.twn = wf->d_twn; c.y = wf->d_y; c.every_n = wf->every_n;
-        c.first_frame = first_frame;
-        dim3 grid(4096 / 256, (unsigned)frames);
-        switch (wf->r0) {
-        case 2:  wf_colpass_kernel<2><<<grid, 256, 0, st>>>(c); break;
-        case 4:  wf_colpass_kernel<4><<<grid, 256, 0, st>>>(c); break;
-        case 8:  wf_colpass_kernel<8><<<grid, 256, 0, st>>>(c); break;
-        case 16: wf_colpass_kernel<16><<<grid, 256, 0, st>>>(c); break;
-        default: return fail(OWRX_E_INVALID, "unsupported fft size");
-        }
-        OWRX_LAUNCH_CHECK();
-        p.src = wf->d_y; p.first_frame = 0;
-        if ((rc = wf_use_packed() ? launch_fft2<false>(p, units, wf->sm_count, st) : launch_fft<12, false>(p, units, st)) != OWRX_OK) return rc;
     }
 
-    // finalize: log / swap / quantise.  The ADPCM encoder runs once per batch (wf_process), not per chunk:
-    // its run time is the serial latency of ONE line however many lines are in flight.
+    // finalize: log / swap / quantise.  The ADPCM encoder runs once per batch (wf_process), not here: its run time is the
+    // serial latency of ONE line however many lines are in flight.
     const bool adpcm = wf->compression == OWRX_COMPRESSION_ADPCM;
     float* db = db_dev;
     if (!adpcm && out_dev) db = (float*)out_dev;   // compression "none": the line IS the float32 dB row
@@ -919,16 +825,6 @@ static int wf_process(owrx_wf* wf, const float2* iq_dev, size_t n_samples, uint8
     const size_t lines = wf_lines_for(wf, n_samples);
     const size_t lb = wf_line_bytes(wf);
     if (out_dev && lines * lb > out_cap) return fail(OWRX_E_OVERFLOW, "output buffer too small: need %zu bytes", lines * lb);
-    const int fpl = wf->avg > 0 ? wf->avg : 1;
-    // chunk so that the four-step scratch stays bounded (<= 256 MiB; measured: an L2-sized scratch is no faster) and
-    // grid.y <= 65535
-    size_t chunk = lines;
-    if (wf->r0 > 1 && !wf_use_fused()) {
-        const size_t per_line = (size_t)fpl * (size_t)wf->n * sizeof(float2);
-        static const size_t y_budget = (size_t)(getenv("OWRX_WF_Y_MB") ? atoi(getenv("OWRX_WF_Y_MB")) : 256) << 20;
-        chunk = std::max<size_t>(1, y_budget / per_line);
-        chunk = std::min(chunk, (size_t)65535 / (size_t)fpl > 0 ? (size_t)65535 / (size_t)fpl : 1);
-    }
     const bool adpcm = wf->compression == OWRX_COMPRESSION_ADPCM;
     const int n = wf->n;
     int16_t* s16 = s16_dev;
@@ -946,13 +842,7 @@ static int wf_process(owrx_wf* wf, const float2* iq_dev, size_t n_samples, uint8
             return rc;
         s16 = alt ? wf->d_s16_alt : wf->d_s16;
     }
-    for (size_t l0 = 0; l0 < lines; l0 += chunk) {
-        const size_t lc = std::min(chunk, lines - l0);
-        rc = wf_run_chunk(wf, iq_dev, (long long)l0 * fpl, lc, out_dev ? out_dev + l0 * lb : nullptr,
-                          db_dev ? db_dev + l0 * (size_t)wf->n : nullptr,
-                          s16 ? s16 + l0 * (size_t)(wf->n + 10) : nullptr, st);
-        if (rc != OWRX_OK) return rc;
-    }
+    if (lines && (rc = wf_run_lines(wf, iq_dev, lines, out_dev, db_dev, s16, st)) != OWRX_OK) return rc;
     if (adpcm && out_dev && lines) {
         cudaStream_t sa = st;
         if (side_adpcm) {
@@ -1057,7 +947,7 @@ void owrx_wf_destroy(owrx_wf_t* wf)
     if (wf->stream) cudaStreamSynchronize(wf->stream);
     cudaFree(wf->d_window); cudaFree(wf->d_tw2); cudaFree(wf->d_tw3); cudaFree(wf->d_twn); cudaFree(wf->d_counter); cudaFree(wf->d_ybig);
     cudaDeviceSynchronize();
-    cudaFree(wf->d_partial); cudaFree(wf->d_y); cudaFree(wf->d_s16); cudaFree(wf->d_s16_alt);
+    cudaFree(wf->d_partial); cudaFree(wf->d_s16); cudaFree(wf->d_s16_alt);
     if (wf->fin_done) cudaEventDestroy(wf->fin_done);
     if (wf->adpcm_done[0]) cudaEventDestroy(wf->adpcm_done[0]);
     if (wf->adpcm_done[1]) cudaEventDestroy(wf->adpcm_done[1]);

@@ -90,7 +90,7 @@ def test_c2_full_block_against_the_oracle(gpu, monkeypatch):
     pick = sorted({int(order[0]), int(order[1]), int(order[31]), int(order[32]), int(order[-2]), int(order[-1])})
     refs = dict(zip(pick, _oracle_many(iq, fs, out, [cars[i] for i in pick])))
     monkeypatch.delenv("OWRX_FC_TC_FMT", raising=False)
-    for mode, env in (("auto", {}), ("auto", {"OWRX_FC_TC_KC": "32"}), ("auto", {"OWRX_FC_TC_FMT": "f16x2"}), ("fastconv", {}), ("direct", {})):
+    for mode, env in (("auto", {}), ("auto", {"OWRX_FC_TC_FMT": "f16x2"}), ("fastconv", {}), ("direct", {})):
         with monkeypatch.context() as mp:
             for k, v in env.items():
                 mp.setenv(k, v)
@@ -149,11 +149,10 @@ def test_c3_shape_128_channels_in_one_group_every_form(gpu, monkeypatch):
     oracle_vs_f64 = max(rel_rms(refs[i]["if_"], truth[i]) for i in weakest)
     monkeypatch.delenv("OWRX_FC_M", raising=False)
     monkeypatch.delenv("OWRX_FC_TC_FORM", raising=False)
-    monkeypatch.delenv("OWRX_FC_TCT_KC", raising=False)
     monkeypatch.delenv("OWRX_FC_TC_FMT", raising=False)
     for mode, env in (("auto", {}), ("fastconv_tc", {"OWRX_FC_TC_FORM": "0"}), ("fastconv_tc", {"OWRX_FC_M": "256"}),
-                      ("fastconv_tc", {"OWRX_FC_M": "256", "OWRX_FC_TC_FORM": "0"}), ("fastconv_tc", {"OWRX_FC_TCT_KC": "32"}),
-                      ("fastconv_tc", {"OWRX_FC_TC_FMT": "bf16x3"}), ("fastconv", {})):
+                      ("fastconv_tc", {"OWRX_FC_M": "256", "OWRX_FC_TC_FORM": "0"}), ("fastconv_tc", {"OWRX_FC_TC_FMT": "bf16x3"}),
+                      ("fastconv", {})):
         with monkeypatch.context() as mp:
             for k, v in env.items():
                 mp.setenv(k, v)

@@ -31,7 +31,7 @@ def fir_mode(request, monkeypatch):
     M (fc_contract_tct_kernel: what the cost model picks for groups of >= 128 slots and short passes) — with both branch FFT
     sizes (256 points; 64 points: the default of groups with D >= 2048) and both operand splits (block-scaled fp16 x 2: the
     default; bf16 x 3)
-    (owrx_bank_create reads OWRX_FIR_MODE, a new group OWRX_FC_M and OWRX_FC_TC_FMT, fc_launch_contract_tc OWRX_FC_TC_FORM per launch)"""
+    (owrx_bank_create reads every one of these variables: a bank keeps the forms of the environment it was created in)"""
     mode, form, m, fmt = _FORMS[request.param]
     monkeypatch.setenv("OWRX_FIR_MODE", str(N.FIR_MODES[mode]))
     monkeypatch.setenv("OWRX_FC_TC_FORM", form)
@@ -407,18 +407,17 @@ def test_deferred_drain_streams_the_same_outputs(gpu):
     assert got[True][2] == got[False][2] and len(got[True][2]) > 1000
 
 
-def test_fused_tail_and_warp_agc_equal_the_reference_kernels(gpu, monkeypatch):
-    """round 2 kernels against the round 1 evaluation they replace, bit for bit: tail_front_kernel (Squelch + demodulator front +
-    DcBlock means in one launch, gate from local block powers) vs the seven-kernel tail, and agc_warp_kernel (one warp per
-    channel, no CTA barrier) vs the 8-channel-CTA Agc — ragged streaming feeds, a squelched channel, all three demodulators"""
+def test_fused_tail_equals_the_seven_kernel_tail(gpu, monkeypatch):
+    """tail_front_kernel (Squelch + demodulator front + DcBlock means in one launch, gate from local block powers) against the
+    seven-kernel low-rate tail it replaces for short squelch blocks, bit for bit — ragged streaming feeds, a squelched channel,
+    all three demodulators"""
     fs, out = 2.4e6, 12000
     cars = carrier_plan(7, fs, seed=61)
     iq = make_iq(5333 + 200 * (750 * 9 + 123), fs, cars, seed=61)
     iq[200 * 750 * 3:200 * 750 * 6] *= 1e-4                       # a quiet stretch: squelched channels close and reopen
 
-    def run(tail_fused, agc_cta):
+    def run(tail_fused):
         monkeypatch.setenv("OWRX_TAIL_FUSED", "1" if tail_fused else "0")
-        monkeypatch.setenv("OWRX_AGC_CTA", "1" if agc_cta else "0")
         bank = ChannelBank(fs, outputs=N.OUT_AUDIO | N.OUT_DEMOD | N.OUT_POWER)
         chans = [bank.add_channel(out, demod=c["kind"], offset=c["offset"], bandpass=BANDPASS[c["kind"]]) for c in cars]
         for ch, c in zip(chans[:4], cars):
@@ -431,8 +430,8 @@ def test_fused_tail_and_warp_agc_equal_the_reference_kernels(gpu, monkeypatch):
         bank.close()
         return res
 
-    ref = run(False, True)
-    new = run(True, False)
+    ref = run(False)
+    new = run(True)
     assert len(ref[0][0]) >= 750 * 8
     for (d0, a0, p0), (d1, a1, p1) in zip(ref, new):
         assert np.array_equal(d0, d1) and np.array_equal(a0, a1) and np.array_equal(p0, p1)

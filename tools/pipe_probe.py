@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Stage times of the C2 device path with the three-stream pipeline on and off (each stage's own CUDA-event bracket):
 off = every stage alone on the GPU, on = what the stages cost while they overlap.  One JSON line per run; the environment
-selects the kernel variants (OWRX_AGC_CTA, OWRX_TAIL_FUSED, OWRX_AGCW_PAD_KB, ...), so A/B runs are separate invocations."""
+selects the kernel variants (OWRX_TAIL_FUSED, OWRX_AGC_PAD_KB, ...), so A/B runs are separate invocations."""
 import json
 import os
 import sys

@@ -3,8 +3,7 @@
   wf_probe.py c1 [lines]     2.4 MS/s, 4096-pt, 9 fps   (avg 93, hop 2867)        default 592 lines
   wf_probe.py c4 [lines]     61.44 MS/s, 65536-pt, 30 fps (avg 45, hop 45511)      default 128 lines
 Reports the whole chain with ADPCM (pipelined side-stream encoder) and with compression "none" (FFT + finalize only),
-each as ms per batch, lines/s and the fraction of the measured HBM peak on SURVEY 8(d)'s algorithmic bytes (8 U + out per line).
-OWRX_WF_SCALAR=1 selects the one-frame-per-pass scalar FFT kernel for A/B runs."""
+each as ms per batch, lines/s and the fraction of the measured HBM peak on SURVEY 8(d)'s algorithmic bytes (8 U + out per line)."""
 import json
 import os
 import sys
@@ -31,8 +30,7 @@ def run(which, lines, steps=5):
     iq[:, 0] += 0.3 * torch.cos(0.7 * tt); iq[:, 1] += 0.3 * torch.sin(0.7 * tt)
     del tt
     st = torch.cuda.Stream(device=dev)
-    out = {"shape": which, "lines": lines, "avg": avg, "every_n": every_n, "input_GB": ns * 8 / 1e9,
-           "fft_kernel": "scalar" if os.environ.get("OWRX_WF_SCALAR") else "packed two-frame"}
+    out = {"shape": which, "lines": lines, "avg": avg, "every_n": every_n, "input_GB": ns * 8 / 1e9}
     for comp in ("adpcm", "none"):
         wf = Waterfall(fs, n, ov, fps, comp, device=0)
         buf = torch.empty(lines * wf.line_bytes, dtype=torch.uint8, device=dev)
