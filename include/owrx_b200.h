@@ -232,6 +232,21 @@ int owrx_chan_read_message(owrx_bank_t* bank, int chan, int type_byte, void* out
 #define OWRX_OUT_IF    4
 #define OWRX_OUT_POWER 8
 int owrx_bank_set_outputs(owrx_bank_t* bank, int mask);
+/* WFM multiplex tap.  The reference's WFm chain writes its Limit output (FmDemod + Limit at the IF rate, before the audio
+ * FractionalDecimator) into a tap buffer of its own, metaTapBuffer (csdr/chain/analog.py:62,73-76); the RDS path reads it
+ * through Convert(Format.FLOAT, Format.SHORT) into redsea.  owrx_chan_set_mpx delivers that signal per channel:
+ *   OWRX_MPX_F32  the limited discriminator output, float32 (what metaTapBuffer carries)
+ *   OWRX_MPX_S16  the same after Convert(FLOAT, SHORT): int16 little-endian, x * 32767 truncated toward zero
+ * WFM channels only (OWRX_E_INVALID otherwise).  Like every setter it takes effect at the next block boundary; a format change
+ * discards queued samples of the old format, and re-moding the channel away from WFM turns the tap off.  Every drain path
+ * (owrx_bank_feed*, deferred drain, owrx_bank_drain, owrx_bank_drain_begin / _end) queues the samples, in order;
+ * owrx_chan_read_mpx pops up to cap_bytes of whole samples.  A channel id handed out again never receives samples of the
+ * client that held it before. */
+#define OWRX_MPX_OFF 0
+#define OWRX_MPX_F32 1
+#define OWRX_MPX_S16 2
+int owrx_chan_set_mpx(owrx_bank_t* bank, int chan, int format);
+int owrx_chan_read_mpx(owrx_bank_t* bank, int chan, void* out, size_t cap_bytes, size_t* n_bytes);
 
 /* Device-resident batch path (bench / embedding): process one wideband block that already lives
  * in device memory; outputs stay on the device and are NOT queued for the host.
@@ -255,7 +270,8 @@ int owrx_bank_drain(owrx_bank_t* bank);
  * owrx_bank_process_device block behind that block's kernels and returns; the caller may issue the NEXT
  * owrx_bank_process_device before _end, which waits for the copies and fills the queues exactly as owrx_bank_drain would
  * have.  One drain in flight at a time (_begin before the previous _end is OWRX_E_INVALID); _end without _begin is a
- * no-op.  When S-meter power reports (OWRX_OUT_POWER) or a client-audio format are enabled, _begin drains synchronously. */
+ * no-op.  When S-meter power reports (OWRX_OUT_POWER) or a client-audio format are enabled, _begin drains synchronously.
+ * The multiplex tap (owrx_chan_set_mpx) goes asynchronously like the other outputs. */
 int owrx_bank_drain_begin(owrx_bank_t* bank);
 int owrx_bank_drain_end(owrx_bank_t* bank);
 /* samples of audio produced per channel by the last owrx_bank_process_device call */

@@ -32,6 +32,7 @@ class Channel:
         self.outputRate = output_rate
         self.frequencyOffset = 0
         self.bandpassCutoffs = [None, None]
+        self._mpx = "off"
 
     def setFrequencyOffset(self, offset):            # csdr/chain/selector.py:132-140
         self.frequencyOffset = offset
@@ -52,6 +53,8 @@ class Channel:
         k = _KINDS[kind] if isinstance(kind, str) else int(kind)
         prof = N.AGC_FAST if str(agc_profile).lower() == "fast" else N.AGC_SLOW
         N.check(N.lib.owrx_chan_set_demod(self.bank._h, self.id, k, float(audio_rate), float(tau), prof))
+        if k != N.DEMOD_WFM:
+            self._mpx = "off"                        # the library turns the tap off with the WFm chain
 
     def _read(self, fn, width=1):
         chunks = []
@@ -87,6 +90,29 @@ class Channel:
                 break
             chunks.append(buf[:n.value].copy())
         return np.concatenate(chunks) if chunks else np.empty(0, np.uint8)
+
+    def set_mpx(self, fmt):
+        """WFM multiplex tap (the WFm chain's Limit output, csdr/chain/analog.py:62,73-76): "off" | "f32" | "s16" (after
+        Convert(FLOAT, SHORT), what the reference's RDS path feeds redsea).  WFM channels only (ValueError otherwise)."""
+        codes = {"off": N.MPX_OFF, "f32": N.MPX_F32, "s16": N.MPX_S16}
+        if fmt not in codes:
+            raise ValueError("unknown multiplex format %r (off | f32 | s16)" % (fmt,))
+        code = codes[fmt]
+        N.check(N.lib.owrx_chan_set_mpx(self.bank._h, self.id, code))
+        self._mpx = fmt
+
+    def read_mpx(self):
+        """queued multiplex samples: np.float32 ("f32") or np.int16 ("s16")"""
+        dtype = np.int16 if self._mpx == "s16" else np.float32
+        chunks = []
+        buf = np.empty(1 << 18, np.uint8)
+        while True:
+            n = C.c_size_t()
+            N.check(N.lib.owrx_chan_read_mpx(self.bank._h, self.id, buf.ctypes.data_as(C.c_void_p), buf.size, C.byref(n)))
+            if n.value == 0:
+                break
+            chunks.append(buf[:n.value].copy())
+        return (np.concatenate(chunks) if chunks else np.empty(0, np.uint8)).view(dtype)
 
     def read_audio(self):
         return self._read(N.lib.owrx_chan_read_audio)

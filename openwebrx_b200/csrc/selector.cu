@@ -229,9 +229,17 @@ struct Chan {
     owrx_chan_spec_t spec{};
     float agc_initial = 1.0f;
     int audio_fmt = OWRX_AUDIO_F32;
+    int mpx_fmt = OWRX_MPX_OFF;
+    unsigned long long gen = 0;            // bank-unique: tells this client from a later one that gets the same id
     FQ q_audio, q_demod, q_if, q_power;
-    std::vector<unsigned char> q_bytes;
+    std::vector<unsigned char> q_bytes, q_mpx;
     size_t last_audio = 0;
+};
+
+// one tapped channel of a block (owrx_chan_set_mpx): where its run sits in the staging region and whom it belongs to
+struct MpxRun {
+    int chan, fmt, run;
+    unsigned long long gen;
 };
 
 struct Group {
@@ -308,6 +316,15 @@ struct Group {
     void* d_fc_tabp = nullptr; void* d_fc_Fp = nullptr; size_t fc_blocks_cap_tc = 0;
     std::vector<double> fc_tabp_rate;
     std::vector<float> fc_taps;                      // h[t] rounded to float (same values K3 uses)
+    // WFM multiplex tap (mpx_gather_kernel): the tapped slots of the block being issued (rebuilt at every block boundary) and
+    // a staging region per block parity of mpx_cap rows per run; the split-phase drain's copy of a region is awaited through
+    // mpx_drained before the region is written again
+    std::vector<MpxRun> mpx_runs;
+    int mpx_nf = 0, mpx_ns = 0;
+    unsigned char* d_mpx[2] = {nullptr, nullptr};
+    size_t mpx_cap = 0, mpx_bytes = 0;
+    size_t mpx_rows = 0;                             // rows gathered in this feed
+    cudaEvent_t mpx_drained[2] = {nullptr, nullptr};
 };
 
 }  // namespace
@@ -319,6 +336,7 @@ struct owrx_bank {
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     std::mutex mu;
     std::vector<std::unique_ptr<Chan>> chans;
+    unsigned long long chan_gen = 0;                 // Chan::gen of the latest client
     std::vector<std::unique_ptr<Group>> groups;
     int out_mask = OWRX_OUT_AUDIO;
     // streaming wideband buffer
@@ -331,9 +349,11 @@ struct owrx_bank {
     // split-phase drain of the device path (owrx_bank_drain_begin / _end): its own staging, so a synchronous drain in between
     // cannot clobber it; one item per (group, output) that is in flight
     struct AsyncDrainItem { int which, width; size_t n, off; std::vector<int> chans; };
+    struct AsyncMpxItem { size_t n, off; int nf; std::vector<MpxRun> runs; };     // off: floats into h_adrain
     float* h_adrain = nullptr; size_t h_adrain_cap = 0;
     float* d_adrain = nullptr; size_t d_adrain_cap = 0;
     std::vector<AsyncDrainItem> adrain_items;
+    std::vector<AsyncMpxItem> adrain_mpx;
     bool adrain_pending = false;
     cudaEvent_t adrain_done = nullptr;                         // the D2H copies have landed
     owrx_bank_stats_t stats{};
@@ -400,6 +420,10 @@ void group_release(Group* g)
     cudaFree(g->d_fc_h); cudaFree(g->d_fc_tab); cudaFree(g->d_fc_F); cudaFree(g->d_fc_Z); cudaFree(g->d_fc_slots); cudaFree(g->d_fc_rates);
     cudaFree(g->d_fc_scale);
     cudaFree(g->d_fc_tabp); cudaFree(g->d_fc_Fp);
+    for (int k = 0; k < 2; k++) {
+        cudaFree(g->d_mpx[k]);
+        if (g->mpx_drained[k]) cudaEventDestroy(g->mpx_drained[k]);
+    }
     g->s1.release(); g->s2.release(); g->s3.release(); g->f1.release(); g->f1p.release(); g->f1b.release(); g->f2.release(); g->f3.release();
 }
 
@@ -821,6 +845,23 @@ int apply_pending(owrx_bank* bank, Group* g, cudaStream_t st_fir, cudaStream_t s
         }
         g->bp_pending = false;
     }
+    if (g->wfm) {
+        // multiplex tap layout of this block: F32 runs, then S16 runs, in slot order (ChanCfg::mpx / mpx_run)
+        g->mpx_runs.clear();
+        g->mpx_nf = g->mpx_ns = 0;
+        for (int s = 0; s < S; s++) {
+            const int cid = g->slot_chan[(size_t)s];
+            const Chan* ch = cid >= 0 ? bank->chans[(size_t)cid].get() : nullptr;
+            const int fmt = ch ? ch->mpx_fmt : OWRX_MPX_OFF;
+            const int run = fmt == OWRX_MPX_F32 ? g->mpx_nf++ : (fmt == OWRX_MPX_S16 ? g->mpx_ns++ : 0);
+            ChanCfg& c = g->h_cfg[(size_t)s];
+            if (c.mpx != fmt || c.mpx_run != run) {
+                c.mpx = fmt; c.mpx_run = run;
+                g->cfg_stale[0] = g->cfg_stale[1] = true;
+            }
+            if (fmt != OWRX_MPX_OFF) g->mpx_runs.push_back(MpxRun{cid, fmt, run, ch->gen});
+        }
+    }
     // per-slot tables of this block's parity: a block still in flight on the other streams keeps reading the other copy
     g->d_cfg = g->d_cfg2[g->cur]; g->d_bp_en = g->d_bp_en2[g->cur]; g->d_tail_mode = g->d_tail_mode2[g->cur];
     if (g->cfg_stale[g->cur]) {
@@ -1210,6 +1251,18 @@ int group_tail(owrx_bank* bank, Group* g, cudaStream_t st)
         const long long f1_first = g->f1.abs_end;
         g->f1.appended(n4);
         g->sq_abs += (long long)n4;
+        if (g->wfm && !g->mpx_runs.empty()) {
+            // ---- multiplex tap: the tapped slots' new f1 rows -> their staging runs (on the stream that owns f1, before it rolls)
+            if (g->mpx_rows + n4 > g->mpx_cap) return fail(OWRX_E_STATE, "multiplex tap staging under-provisioned");
+            if (g->mpx_drained[g->cur]) OWRX_CUDA(cudaStreamWaitEvent(st, g->mpx_drained[g->cur], 0));
+            const long long r0 = (long long)g->mpx_rows;
+            const long long tiles = (r0 + (long long)n4 + MG_R - 1) / MG_R - r0 / MG_R;
+            mpx_gather_kernel<<<dim3((unsigned)(S / 32), (unsigned)std::min<long long>(tiles, 65535)), 256, 0, st>>>(
+                g->f1.row_abs(f1_first), S, (int)n4, g->d_cfg, r0, (long long)g->mpx_cap, g->mpx_nf, g->d_mpx[g->cur]);
+            OWRX_LAUNCH_CHECK();
+            bank->stats.kernel_launches++;
+            g->mpx_rows += n4;
+        }
 
         size_t n_audio = 0;
         if (!g->wfm) {
@@ -1400,6 +1453,19 @@ int group_begin_feed(owrx_bank* bank, Group* g, size_t rows, cudaStream_t st_fir
         }
         OWRX_CUDA(cudaMemsetAsync(g->d_tail_count, 0, (size_t)S * sizeof(int), st_serial));
     }
+    g->mpx_rows = 0;
+    if (!g->mpx_runs.empty()) {
+        // the multiplex staging follows the tap layout apply_pending has just rebuilt; f1 appends at most `low` rows per feed
+        const size_t cap = std::max(g->mpx_cap, (low + 7) / 8 * 8);
+        const size_t bytes = cap * (4 * (size_t)g->mpx_nf + 2 * (size_t)g->mpx_ns);
+        if (cap != g->mpx_cap || bytes > g->mpx_bytes) {
+            OWRX_CUDA(cudaDeviceSynchronize());
+            for (int k = 0; k < 2; k++) { cudaFree(g->d_mpx[k]); g->d_mpx[k] = nullptr; }
+            g->mpx_cap = g->mpx_bytes = 0;
+            for (int k = 0; k < 2; k++) OWRX_CUDA(cudaMalloc((void**)&g->d_mpx[k], bytes));
+            g->mpx_cap = cap; g->mpx_bytes = bytes;
+        }
+    }
     return OWRX_OK;
 }
 
@@ -1476,6 +1542,42 @@ int drain_tail(owrx_bank* bank, Group* g)
             ch->q_bytes.insert(ch->q_bytes.end(), hb + s * (size_t)g->tail_cap, hb + s * (size_t)g->tail_cap + hc[s]);
         }
     }
+    return OWRX_OK;
+}
+
+// multiplex tap: the D2H of a block's runs, packed as [F32 runs][S16 runs] of n rows each (at most two copies)
+int enqueue_mpx_copy(const Group* g, unsigned char* host, cudaStream_t ds)
+{
+    const size_t n = g->mpx_rows, nf = (size_t)g->mpx_nf, ns = (size_t)g->mpx_ns, cap = g->mpx_cap;
+    const unsigned char* d = g->d_mpx[g->cur];
+    if (nf) OWRX_CUDA(cudaMemcpy2DAsync(host, n * 4, d, cap * 4, n * 4, nf, cudaMemcpyDeviceToHost, ds));
+    if (ns) OWRX_CUDA(cudaMemcpy2DAsync(host + nf * n * 4, n * 2, d + nf * cap * 4, cap * 2, n * 2, ns, cudaMemcpyDeviceToHost, ds));
+    return OWRX_OK;
+}
+
+size_t mpx_packed_bytes(const Group* g) { return g->mpx_rows * (4 * (size_t)g->mpx_nf + 2 * (size_t)g->mpx_ns); }
+
+// packed runs -> per-channel queues; a run goes only to the client it was gathered for, in the format it was gathered in
+void deliver_mpx(owrx_bank* bank, const std::vector<MpxRun>& runs, size_t nf, size_t n, const unsigned char* host)
+{
+    for (const MpxRun& r : runs) {
+        if (r.chan < 0 || (size_t)r.chan >= bank->chans.size()) continue;
+        Chan* ch = bank->chans[(size_t)r.chan].get();
+        if (!ch || ch->gen != r.gen || ch->mpx_fmt != r.fmt) continue;
+        const unsigned char* src = r.fmt == OWRX_MPX_F32 ? host + (size_t)r.run * n * 4 : host + nf * n * 4 + (size_t)r.run * n * 2;
+        ch->q_mpx.insert(ch->q_mpx.end(), src, src + n * (r.fmt == OWRX_MPX_F32 ? 4 : 2));
+    }
+}
+
+int drain_mpx(owrx_bank* bank, Group* g, cudaStream_t ds)
+{
+    if (!g->mpx_rows || g->mpx_runs.empty()) return OWRX_OK;
+    int rc = ensure_stage(bank, (mpx_packed_bytes(g) + 3) / 4);
+    if (rc != OWRX_OK) return rc;
+    unsigned char* h = reinterpret_cast<unsigned char*>(bank->h_stage);
+    if ((rc = enqueue_mpx_copy(g, h, ds)) != OWRX_OK) return rc;
+    OWRX_CUDA(cudaStreamSynchronize(ds));
+    deliver_mpx(bank, g->mpx_runs, (size_t)g->mpx_nf, g->mpx_rows, h);
     return OWRX_OK;
 }
 
@@ -1584,6 +1686,7 @@ static int add_channel_spec(owrx_bank_t* bank, const owrx_chan_spec_t& sp, int* 
     size_t id = 0;
     while (id < bank->chans.size() && bank->chans[id]) id++;
     ch->id = (int)id;
+    ch->gen = ++bank->chan_gen;
     ch->spec = sp;
     agc_defaults(ch->cfg, sp.wfm ? OWRX_DEMOD_WFM : OWRX_DEMOD_NONE, OWRX_AGC_SLOW);
     Chan* raw = ch.get();
@@ -1709,6 +1812,7 @@ int owrx_chan_set_demod(owrx_bank_t* bank, int chan, int kind, double audio_rate
     ch->agc_initial = agc_initial_gain(kind);
     const bool wfm = kind == OWRX_DEMOD_WFM;
     if (wfm && !(audio_rate > 0.0 && tau > 0.0)) return fail(OWRX_E_INVALID, "WFM needs audio_rate and tau");
+    if (!wfm) { ch->mpx_fmt = OWRX_MPX_OFF; ch->q_mpx.clear(); }          // the multiplex tap is a WFm chain's
     owrx_chan_spec_t sp = ch->spec;
     sp.wfm = wfm ? 1 : 0;
     if (wfm) {
@@ -1803,6 +1907,37 @@ int owrx_chan_read_bytes(owrx_bank_t* bank, int chan, void* out, size_t cap_byte
     return OWRX_OK;
 }
 
+int owrx_chan_set_mpx(owrx_bank_t* bank, int chan, int format)
+{
+    if (!bank) return fail(OWRX_E_INVALID, "NULL bank");
+    if (format != OWRX_MPX_OFF && format != OWRX_MPX_F32 && format != OWRX_MPX_S16) return fail(OWRX_E_INVALID, "unknown multiplex format %d", format);
+    std::lock_guard<std::mutex> lk(bank->mu);
+    Chan* ch = get_chan(bank, chan);
+    if (!ch) return fail(OWRX_E_INVALID, "no such channel %d", chan);
+    if (format != OWRX_MPX_OFF && !ch->spec.wfm) return fail(OWRX_E_INVALID, "channel %d is not a WFM channel: it has no multiplex tap", chan);
+    if (bank->pending_final) { cudaSetDevice(bank->device); int rcp = finish_pending(bank); if (rcp != OWRX_OK) return rcp; }
+    if (format != ch->mpx_fmt) {
+        ch->q_mpx.clear();
+        ch->mpx_fmt = format;                        // the group's tap layout is rebuilt at the next block boundary
+    }
+    return OWRX_OK;
+}
+
+int owrx_chan_read_mpx(owrx_bank_t* bank, int chan, void* out, size_t cap_bytes, size_t* n_bytes)
+{
+    if (!bank || !out || !n_bytes) return fail(OWRX_E_INVALID, "bad argument");
+    std::lock_guard<std::mutex> lk(bank->mu);
+    Chan* ch = get_chan(bank, chan);
+    if (!ch) return fail(OWRX_E_INVALID, "no such channel %d", chan);
+    const size_t unit = ch->mpx_fmt == OWRX_MPX_S16 ? 2 : 4;
+    size_t take = std::min(cap_bytes, ch->q_mpx.size());
+    take -= take % unit;
+    memcpy(out, ch->q_mpx.data(), take);
+    ch->q_mpx.erase(ch->q_mpx.begin(), ch->q_mpx.begin() + (ptrdiff_t)take);
+    *n_bytes = take;
+    return OWRX_OK;
+}
+
 int owrx_chan_read_message(owrx_bank_t* bank, int chan, int type_byte, void* out, size_t cap_bytes, size_t* n)
 {
     if (!bank || !out || !n) return fail(OWRX_E_INVALID, "bad argument");
@@ -1842,6 +1977,7 @@ static int group_drain(owrx_bank* bank, Group* g, cudaStream_t ds, const DrainMa
         return rc;
     g->dr_audio = std::max(g->dr_audio, upto.audio);
     if (final && g->any_tail && g->tail_ran && g->last_audio && (rc = drain_tail(bank, g)) != OWRX_OK) return rc;
+    if (final && (rc = drain_mpx(bank, g, ds)) != OWRX_OK) return rc;
     if ((bank->out_mask & OWRX_OUT_DEMOD) && upto.demod > g->dr_demod &&
         (rc = drain_to_queues(bank, g, g->f2.rows(g->f2.fill - g->last_demod + g->dr_demod), upto.demod - g->dr_demod, 1, 1, ds)))
         return rc;
@@ -2252,7 +2388,18 @@ int owrx_bank_drain_begin(owrx_bank_t* bank)
             srcs.push_back(Src{o.rows, g->slots, o.buf});
         }
     }
-    if (bank->adrain_items.empty()) return OWRX_OK;
+    // the multiplex tap's packed runs land behind the transposed outputs in the same page-locked staging
+    const size_t total_xpose = total;
+    bank->adrain_mpx.clear();
+    std::vector<Group*> mpx_groups;
+    for (auto& gp : bank->groups) {
+        Group* g = gp.get();
+        if (!g || !g->mpx_rows || g->mpx_runs.empty()) continue;
+        bank->adrain_mpx.push_back(owrx_bank::AsyncMpxItem{g->mpx_rows, total, g->mpx_nf, g->mpx_runs});
+        mpx_groups.push_back(g);
+        total += (mpx_packed_bytes(g) + 3) / 4;
+    }
+    if (bank->adrain_items.empty() && bank->adrain_mpx.empty()) return OWRX_OK;
     if (total > bank->h_adrain_cap) {
         // (the previous drain has been ended: nothing is in flight on these buffers)
         OWRX_CUDA(cudaStreamSynchronize(bank->drain_stream));
@@ -2278,7 +2425,15 @@ int owrx_bank_drain_begin(owrx_bank_t* bank)
         int rcm = srcs[i].buf->mark_drained(ds);                      // the next writer of THIS buffer waits for the transpose
         if (rcm != OWRX_OK) return rcm;
     }
-    OWRX_CUDA(cudaMemcpyAsync(bank->h_adrain, bank->d_adrain, total * sizeof(float), cudaMemcpyDeviceToHost, ds));
+    if (total_xpose) OWRX_CUDA(cudaMemcpyAsync(bank->h_adrain, bank->d_adrain, total_xpose * sizeof(float), cudaMemcpyDeviceToHost, ds));
+    for (size_t i = 0; i < mpx_groups.size(); i++) {
+        Group* g = mpx_groups[i];
+        int rcm = enqueue_mpx_copy(g, reinterpret_cast<unsigned char*>(bank->h_adrain + bank->adrain_mpx[i].off), ds);
+        if (rcm != OWRX_OK) return rcm;
+        // the next gather into this parity's region waits for the copy
+        if (!g->mpx_drained[g->cur]) OWRX_CUDA(cudaEventCreateWithFlags(&g->mpx_drained[g->cur], cudaEventDisableTiming));
+        OWRX_CUDA(cudaEventRecord(g->mpx_drained[g->cur], ds));
+    }
     OWRX_CUDA(cudaEventRecord(bank->adrain_done, ds));
     bank->adrain_pending = true;
     return OWRX_OK;
@@ -2302,6 +2457,10 @@ int owrx_bank_drain_end(owrx_bank_t* bank)
         }
     }
     bank->adrain_items.clear();
+    // (the tap's runs carry their client's generation: a channel id reused since _begin gets nothing of the old client)
+    for (const auto& it : bank->adrain_mpx)
+        deliver_mpx(bank, it.runs, (size_t)it.nf, it.n, reinterpret_cast<const unsigned char*>(bank->h_adrain + it.off));
+    bank->adrain_mpx.clear();
     return OWRX_OK;
 }
 

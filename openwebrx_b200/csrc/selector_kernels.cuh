@@ -220,6 +220,8 @@ struct ChanCfg {
     int agc_hang_time;
     int active;
     float agc_thr;      // largest float a with fl(a / agc_ref) <= 1: "err > 1" <=> abs(v)*gain > agc_thr, exactly
+    int mpx;            // WFM multiplex tap: OWRX_MPX_OFF / _F32 / _S16 (mpx_gather_kernel)
+    int mpx_run;        // index of this slot's run among the group's tapped slots of the same format
 };
 
 // Squelch (SURVEY A.10).  Block power = mean |x|^2 over every `decim`-th sample.  CTA = (32 slots, one block): eight
@@ -1211,6 +1213,87 @@ audio_tail_kernel(const float* __restrict__ in, int slots, int n, const int* __r
             flush(b);
         }
         if (w == 1 && live && md != 0) count_out[s] = cnt;
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
+// WFM multiplex tap (csdr/chain/analog.py:62,73-76): the WFm chain writes its Limit output into a tap buffer that the audio
+// path and the RDS path (Convert(FLOAT, SHORT) -> redsea) both read.  Here that signal is f1, channel-minor at the IF rate.
+// The kernel copies the new rows of the tapped slots only, one contiguous run per channel in a staging region, so the D2H
+// moves just the tapped bytes (C5: 128 slots; copying all of f1 would be 512 B per IF sample):
+//   F32 runs first, run k at byte k * cap * 4;  then S16 runs, run k at byte n_f32 * cap * 4 + k * cap * 2
+// (cap is a multiple of 8: every run starts on 16 bytes).  This launch's rows land at rows [r0, r0 + n) of the runs.
+// CTA = 32 slots x tiles of MG_R destination rows: warps read 32-slot row segments (128-byte rows) into shared memory, then each
+// tapped slot's column leaves as 16-byte stores (F32: 4 rows per lane, all 32 lanes; S16: 8 rows per lane, 16 lanes), read from
+// shared memory in a per-lane rotated row order so that neither phase has bank conflicts.
+// S16 is Convert(FLOAT, SHORT) exactly as the client audio tail does it (SURVEY A.12).
+// ------------------------------------------------------------------------------------------------
+constexpr int MG_R = 128;
+__global__ void __launch_bounds__(256)
+mpx_gather_kernel(const float* __restrict__ in, int slots, int n, const ChanCfg* __restrict__ cfg, long long r0, long long cap,
+                  int n_f32, unsigned char* __restrict__ out)
+{
+    __shared__ float tile[MG_R][33];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int s0 = blockIdx.x * 32, s = s0 + lane;
+    const unsigned tapped = __ballot_sync(0xffffffffu, s < slots && cfg[s].mpx != 0);
+    if (!tapped) return;                                         // the same ballot in every warp: the whole CTA leaves
+    const long long t_first = r0 / MG_R, t_end = (r0 + n + MG_R - 1) / MG_R;
+    for (long long t = t_first + blockIdx.y; t < t_end; t += gridDim.y) {
+        const long long d0 = t * MG_R;                           // destination row of tile row 0
+        for (int j = w; j < MG_R; j += 8) {
+            const long long i = d0 + j - r0;
+            tile[j][lane] = (i >= 0 && i < n && s < slots) ? in[i * slots + s] : 0.f;
+        }
+        __syncthreads();
+        for (int l = w; l < 32; l += 8) {
+            if (!((tapped >> l) & 1u)) continue;
+            const ChanCfg c = cfg[s0 + l];
+            if (c.mpx == OWRX_MPX_F32) {
+                const long long d = d0 + 4 * lane;
+                float* o = reinterpret_cast<float*>(out + (size_t)c.mpx_run * cap * 4) + d;
+                // rows 4*lane + k sit 4*lane banks apart: each group of 8 lanes starts at another k (rot), so the 32 lanes of a read
+                // hit 32 different banks; the selects put the values back in row order
+                const int rot = lane >> 3;
+                float a[4], v[4];
+#pragma unroll
+                for (int kk = 0; kk < 4; kk++) a[kk] = tile[4 * lane + ((kk + rot) & 3)][l];
+#pragma unroll
+                for (int k = 0; k < 4; k++) {
+                    const int i = (k - rot) & 3;
+                    v[k] = i == 0 ? a[0] : (i == 1 ? a[1] : (i == 2 ? a[2] : a[3]));
+                }
+                if (d >= r0 && d + 4 <= r0 + n) {
+                    *reinterpret_cast<float4*>(o) = make_float4(v[0], v[1], v[2], v[3]);
+                } else {
+#pragma unroll
+                    for (int k = 0; k < 4; k++)
+                        if (d + k >= r0 && d + k < r0 + n) o[k] = v[k];
+                }
+            } else if (lane < 16) {
+                const long long d = d0 + 8 * lane;
+                int16_t* o = reinterpret_cast<int16_t*>(out + (size_t)n_f32 * cap * 4 + (size_t)c.mpx_run * cap * 2) + d;
+                // the same bank rotation over 8 rows (lanes 0, 4, 8, 12 share banks without it); each converted sample goes straight
+                // to its 16-bit place in the two 64-bit halves of the 16-byte store
+                const int rot = 2 * (lane >> 2);
+                unsigned long long lo = 0ull, hi = 0ull;
+#pragma unroll
+                for (int kk = 0; kk < 8; kk++) {
+                    const int k = (kk + rot) & 7;
+                    const float x = tile[8 * lane + k][l] * 32767.0f;                   // Convert(FLOAT, SHORT), SURVEY A.12
+                    const int q = x > 32767.0f ? 32767 : (x < -32768.0f ? -32768 : __float2int_rz(x));
+                    const unsigned long long b = (unsigned long long)(uint16_t)q << (16 * (k & 3));
+                    if (k < 4) lo |= b; else hi |= b;
+                }
+                if (d >= r0 && d + 8 <= r0 + n) {
+                    *reinterpret_cast<uint4*>(o) = make_uint4((unsigned)lo, (unsigned)(lo >> 32), (unsigned)hi, (unsigned)(hi >> 32));
+                } else {
+                    for (int k = 0; k < 8; k++)
+                        if (d + k >= r0 && d + k < r0 + n) o[k] = (int16_t)(uint16_t)((k < 4 ? lo : hi) >> (16 * (k & 3)));
+                }
+            }
+        }
+        __syncthreads();
     }
 }
 

@@ -807,13 +807,105 @@ class TcpSource(Module):
             pass
 
 
+class ExecModule(Module):
+    """ExecModule(inFormat, outFormat, args, ...): pycsdr's base of the modules that run an external decoder process.  In
+    OpenWebRX+ the RDS decoder module (RedseaModule, fed by WFm.setMetaWriter through Convert(FLOAT, SHORT)) is described as
+    one of them; that base class and wiring have not been checked against OpenWebRX source in this project, so no lines are
+    cited.  The WFM tap works whether its consumer is an ExecModule or a Python module reading the Buffer.  This is a host
+    process, not DSP: one thread copies the reader into the child's stdin, one copies its stdout into the writer.  stop()
+    closes stdin, terminates the child and waits for it, so no process outlives the module."""
+
+    _STOP_WAIT_S = 5.0
+
+    def __init__(self, inFormat, outFormat, args, *rest, **kw):
+        import subprocess
+        self.IN, self.OUT = inFormat, outFormat
+        self._reader = None
+        self._writer = None
+        self._stopped = False
+        self._cond = threading.Condition()
+        self._proc = subprocess.Popen([str(a) for a in args], stdin=subprocess.PIPE, stdout=subprocess.PIPE)
+        self._threads = [threading.Thread(target=f, daemon=True, name="pycsdr-exec") for f in (self._pump_in, self._pump_out)]
+        for t in self._threads:
+            t.start()
+
+    def getInputFormat(self):
+        return self.IN
+
+    def getOutputFormat(self):
+        return self.OUT
+
+    def setReader(self, reader):
+        with self._cond:
+            old, self._reader = self._reader, reader
+            self._cond.notify_all()
+        if old is not None and old is not reader:
+            old.stop()                             # the module's previous cursor: wakes a stdin pump blocked on it
+
+    def setWriter(self, writer):
+        self._writer = writer
+
+    def _pump_in(self):
+        while True:
+            with self._cond:
+                while self._reader is None and not self._stopped:
+                    self._cond.wait()
+                if self._stopped:
+                    break
+                reader = self._reader
+            data = reader.read()
+            if data is None:
+                if self._stopped or reader is self._reader:
+                    break
+                continue                           # setReader() swapped the cursor
+            try:
+                self._proc.stdin.write(data)
+                self._proc.stdin.flush()
+            except (OSError, ValueError):          # the child went away / stop() closed stdin
+                break
+
+    def _pump_out(self):
+        out = self._proc.stdout
+        while True:
+            data = out.read1(1 << 16)
+            if not data:
+                break
+            w = self._writer
+            if w is not None:
+                w.write(data)
+
+    def stop(self):
+        import subprocess
+        with self._cond:
+            if self._stopped:
+                return
+            self._stopped = True
+            reader = self._reader
+            self._cond.notify_all()
+        if reader is not None:
+            reader.stop()                          # wakes the stdin pump
+        try:
+            self._proc.stdin.close()
+        except OSError:
+            pass
+        self._proc.terminate()
+        try:
+            self._proc.wait(self._STOP_WAIT_S)
+        except subprocess.TimeoutExpired:
+            self._proc.kill()
+            self._proc.wait()
+        for t in self._threads:
+            t.join(self._STOP_WAIT_S)
+        self._proc.stdout.close()
+
+
 def _unavailable(name):
     def ctor(*a, **k):
         raise NotImplementedError("pycsdr.modules.%s is outside the B200 hot path (SURVEY Appendix C)" % name)
     return type(name, (Module,), {"__init__": lambda self, *a, **k: ctor()})
 
 
-for _n in ("Lowpass", "Downmix", "Throttle", "ExecModule", "SnrSquelch", "SmartSquelch", "TimingRecovery", "DBPskDecoder",
+for _n in ("Lowpass", "Downmix", "Throttle", "SnrSquelch", "SmartSquelch", "TimingRecovery", "DBPskDecoder",
            "VaricodeDecoder", "RttyDecoder", "BaudotDecoder", "MFRttyDecoder", "CwDecoder", "SstvDecoder", "FaxDecoder",
            "SitorBDecoder", "Ccir476Decoder", "DscDecoder", "Ccir493Decoder", "NavtexDecoder"):
     globals()[_n] = _unavailable(_n)
@@ -832,12 +924,14 @@ def _walk(head):
             break
         # the stage that continues THIS chain: a Buffer can have further readers that start chains of their own (the secondary
         # FFT and the SecondarySelector on ClientDemodulatorChain.selectorBuffer, owrx/dsp.py:49,188-225) — those are heads
+        # A fused stage goes before an unfused one: the WFm chain's tap buffer is read by the FractionalDecimator AND by the
+        # RDS path's Convert(FLOAT, SHORT) (csdr/chain/analog.py:62,73-76); the chain goes on through the former.
         nxt = None
         for m in list(_GRAPH.modules):
             r = m._reader
             if r is not None and r._buffer is w and not m._stopped and not r._stopped and not m.HEAD:
-                nxt = m
-                break
+                if nxt is None or (isinstance(nxt, _Unfused) and not isinstance(m, _Unfused)):
+                    nxt = m
         if nxt is None:
             break
         links.append(w)
@@ -918,12 +1012,39 @@ class _WaterfallPlan:
 _DEMODS = ("nfm", "am", "ssb", "wfm", "none")
 
 
+_MPX_WARNED = set()      # ids of tap Buffers whose float reader has been reported as not served
+
+
 class _ChannelPlan:
     """one client chain = one channel of the source's bank"""
 
     def __init__(self):
         self.cid = None
         self.spec_key = None
+
+    @staticmethod
+    def _mpx_tap(limit, frac):
+        """the WFm chain's multiplex tap (csdr/chain/analog.py:62,73-76): the Limit writes into a Buffer of its own that the
+        audio path's FractionalDecimator reads; any other reader of it is a tap consumer.  A Convert(FLOAT, SHORT) reader (the
+        RDS path) is fused: ("s16", the Convert's writer).  Any other reader gets the float samples in the tap Buffer itself:
+        ("f32", that Buffer).  With both kinds of reader only the Convert is served (logged once).  (None, None) without a
+        consumer."""
+        tap = limit._writer
+        if not isinstance(tap, Buffer):
+            return None, None
+        for m in list(_GRAPH.modules):
+            r = m._reader
+            if (m is not frac and isinstance(m, Convert) and r is not None and r._buffer is tap and not m._stopped and not r._stopped
+                    and m.IN is Format.FLOAT and m.OUT is Format.SHORT and isinstance(m._writer, Buffer)):
+                if tap._extra_readers(frac._reader) and id(tap) not in _MPX_WARNED:
+                    # one tap per channel: the bank delivers one format, and the int16 samples of the RDS path win
+                    _MPX_WARNED.add(id(tap))
+                    logger.warning("pycsdr-b200: the WFM tap buffer has a float reader beside Convert(FLOAT, SHORT); only the "
+                                   "Convert is served, the float reader receives nothing")
+                return "s16", m._writer
+        if tap._extra_readers(frac._reader):
+            return "f32", tap
+        return None, None
 
     @staticmethod
     def match(chain):
@@ -964,6 +1085,7 @@ class _ChannelPlan:
             d["demod"], d["agc"], used = "ssb", rest[1], 2
         elif kinds[:4] == [FmDemod, Limit, FractionalDecimator, WfmDeemphasis] and rest[2].format is Format.FLOAT:
             d["demod"], d["wfm_frac"], d["wfm_de"], used = "wfm", rest[2], rest[3], 4
+            d["mpx"], d["mpx_writer"] = _ChannelPlan._mpx_tap(rest[1], rest[2])
         elif not rest:
             d["demod"], used = "none", 0
         else:
@@ -1127,6 +1249,12 @@ class _SourceRunner(threading.Thread):
         if st["level"] != level:
             N.check(N.lib.owrx_chan_set_squelch_level(self.bank, cid, level))
             st["level"] = level
+        # the multiplex tap follows its consumers through the setter: no rebuild of the channel when RDS comes or goes
+        mpx = d.get("mpx")
+        if st.get("mpx") != mpx:
+            N.check(N.lib.owrx_chan_set_mpx(self.bank, cid, {None: N.MPX_OFF, "f32": N.MPX_F32, "s16": N.MPX_S16}[mpx]))
+            st["mpx"] = mpx
+        st["mpx_writer"] = d.get("mpx_writer")
         st["demod"] = d["demod"]
         st["tail_writer"] = d["tail"]._writer
         st["power_writer"] = sq.powerWriter if sq is not None else None
@@ -1202,12 +1330,13 @@ class _SourceRunner(threading.Thread):
             out.append(buf[:n.value * width].tobytes())
         return b"".join(out)
 
-    def _drain_bytes(self, N, cid):
+    def _drain_bytes(self, N, cid, fn=None):
+        fn = fn or N.lib.owrx_chan_read_bytes
         out = []
         buf = np.empty(1 << 16, np.uint8)
         while True:
             n = C.c_size_t()
-            N.check(N.lib.owrx_chan_read_bytes(self.bank, cid, buf.ctypes.data_as(C.c_void_p), buf.size, C.byref(n)))
+            N.check(fn(self.bank, cid, buf.ctypes.data_as(C.c_void_p), buf.size, C.byref(n)))
             if n.value == 0:
                 break
             out.append(buf[:n.value].tobytes())
@@ -1239,6 +1368,10 @@ class _SourceRunner(threading.Thread):
                     bi = self._drain(N, N.lib.owrx_chan_read_if, cid, 2)
                     if bi:
                         st["if_writer"].write(bi)
+                if st.get("mpx_writer") is not None:
+                    bm = self._drain_bytes(N, cid, N.lib.owrx_chan_read_mpx)
+                    if bm:
+                        st["mpx_writer"].write(bm)
             if st.get("power_writer") is not None:
                 bp = self._drain(N, N.lib.owrx_chan_read_power, cid, 1)
                 if bp:
