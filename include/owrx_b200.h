@@ -223,6 +223,17 @@ int owrx_chan_read_power(owrx_bank_t* bank, int chan, float* out, size_t cap, si
 #define OWRX_AUDIO_S16   1
 #define OWRX_AUDIO_ADPCM 2
 int owrx_chan_set_audio_format(owrx_bank_t* bank, int chan, int format);
+/* Client-audio resampler.  When the client's audio rate differs from the demodulator's, the reference's Converter is
+ * AudioResampler(inputRate, clientRate) -> Limit -> Convert(FLOAT, SHORT) [-> AdpcmEncoder(sync=True)]
+ * (csdr/chain/clientaudio.py:6-19,34).  owrx_chan_set_audio_resampler puts AudioResampler + Limit in front of this channel's
+ * S16 / ADPCM bytes; owrx_chan_read_audio / _demod and the multiplex tap stay at the demodulator rate.  The resampler is
+ * SPEC-DEFINED (the reference's libsamplerate is not reproduced, see DESIGN.md): with out/in = L/M reduced, a polyphase
+ * Kaiser-windowed sinc (96 dB stop band, cutoff 0.45 * min(in, out)) evaluated causally, so that after n input samples exactly
+ * ceil(n * L / M) output samples exist; then Limit clamps to +-1.  Rates are positive integers; 0, 0 or equal rates remove
+ * it.  OWRX_E_INVALID for a ratio needing more than 65536 taps or a channel without a demodulator (OWRX_DEMOD_NONE).  Like
+ * every setter it takes effect at the next block boundary; setting or changing it starts it from empty history and leaves
+ * the selector, demodulator and Agc state alone.  The ratio is per channel: a channel keeps its group. */
+int owrx_chan_set_audio_resampler(owrx_bank_t* bank, int chan, int input_rate, int output_rate);
 int owrx_chan_read_bytes(owrx_bank_t* bank, int chan, void* out, size_t cap_bytes, size_t* n);
 /* the same bytes as one websocket message: type_byte (0x02 audio / 0x04 HD audio) + data; see owrx_wf_read_message */
 int owrx_chan_read_message(owrx_bank_t* bank, int chan, int type_byte, void* out, size_t cap_bytes, size_t* n);
@@ -302,7 +313,8 @@ int owrx_bank_profile_read(owrx_bank_t* bank, double* k3_ms, uint64_t* k3_launch
 #define OWRX_PROF_FC_INVERSE  3   /* fc_inverse_kernel: per-channel inverse FFT + post-rotation               */
 #define OWRX_PROF_TAIL        4   /* every parallel stage between FirDecimate and the Agc (one bracket per block)  */
 #define OWRX_PROF_AGC         5   /* agc_kernel: the sample-serial Agc                                        */
-#define OWRX_PROF_KINDS       6
+#define OWRX_PROF_RESAMPLE    6   /* audio_resample_kernel: the client-audio resampler                        */
+#define OWRX_PROF_KINDS       7
 int owrx_bank_profile_read_ex(owrx_bank_t* bank, double* ms, uint64_t* launches, int reset);
 
 /* How Shift + FirDecimate (csdr/chain/selector.py:29,95) is evaluated.  All forms compute the same sums

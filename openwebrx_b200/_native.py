@@ -92,6 +92,7 @@ SIGNATURES = {
     "owrx_bank_set_outputs": (_i, [_vp, _i]),
     "owrx_chan_set_audio_format": (_i, [_vp, _i, _i]),
     "owrx_chan_read_bytes": (_i, [_vp, _i, _vp, _sz, _psz]),
+    "owrx_chan_set_audio_resampler": (_i, [_vp, _i, _i, _i]),
     "owrx_chan_set_mpx": (_i, [_vp, _i, _i]),
     "owrx_chan_read_mpx": (_i, [_vp, _i, _vp, _sz, _psz]),
     "owrx_bank_process_device": (_i, [_vp, _vp, _sz, _vp]),
@@ -111,7 +112,7 @@ SIGNATURES = {
     "owrx_bank_set_fir_mode": (_i, [_vp, _i]),
     "owrx_bank_fir_form": (_i, [_vp]),
 }
-PROF_KINDS = ("k3_direct", "fc_forward", "fc_contract", "fc_inverse", "tail", "agc")
+PROF_KINDS = ("k3_direct", "fc_forward", "fc_contract", "fc_inverse", "tail", "agc", "resample")
 FIR_MODES = {"auto": 0, "direct": 1, "fastconv": 2, "fastconv_tc": 3}
 
 for _name, (_res, _args) in SIGNATURES.items():

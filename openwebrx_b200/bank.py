@@ -72,6 +72,14 @@ class Channel:
         code = {"f32": N.AUDIO_F32, "s16": N.AUDIO_S16, "adpcm": N.AUDIO_ADPCM}[fmt]
         N.check(N.lib.owrx_chan_set_audio_format(self.bank._h, self.id, code))
 
+    def set_audio_resampler(self, in_rate, out_rate=None):
+        """AudioResampler(in_rate, out_rate) + Limit in front of the S16 / ADPCM bytes (csdr/chain/clientaudio.py:6-19; the
+        resampler is spec-defined, see owrx_b200.h).  None removes it, as do equal rates.  ValueError for a rejected ratio or
+        a channel without a demodulator."""
+        if in_rate is None or out_rate is None:
+            in_rate = out_rate = 0
+        N.check(N.lib.owrx_chan_set_audio_resampler(self.bank._h, self.id, int(in_rate), int(out_rate)))
+
     def read_message(self, hd=False, cap=1 << 16):
         """queued client-audio bytes as one websocket message: b"\x02" + data (write_dsp_data) or b"\x04" + data
         (write_hd_audio), owrx/connection.py:477-481; None when nothing is queued"""

@@ -120,6 +120,48 @@ void design_nfm_deemphasis(std::vector<float>& out, int sample_rate)
     for (int n = 0; n < len; n++) out[n] = (float)(h[n] / g);
 }
 
+// AudioResampler(in, out) prototype — spec-defined (libsamplerate's converter is not recoverable): L/M = out/in reduced,
+// Kaiser-windowed sinc at the rate L*in with a 96 dB stop band, transition 0.1*min(in, out) and cutoff 0.45*min(in, out);
+// K taps per phase, N = L*K, sum h = L.  Returns false for a ratio whose N exceeds 65536.  Written to `tab` as the polyphase
+// table tab[p * K + j] = h[p + j * L], rounded once to float.
+bool design_audio_resampler(int in_rate, int out_rate, int* L, int* M, int* K, std::vector<float>* tab)
+{
+    long long a = in_rate, b = out_rate;
+    while (b) { const long long t = a % b; a = b; b = t; }
+    const long long l = out_rate / a, m = in_rate / a;
+    const double A = 96.0, beta = 0.1102 * (A - 8.7);
+    const double f_lo = std::min(in_rate, out_rate), fs = (double)l * in_rate;
+    const double df = 0.1 * f_lo / fs, fc = 0.45 * f_lo / fs;
+    const double k = ceil(((A - 7.95) / (14.36 * df) + 1.0) / (double)l);
+    if (k * (double)l > 65536.0) return false;
+    *L = (int)l; *M = (int)m; *K = (int)k;
+    if (!tab) return true;
+    auto i0 = [](double x) {
+        double sum = 1.0, term = 1.0;
+        for (int j = 1; j < 500; j++) {
+            term *= (x / (2.0 * j)) * (x / (2.0 * j));
+            sum += term;
+            if (term < 1e-17 * sum) break;
+        }
+        return sum;
+    };
+    const int n = *L * *K;
+    const double i0b = i0(beta), c = (n - 1) / 2.0;
+    std::vector<double> h((size_t)n);
+    double sum = 0.0;
+    for (int i = 0; i < n; i++) {
+        const double t = 2.0 * fc * (i - c);
+        const double sinc = t == 0.0 ? 1.0 : sin(M_PI * t) / (M_PI * t);
+        const double r = n > 1 ? 2.0 * i / (n - 1) - 1.0 : 0.0;
+        h[(size_t)i] = 2.0 * fc * sinc * i0(beta * sqrt(std::max(0.0, 1.0 - r * r))) / i0b;
+        sum += h[(size_t)i];
+    }
+    tab->resize((size_t)n);
+    for (int p = 0; p < *L; p++)
+        for (int j = 0; j < *K; j++) (*tab)[(size_t)p * *K + j] = (float)(h[(size_t)p + (size_t)j * *L] * (double)l / sum);
+    return true;
+}
+
 // ---------------------------------------------------------------- stage buffer with history
 // rows of `slots * width` floats; rows [0, fill) hold absolute indices [abs_end - fill, abs_end).
 struct StageBuf {
@@ -230,6 +272,8 @@ struct Chan {
     float agc_initial = 1.0f;
     int audio_fmt = OWRX_AUDIO_F32;
     int mpx_fmt = OWRX_MPX_OFF;
+    int rs_in = 0, rs_out = 0;             // owrx_chan_set_audio_resampler: 0 = none
+    bool rs_dirty = false;                 // the resampler (re)starts at the next block boundary (apply_pending)
     unsigned long long gen = 0;            // bank-unique: tells this client from a later one that gets the same id
     FQ q_audio, q_demod, q_if, q_power;
     std::vector<unsigned char> q_bytes, q_mpx;
@@ -295,14 +339,25 @@ struct Group {
     size_t feed_blocks = 0;                          // squelch blocks processed so far in this feed
     size_t pend_rows = 0;                            // FirDecimate rows appended to s1 since the last tail pass
     long long pend_first = 0;
-    // client audio tail (Convert / AdpcmEncoder)
+    // client audio tail (Convert / AdpcmEncoder), and the resampler in front of it
     std::vector<int> h_tail_mode;
+    std::vector<RsCfg> h_rs;
+    RsCfg* d_rs_cfg2[2] = {nullptr, nullptr};
+    RsCfg* d_rs_cfg = nullptr;                       // = d_rs_cfg2[cur]
     int* d_tail_mode2[2] = {nullptr, nullptr};
     int* d_tail_mode = nullptr;                      // = d_tail_mode2[cur]
     TailState* d_tail = nullptr; int* d_tail_count = nullptr;
     int16_t* d_tail_s16 = nullptr; unsigned char* d_tail_bytes = nullptr;
     size_t tail_rows_cap = 0; int tail_cap = 0;
     bool any_tail = false, tail_ran = false;
+    // client-audio resampler (audio_resample_kernel): some slot has one (per-slot state in ChanCfg::rs_*), the largest L/M of
+    // them, its outputs of this feed (rows of d_rs and of the int16 scratch), and the feed's first absolute audio row.  f3 keeps
+    // the K - 1 rows the resampler looks back over its passes (f3.hist).
+    bool any_rs = false, rs_pending = false;
+    double rs_up = 1.0;
+    float* d_rs = nullptr;
+    size_t rs_rows = 0;
+    long long audio_af = 0;
     // K3F fast-convolution channeliser (fastconv.cuh): tables are built lazily on the first eligible pass
     bool fc_ok = false;
     FcShape fc{};
@@ -390,6 +445,9 @@ struct owrx_bank {
     std::vector<std::pair<std::unique_ptr<Group>, cudaEvent_t>> graveyard;
     cudaStream_t ctl_stream = nullptr;
     unsigned long long feeds = 0;                    // host-path feeds so far (parity of the per-slot table copies)
+    // client-audio resampler polyphase tables, one per (L, M) for the bank's lifetime (RsCfg::tab points into them)
+    struct RsTab { float* d; int K; };
+    std::map<std::pair<int, int>, RsTab> rs_tabs;
 };
 
 namespace {
@@ -415,8 +473,8 @@ void group_release(Group* g)
     }
     cudaFree(g->d_bp_H); cudaFree(g->d_bp_X); cudaFree(g->d_bp_Y);
     cudaFree(g->d_partial); cudaFree(g->d_gate); cudaFree(g->d_power); cudaFree(g->d_dcmean); cudaFree(g->d_dcprev);
-    cudaFree(g->d_tail_mode2[0]); cudaFree(g->d_tail_mode2[1]); cudaFree(g->d_tail); cudaFree(g->d_tail_count); cudaFree(g->d_tail_s16);
-    cudaFree(g->d_tail_bytes);
+    cudaFree(g->d_tail_mode2[0]); cudaFree(g->d_tail_mode2[1]); cudaFree(g->d_rs_cfg2[0]); cudaFree(g->d_rs_cfg2[1]); cudaFree(g->d_tail); cudaFree(g->d_tail_count); cudaFree(g->d_tail_s16);
+    cudaFree(g->d_tail_bytes); cudaFree(g->d_rs);
     cudaFree(g->d_fc_h); cudaFree(g->d_fc_tab); cudaFree(g->d_fc_F); cudaFree(g->d_fc_Z); cudaFree(g->d_fc_slots); cudaFree(g->d_fc_rates);
     cudaFree(g->d_fc_scale);
     cudaFree(g->d_fc_tabp); cudaFree(g->d_fc_Fp);
@@ -527,10 +585,12 @@ int group_create(owrx_bank* bank, const owrx_chan_spec_t& sp, int* index)
         (rc = dev_alloc(&g->d_bp_en2[0], S)) || (rc = dev_alloc(&g->d_bp_en2[1], S)) || (rc = dev_alloc(&g->d_cfg2[0], S)) ||
         (rc = dev_alloc(&g->d_cfg2[1], S)) || (rc = dev_alloc(&g->d_state, S)) || (rc = dev_alloc(&g->d_tail_mode2[0], S)) ||
         (rc = dev_alloc(&g->d_tail_mode2[1], S)) || (rc = dev_alloc(&g->d_tail, S)) || (rc = dev_alloc(&g->d_tail_count, S)) ||
+        (rc = dev_alloc(&g->d_rs_cfg2[0], S)) || (rc = dev_alloc(&g->d_rs_cfg2[1], S)) ||
         (rc = dev_alloc(&g->d_stash, S)))
         return rc;
-    g->d_cfg = g->d_cfg2[0]; g->d_bp_en = g->d_bp_en2[0]; g->d_tail_mode = g->d_tail_mode2[0];
+    g->d_cfg = g->d_cfg2[0]; g->d_bp_en = g->d_bp_en2[0]; g->d_tail_mode = g->d_tail_mode2[0]; g->d_rs_cfg = g->d_rs_cfg2[0];
     g->h_tail_mode.assign(S, 0);
+    g->h_rs.assign(S, RsCfg{});
     g->h_rate.assign(S, 0.0); g->h_phase.assign(S, 0.0); g->h_w.assign(S, make_float2(1.f, 0.f));
     g->h_bp_en.assign(S, 0);
     ChanCfg idle{}; idle.kind = OWRX_DEMOD_NONE; idle.agc_ref = 0.8f; idle.agc_max = 1.f; idle.agc_thr = 0.8f;
@@ -637,7 +697,9 @@ int place_channel(owrx_bank* bank, Chan* ch, int gi)
     g->h_cfg[(size_t)slot] = ch->cfg;
     g->h_bp_en[(size_t)slot] = 0;
     g->h_tail_mode[(size_t)slot] = ch->audio_fmt;
+    g->h_rs[(size_t)slot] = RsCfg{};
     g->cfg_stale[0] = g->cfg_stale[1] = true;
+    if (ch->rs_in) { ch->rs_dirty = true; g->rs_pending = true; }    // a moved resampler restarts from empty history
     return OWRX_OK;
 }
 
@@ -665,11 +727,13 @@ int group_grow(owrx_bank* bank, Group* g)
         (rc = regrow(&g->d_bp_en2[0], 1)) || (rc = regrow(&g->d_bp_en2[1], 1)) || (rc = regrow(&g->d_cfg2[0], 1)) ||
         (rc = regrow(&g->d_cfg2[1], 1)) || (rc = regrow(&g->d_state, 1)) || (rc = regrow(&g->d_tail_mode2[0], 1)) ||
         (rc = regrow(&g->d_tail_mode2[1], 1)) || (rc = regrow(&g->d_tail, 1)) || (rc = regrow(&g->d_tail_count, 1)) ||
+        (rc = regrow(&g->d_rs_cfg2[0], 1)) || (rc = regrow(&g->d_rs_cfg2[1], 1)) ||
         (rc = regrow(&g->d_stash, 1)))
         return rc;
     g->d_cfg = g->d_cfg2[g->cur]; g->d_bp_en = g->d_bp_en2[g->cur]; g->d_tail_mode = g->d_tail_mode2[g->cur];
-    cudaFree(g->d_tail_s16); cudaFree(g->d_tail_bytes);
-    g->d_tail_s16 = nullptr; g->d_tail_bytes = nullptr; g->tail_rows_cap = 0; g->tail_cap = 0;
+    g->d_rs_cfg = g->d_rs_cfg2[g->cur];
+    cudaFree(g->d_tail_s16); cudaFree(g->d_tail_bytes); cudaFree(g->d_rs);
+    g->d_tail_s16 = nullptr; g->d_tail_bytes = nullptr; g->d_rs = nullptr; g->tail_rows_cap = 0; g->tail_cap = 0;
     auto regrow_buf = [&](StageBuf& b) -> int {
         if (!b.d[0]) return OWRX_OK;
         for (int k = 0; k < 2; k++) {
@@ -703,6 +767,7 @@ int group_grow(owrx_bank* bank, Group* g)
     g->h_rate.resize((size_t)ns, 0.0); g->h_phase.resize((size_t)ns, 0.0); g->h_w.resize((size_t)ns, make_float2(1.f, 0.f));
     g->h_bp_en.resize((size_t)ns, 0);
     g->h_tail_mode.resize((size_t)ns, 0);
+    g->h_rs.resize((size_t)ns, RsCfg{});
     ChanCfg idle{}; idle.kind = OWRX_DEMOD_NONE; idle.agc_ref = 0.8f; idle.agc_max = 1.f; idle.agc_thr = 0.8f;
     g->h_cfg.resize((size_t)ns, idle);
     g->cfg_stale[0] = g->cfg_stale[1] = true;
@@ -862,12 +927,43 @@ int apply_pending(owrx_bank* bank, Group* g, cudaStream_t st_fir, cudaStream_t s
             if (fmt != OWRX_MPX_OFF) g->mpx_runs.push_back(MpxRun{cid, fmt, run, ch->gen});
         }
     }
+    if (g->rs_pending) {
+        // resamplers set, changed or moved since the last block start from empty history at this block's first audio row
+        for (int s = 0; s < S; s++) {
+            const int cid = g->slot_chan[(size_t)s];
+            Chan* ch = cid >= 0 ? bank->chans[(size_t)cid].get() : nullptr;
+            if (!ch || !ch->rs_dirty) continue;
+            RsCfg c{};
+            c.origin = g->f3.abs_end;
+            if (ch->rs_in) {
+                int L = 0, M = 0, K = 0;
+                design_audio_resampler(ch->rs_in, ch->rs_out, &L, &M, &K, nullptr);
+                const auto& t = bank->rs_tabs.at(std::make_pair(L, M));         // built by the setter
+                c.L = L; c.M = M; c.K = t.K; c.tab = t.d;
+            }
+            g->h_rs[(size_t)s] = c;
+            ch->rs_dirty = false;
+            g->cfg_stale[0] = g->cfg_stale[1] = true;
+        }
+        g->rs_pending = false;
+    }
+    g->any_rs = false; g->rs_up = 1.0;
+    size_t rs_hist = 0;
+    for (const RsCfg& c : g->h_rs) {
+        if (!c.L) continue;
+        g->any_rs = true;
+        g->rs_up = std::max(g->rs_up, (double)c.L / c.M);
+        rs_hist = std::max(rs_hist, (size_t)c.K);
+    }
+    g->f3.hist = rs_hist;                            // kept by the next roll (K - 1 rows back from a pass's first output)
     // per-slot tables of this block's parity: a block still in flight on the other streams keeps reading the other copy
     g->d_cfg = g->d_cfg2[g->cur]; g->d_bp_en = g->d_bp_en2[g->cur]; g->d_tail_mode = g->d_tail_mode2[g->cur];
+    g->d_rs_cfg = g->d_rs_cfg2[g->cur];
     if (g->cfg_stale[g->cur]) {
         OWRX_CUDA(cudaMemcpyAsync(g->d_cfg, g->h_cfg.data(), (size_t)S * sizeof(ChanCfg), cudaMemcpyHostToDevice, st_tail));
         OWRX_CUDA(cudaMemcpyAsync(g->d_bp_en, g->h_bp_en.data(), (size_t)S * sizeof(int), cudaMemcpyHostToDevice, st_tail));
         OWRX_CUDA(cudaMemcpyAsync(g->d_tail_mode, g->h_tail_mode.data(), (size_t)S * sizeof(int), cudaMemcpyHostToDevice, st_tail));
+        OWRX_CUDA(cudaMemcpyAsync(g->d_rs_cfg, g->h_rs.data(), (size_t)S * sizeof(RsCfg), cudaMemcpyHostToDevice, st_tail));
         g->cfg_stale[g->cur] = false;
     }
     g->any_tail = false;
@@ -1371,18 +1467,58 @@ int group_tail_serial(owrx_bank* bank, Group* g, cudaStream_t st)
             bank->stats.kernel_launches++;
             g->f3.appended(n_audio);
             if (g->any_tail) {
-                // ---- client audio tail: Convert(FLOAT, SHORT) [+ AdpcmEncoder(sync=True)]; appends behind earlier passes
-                const size_t row0 = g->last_audio - n_audio;
+                // ---- client audio tail: [AudioResampler + Limit] Convert(FLOAT, SHORT) [+ AdpcmEncoder(sync=True)]; appends
+                // behind earlier passes.  a0: absolute audio row of this pass's first row; the feed's rows start at audio_af.
+                const long long a0 = g->f3.abs_end - (long long)n_audio;
                 if (g->last_audio > g->tail_rows_cap) return fail(OWRX_E_STATE, "audio tail scratch under-provisioned");
+                if (g->any_rs) {
+                    // per-slot output counts follow from (L, M, origin) alone: the host sizes the launch without a read-back
+                    long long most = 0;
+                    for (const RsCfg& c : g->h_rs) {
+                        if (!c.L) continue;
+                        g->rs_rows = std::max(g->rs_rows, (size_t)(rs_outputs(c, a0 + (long long)n_audio) - rs_outputs(c, g->audio_af)));
+                        most = std::max(most, rs_outputs(c, a0 + (long long)n_audio) - rs_outputs(c, a0));
+                    }
+                    if (g->rs_rows > g->tail_rows_cap) return fail(OWRX_E_STATE, "audio resampler scratch under-provisioned");
+                    const long long per_cta = (long long)RS_WARPS * RS_T;
+                    const unsigned gy = (unsigned)std::max(1LL, std::min(65535LL, (most + per_cta - 1) / per_cta));
+                    if ((rc = prof_mark(bank, OWRX_PROF_RESAMPLE, st, true)) != OWRX_OK) return rc;
+                    audio_resample_kernel<<<dim3((unsigned)(S / 32), gy), 32 * RS_WARPS, 0, st>>>(
+                        g->f3.rows(0), g->f3.abs_end - (long long)g->f3.fill, S, g->d_rs_cfg, g->d_tail_mode, a0, (int)n_audio,
+                        g->audio_af, g->d_rs);
+                    OWRX_LAUNCH_CHECK();
+                    if ((rc = prof_mark(bank, OWRX_PROF_RESAMPLE, st, false)) != OWRX_OK) return rc;
+                    bank->stats.kernel_launches++;
+                }
                 audio_tail_kernel<<<(S + 31) / 32, 128, 0, st>>>(g->f3.rows(g->f3.fill - n_audio), S, (int)n_audio, g->d_tail_mode,
-                                                               g->d_tail, g->d_tail_s16 + row0 * (size_t)S, g->d_tail_bytes,
-                                                               g->d_tail_count, g->tail_cap);
+                                                               g->d_tail, g->d_tail_s16, g->d_tail_bytes, g->d_tail_count, g->tail_cap,
+                                                               g->d_rs, g->any_rs ? g->d_rs_cfg : nullptr, a0, g->audio_af);
                 OWRX_LAUNCH_CHECK();
                 bank->stats.kernel_launches++;
                 g->tail_ran = true;
             }
         }
     }
+    return OWRX_OK;
+}
+
+// rows of the client-audio tail's scratch for a feed of up to `low` audio rows: a resampled slot may produce more (L > M)
+size_t tail_rows(const Group* g, size_t low)
+{
+    return g->any_rs ? std::max(low, (size_t)ceil((double)low * g->rs_up) + 2) : low;
+}
+
+// (re)allocates the audio tail's scratch: int16 rows, ADPCM bytes per slot and, with a resampler, the resampled float rows
+int alloc_tail(Group* g, size_t rows)
+{
+    const size_t S = (size_t)g->slots;
+    const int cap = (int)(rows / 2 + 8 * (rows / 2002 + 2) + 16);
+    cudaFree(g->d_tail_s16); cudaFree(g->d_tail_bytes); cudaFree(g->d_rs);
+    g->d_tail_s16 = nullptr; g->d_tail_bytes = nullptr; g->d_rs = nullptr; g->tail_rows_cap = 0; g->tail_cap = 0;
+    OWRX_CUDA(cudaMalloc((void**)&g->d_tail_s16, rows * S * sizeof(int16_t)));
+    OWRX_CUDA(cudaMalloc((void**)&g->d_tail_bytes, (size_t)cap * S));
+    if (g->any_rs) OWRX_CUDA(cudaMalloc((void**)&g->d_rs, rows * S * sizeof(float)));
+    g->tail_rows_cap = rows; g->tail_cap = cap;
     return OWRX_OK;
 }
 
@@ -1402,14 +1538,19 @@ int group_begin_feed(owrx_bank* bank, Group* g, size_t rows, cudaStream_t st_fir
     if ((rc = g->f1.roll(g->f1.hist, st_tail)) != OWRX_OK) return rc;
     if (g->wfm) { g->f1b.roll(0, st_tail); if ((rc = g->f1p.roll(g->f1p.hist, st_tail)) != OWRX_OK) return rc; }
     g->f2.roll(0, st_tail);
-    g->f3.roll(0, st_tail);
+    // f3 keeps the resampler's look-back (none without one); the Agc that wrote it and the copy are on the serial stream, and
+    // the copy's destination may still be read by a split-phase drain
+    if (g->f3.hist && g->f3.drained[g->f3.cur ^ 1]) OWRX_CUDA(cudaStreamWaitEvent(st_serial, g->f3.drained[g->f3.cur ^ 1], 0));
+    if ((rc = g->f3.roll(g->f3.hist, st_serial)) != OWRX_OK) return rc;
+    g->audio_af = g->f3.abs_end;
+    g->rs_rows = 0;
     g->last_audio = g->last_demod = g->last_if = g->last_blocks = 0;
     g->dr_audio = g->dr_demod = g->dr_if = g->dr_blocks = 0;
     g->pass_audio = 0; g->feed_blocks = 0; g->tail_ran = false;
     const bool grow = g->s1.fill + rows > g->s1.cap_rows || (g->has_frac && g->s2.fill + low > g->s2.cap_rows) ||
                       g->s3.fill + low > g->s3.cap_rows || g->f1.fill + low > g->f1.cap_rows || low > g->f2.cap_rows ||
-                      low > g->f3.cap_rows || (g->wfm && (low > g->f1b.cap_rows || g->f1p.fill + low > g->f1p.cap_rows)) || blocks > g->blocks_cap ||
-                      (g->any_tail && low > g->tail_rows_cap);
+                      g->f3.fill + low > g->f3.cap_rows || (g->wfm && (low > g->f1b.cap_rows || g->f1p.fill + low > g->f1p.cap_rows)) ||
+                      blocks > g->blocks_cap || (g->any_tail && tail_rows(g, low) > g->tail_rows_cap);
     if (grow) {
         OWRX_CUDA(cudaDeviceSynchronize());
         if ((rc = g->s1.ensure_new(rows, st_fir)) != OWRX_OK) return rc;
@@ -1429,27 +1570,15 @@ int group_begin_feed(owrx_bank* bank, Group* g, size_t rows, cudaStream_t st_fir
             OWRX_CUDA(cudaMalloc((void**)&g->d_dcprev, (size_t)S * sizeof(float)));
             g->blocks_cap = blocks;
         }
-        if (g->any_tail && low > g->tail_rows_cap) {
-            const int cap = (int)(low / 2 + 8 * (low / 2002 + 2) + 16);
-            cudaFree(g->d_tail_s16); cudaFree(g->d_tail_bytes);
-            g->d_tail_s16 = nullptr; g->d_tail_bytes = nullptr; g->tail_rows_cap = 0; g->tail_cap = 0;
-            OWRX_CUDA(cudaMalloc((void**)&g->d_tail_s16, low * (size_t)S * sizeof(int16_t)));
-            OWRX_CUDA(cudaMalloc((void**)&g->d_tail_bytes, (size_t)cap * S));
-            g->tail_rows_cap = low; g->tail_cap = cap;
-        }
+        if (g->any_tail && tail_rows(g, low) > g->tail_rows_cap && (rc = alloc_tail(g, tail_rows(g, low))) != OWRX_OK) return rc;
         OWRX_CUDA(cudaDeviceSynchronize());
     }
     if ((rc = apply_pending(bank, g, st_fir, st_tail, st_serial)) != OWRX_OK) return rc;
     if (g->any_tail) {
-        // the audio tail's scratch follows any_tail, which apply_pending has just refreshed
-        if (low > g->tail_rows_cap) {
+        // the audio tail's scratch follows any_tail and the resamplers, which apply_pending has just refreshed
+        if (tail_rows(g, low) > g->tail_rows_cap || (g->any_rs && !g->d_rs)) {
             OWRX_CUDA(cudaDeviceSynchronize());
-            const int cap = (int)(low / 2 + 8 * (low / 2002 + 2) + 16);
-            cudaFree(g->d_tail_s16); cudaFree(g->d_tail_bytes);
-            g->d_tail_s16 = nullptr; g->d_tail_bytes = nullptr; g->tail_rows_cap = 0; g->tail_cap = 0;
-            OWRX_CUDA(cudaMalloc((void**)&g->d_tail_s16, low * (size_t)S * sizeof(int16_t)));
-            OWRX_CUDA(cudaMalloc((void**)&g->d_tail_bytes, (size_t)cap * S));
-            g->tail_rows_cap = low; g->tail_cap = cap;
+            if ((rc = alloc_tail(g, std::max(tail_rows(g, low), g->tail_rows_cap))) != OWRX_OK) return rc;
         }
         OWRX_CUDA(cudaMemsetAsync(g->d_tail_count, 0, (size_t)S * sizeof(int), st_serial));
     }
@@ -1518,14 +1647,15 @@ int drain_to_queues(owrx_bank* bank, Group* g, const float* dev_rows, size_t n, 
 // client audio tail -> per-channel byte queues (int16 LE samples, or the ADPCM stream)
 int drain_tail(owrx_bank* bank, Group* g)
 {
-    const size_t n = g->last_audio, S = (size_t)g->slots;
-    const size_t s16_floats = (n * S * sizeof(int16_t) + 3) / 4, byte_floats = ((size_t)g->tail_cap * S + 3) / 4;
+    // rows of the int16 scratch: the feed's audio rows, or more when a resampler produced more
+    const size_t n = g->last_audio, S = (size_t)g->slots, rows = std::max(n, g->rs_rows);
+    const size_t s16_floats = (rows * S * sizeof(int16_t) + 3) / 4, byte_floats = ((size_t)g->tail_cap * S + 3) / 4;
     int rc = ensure_stage(bank, s16_floats + byte_floats + S);
     if (rc != OWRX_OK) return rc;
     int16_t* h16 = reinterpret_cast<int16_t*>(bank->h_stage);
     unsigned char* hb = reinterpret_cast<unsigned char*>(bank->h_stage + s16_floats);
     int* hc = reinterpret_cast<int*>(bank->h_stage + s16_floats + byte_floats);
-    OWRX_CUDA(cudaMemcpyAsync(h16, g->d_tail_s16, n * S * sizeof(int16_t), cudaMemcpyDeviceToHost, bank->stream));
+    OWRX_CUDA(cudaMemcpyAsync(h16, g->d_tail_s16, rows * S * sizeof(int16_t), cudaMemcpyDeviceToHost, bank->stream));
     OWRX_CUDA(cudaMemcpyAsync(hb, g->d_tail_bytes, (size_t)g->tail_cap * S, cudaMemcpyDeviceToHost, bank->stream));
     OWRX_CUDA(cudaMemcpyAsync(hc, g->d_tail_count, S * sizeof(int), cudaMemcpyDeviceToHost, bank->stream));
     OWRX_CUDA(cudaStreamSynchronize(bank->stream));
@@ -1534,10 +1664,13 @@ int drain_tail(owrx_bank* bank, Group* g)
         if (cid < 0) continue;
         Chan* ch = bank->chans[(size_t)cid].get();
         if (ch->audio_fmt == OWRX_AUDIO_S16) {
+            // a resampled slot's count follows from its (L, M, origin), like the kernels' (the same RsCfg)
+            const RsCfg& c = g->h_rs[s];
+            const size_t ns = c.L ? std::min(rows, (size_t)(rs_outputs(c, g->f3.abs_end) - rs_outputs(c, g->audio_af))) : n;
             const size_t o = ch->q_bytes.size();
-            ch->q_bytes.resize(o + n * 2);
+            ch->q_bytes.resize(o + ns * 2);
             int16_t* dst = reinterpret_cast<int16_t*>(ch->q_bytes.data() + o);
-            for (size_t i = 0; i < n; i++) dst[i] = h16[i * S + s];
+            for (size_t i = 0; i < ns; i++) dst[i] = h16[i * S + s];
         } else if (ch->audio_fmt == OWRX_AUDIO_ADPCM) {
             ch->q_bytes.insert(ch->q_bytes.end(), hb + s * (size_t)g->tail_cap, hb + s * (size_t)g->tail_cap + hc[s]);
         }
@@ -1667,6 +1800,7 @@ void owrx_bank_destroy(owrx_bank_t* bank)
     if (bank->ev0) cudaEventDestroy(bank->ev0);
     if (bank->ev1) cudaEventDestroy(bank->ev1);
     for (auto& pe : bank->prof_events) { cudaEventDestroy(pe.first); cudaEventDestroy(pe.second); }
+    for (auto& t : bank->rs_tabs) cudaFree(t.second.d);
     if (bank->stream) cudaStreamDestroy(bank->stream);
     delete bank;
 }
@@ -1724,6 +1858,7 @@ int owrx_bank_remove_channel(owrx_bank_t* bank, int chan)
         g->h_cfg[(size_t)ch->slot] = idle;
         g->h_bp_en[(size_t)ch->slot] = 0;
         g->h_tail_mode[(size_t)ch->slot] = 0;
+        g->h_rs[(size_t)ch->slot] = RsCfg{};
         g->cfg_stale[0] = g->cfg_stale[1] = true;
         g->pend.erase(ch->slot);
         bool live = false;
@@ -1813,6 +1948,10 @@ int owrx_chan_set_demod(owrx_bank_t* bank, int chan, int kind, double audio_rate
     const bool wfm = kind == OWRX_DEMOD_WFM;
     if (wfm && !(audio_rate > 0.0 && tau > 0.0)) return fail(OWRX_E_INVALID, "WFM needs audio_rate and tau");
     if (!wfm) { ch->mpx_fmt = OWRX_MPX_OFF; ch->q_mpx.clear(); }          // the multiplex tap is a WFm chain's
+    if (kind == OWRX_DEMOD_NONE && ch->rs_in) {                           // no audio: nothing to resample
+        ch->rs_in = ch->rs_out = 0;
+        ch->rs_dirty = true; g->rs_pending = true;
+    }
     owrx_chan_spec_t sp = ch->spec;
     sp.wfm = wfm ? 1 : 0;
     if (wfm) {
@@ -1831,6 +1970,7 @@ int owrx_chan_set_demod(owrx_bank_t* bank, int chan, int kind, double audio_rate
         {
             ChanCfg idle{}; idle.kind = OWRX_DEMOD_NONE; idle.agc_ref = 0.8f; idle.agc_max = 1.f; idle.agc_thr = 0.8f;
             g->h_cfg[(size_t)old_slot] = idle; g->h_bp_en[(size_t)old_slot] = 0; g->h_tail_mode[(size_t)old_slot] = 0;
+            g->h_rs[(size_t)old_slot] = RsCfg{};
         }
         g->cfg_stale[0] = g->cfg_stale[1] = true;
         g->pend.erase(old_slot);
@@ -1891,6 +2031,38 @@ int owrx_chan_set_audio_format(owrx_bank_t* bank, int chan, int format)
     ch->audio_fmt = format;
     g->h_tail_mode[(size_t)ch->slot] = format;
     g->cfg_stale[0] = g->cfg_stale[1] = true;
+    return OWRX_OK;
+}
+
+int owrx_chan_set_audio_resampler(owrx_bank_t* bank, int chan, int input_rate, int output_rate)
+{
+    if (!bank) return fail(OWRX_E_INVALID, "NULL bank");
+    if (input_rate < 0 || output_rate < 0 || (input_rate == 0) != (output_rate == 0))
+        return fail(OWRX_E_INVALID, "resampler rates must both be positive (or both 0): %d -> %d", input_rate, output_rate);
+    const bool on = input_rate != output_rate;
+    int L = 0, M = 0, K = 0;
+    if (on && !design_audio_resampler(input_rate, output_rate, &L, &M, &K, nullptr))
+        return fail(OWRX_E_INVALID, "resampler %d -> %d needs more than 65536 taps", input_rate, output_rate);
+    std::lock_guard<std::mutex> lk(bank->mu);
+    Chan* ch = get_chan(bank, chan);
+    if (!ch) return fail(OWRX_E_INVALID, "no such channel %d", chan);
+    if (on && ch->cfg.kind == OWRX_DEMOD_NONE) return fail(OWRX_E_INVALID, "channel %d has no demodulator: it has no audio to resample", chan);
+    if (bank->pending_final) { cudaSetDevice(bank->device); int rcp = finish_pending(bank); if (rcp != OWRX_OK) return rcp; }
+    OWRX_CUDA(cudaSetDevice(bank->device));
+    if (on && !bank->rs_tabs.count(std::make_pair(L, M))) {
+        // first use of this ratio in the bank: design and upload its polyphase table (kept for the bank's lifetime)
+        std::vector<float> tab;
+        design_audio_resampler(input_rate, output_rate, &L, &M, &K, &tab);
+        float* d = nullptr;
+        OWRX_CUDA(cudaMalloc((void**)&d, tab.size() * sizeof(float)));
+        OWRX_CUDA(cudaMemcpy(d, tab.data(), tab.size() * sizeof(float), cudaMemcpyHostToDevice));
+        bank->rs_tabs[std::make_pair(L, M)] = owrx_bank::RsTab{d, K};
+    }
+    // a new Converter starts from empty history (taking effect at the next block boundary, like every setter)
+    ch->rs_in = on ? input_rate : 0;
+    ch->rs_out = on ? output_rate : 0;
+    ch->rs_dirty = true;
+    bank->groups[(size_t)ch->group]->rs_pending = true;
     return OWRX_OK;
 }
 

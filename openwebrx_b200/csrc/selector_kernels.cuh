@@ -224,6 +224,22 @@ struct ChanCfg {
     int mpx_run;        // index of this slot's run among the group's tapped slots of the same format
 };
 
+// Per-slot client-audio resampler (audio_resample_kernel), a per-parity table beside ChanCfg (kept apart so that ChanCfg, which
+// the Agc loads whole, keeps its size and alignment): ratio L/M reduced (L = 0: none), K taps per phase, the polyphase table
+// tab[p * K + j] = h[p + j * L], and the absolute audio row that is its input 0 (rows before it read as zero).
+struct RsCfg {
+    int L, M, K, pad;
+    long long origin;
+    const float* tab;
+};
+
+// outputs a resampled slot has produced once the absolute audio row `a` is reached: ceil((a - origin) * L / M)
+__host__ __device__ __forceinline__ long long rs_outputs(const RsCfg& c, long long a)
+{
+    const long long m = a - c.origin;
+    return m > 0 ? (m * c.L + c.M - 1) / c.M : 0;
+}
+
 // Squelch (SURVEY A.10).  Block power = mean |x|^2 over every `decim`-th sample.  CTA = (32 slots, one block): eight
 // warps stage |x|^2 of the block's decimated samples in shared memory (row loads of 32 adjacent slots), then warp 0
 // adds them in sample order (the oracle's summation order) from shared memory.  The gate (threshold + hang counter,
@@ -1079,6 +1095,44 @@ __global__ void __launch_bounds__(256) transpose_kernel(const T* __restrict__ in
 }
 
 // ------------------------------------------------------------------------------------------------
+// Client-audio resampler: AudioResampler(in, out) -> Limit (csdr/chain/clientaudio.py:6-19), in front of the audio tail.
+// SPEC-DEFINED (the reference's libsamplerate is not in the tree): L/M = out/in reduced, polyphase Kaiser-windowed sinc of
+// K taps per phase (designed on the host, RsCfg::tab), causal
+//   y[k] = sum_{j<K} x[floor(kM/L) - j] * h[kM - floor(kM/L) L + jL],   x[n < 0] = 0,
+// with n counted from RsCfg::origin; after n inputs exactly ceil(nL/M) outputs exist, whatever the pass sizes.
+// The ratio is per slot.  x: the group's audio rows (f3), row r holds absolute row x_abs0 + r and the K - 1 rows before this
+// pass are kept as history.  Output k of a slot goes to row k - (outputs before the feed) of `out`, so that the audio tail
+// finds the pass's outputs where it writes their int16 samples.  Slots without a resampler, or whose audio stays float
+// (mode 0), are skipped.  lane = slot; each warp walks RS_T consecutive outputs of its 32 slots; float32 accumulation.
+// ------------------------------------------------------------------------------------------------
+constexpr int RS_T = 8;
+constexpr int RS_WARPS = 4;
+__global__ void __launch_bounds__(32 * RS_WARPS)
+audio_resample_kernel(const float* __restrict__ x, long long x_abs0, int slots, const RsCfg* __restrict__ cfg,
+                      const int* __restrict__ mode, long long a0, int n, long long af, float* __restrict__ out)
+{
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int s = blockIdx.x * 32 + lane;
+    if (s >= slots || !mode[s]) return;
+    const RsCfg c = cfg[s];
+    if (!c.L) return;
+    const long long kf = rs_outputs(c, af), k1 = rs_outputs(c, a0 + n);
+    const long long step = (long long)gridDim.y * RS_WARPS * RS_T;
+    for (long long kb = rs_outputs(c, a0) + ((long long)blockIdx.y * RS_WARPS + w) * RS_T; kb < k1; kb += step) {
+        const long long ke = kb + RS_T < k1 ? kb + RS_T : k1;
+        for (long long k = kb; k < ke; k++) {
+            const long long nmax = k * c.M / c.L;                        // newest input of output k (origin-relative)
+            const float* h = c.tab + (k * c.M - nmax * c.L) * c.K;
+            const float* xp = x + (c.origin + nmax - x_abs0) * slots + s;
+            const int jn = nmax + 1 < c.K ? (int)nmax + 1 : c.K;         // inputs before the origin are zero
+            float acc = 0.f;
+            for (int j = 0; j < jn; j++) acc = fmaf(__ldg(xp - (ptrdiff_t)j * slots), __ldg(h + j), acc);
+            out[(k - kf) * slots + s] = fminf(fmaxf(acc, -1.0f), 1.0f);   // Limit
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
 // Client audio tail (SURVEY 8f-1): Convert(FLOAT -> SHORT) [+ AdpcmEncoder(sync=True)], reference
 // csdr/chain/clientaudio.py:12,34.  Wire format pinned by the browser decoder
 // (htdocs/lib/AudioEngine.js:449-491): "SYNC", int16 LE step index, int16 LE predictor, then 1001
@@ -1106,7 +1160,8 @@ __device__ __forceinline__ void at_bar_arrive(int id) { asm volatile("barrier.ar
 
 __global__ void __launch_bounds__(128)
 audio_tail_kernel(const float* __restrict__ in, int slots, int n, const int* __restrict__ mode, TailState* __restrict__ ts,
-                  int16_t* __restrict__ s16_out, unsigned char* __restrict__ bytes_out, int* __restrict__ count_out, int cap)
+                  int16_t* __restrict__ s16_out, unsigned char* __restrict__ bytes_out, int* __restrict__ count_out, int cap,
+                  const float* __restrict__ rs, const RsCfg* __restrict__ rcfg, long long a0, long long af)
 {
     __shared__ uint4 succ[IMA_TABLE_ENTRIES];
     __shared__ int qt[2][AT_R][32];                  // converted samples of a tile
@@ -1119,14 +1174,26 @@ audio_tail_kernel(const float* __restrict__ in, int slots, int n, const int* __r
     const int sc = live ? s : slots - 1;
     const int md = live ? mode[sc] : 0;
     if (__syncthreads_and(md == 0)) return;          // (also publishes the table)
-    const int n_tiles = (n + AT_R - 1) / AT_R;
+    // this pass's rows of the slot: the n new audio rows, written at feed row a0 - af; or, for a resampled slot
+    // (rcfg != nullptr, L != 0), the resampler's outputs of this pass, read from and written at feed output row k0 - kf
+    int ns = n;
+    long long row0 = a0 - af;
+    if (rcfg && rcfg[sc].L) {
+        const RsCfg c = rcfg[sc];
+        const long long kf = rs_outputs(c, af), k0 = rs_outputs(c, a0);
+        ns = (int)(rs_outputs(c, a0 + n) - k0);
+        row0 = k0 - kf;
+        in = rs + row0 * slots;
+    }
+    s16_out += row0 * slots;
+    const int n_tiles = (__reduce_max_sync(0xffffffffu, ns) + AT_R - 1) / AT_R;     // the same lanes in every warp
     constexpr int FULL = 1, EMPTY = 3;               // barrier ids FULL + b, EMPTY + b
     if (w == 0) {
         // ---------------------------------------------------------------- encoder
         TailState t = ts[sc];
         ImaState cs = ima_state(t.index, t.pred);
         for (int tl = 0; tl < n_tiles; tl++) {
-            const int b = tl & 1, valid = min(AT_R, n - tl * AT_R);
+            const int b = tl & 1, valid = min(AT_R, ns - tl * AT_R);
             at_bar_sync(FULL + b);
             int nb = 0;
             if (md == 2) {
@@ -1187,7 +1254,7 @@ audio_tail_kernel(const float* __restrict__ in, int slots, int n, const int* __r
             }
         };
         for (int tl = 0; tl < n_tiles; tl++) {
-            const int b = tl & 1, r0 = tl * AT_R, valid = min(AT_R, n - r0);
+            const int b = tl & 1, r0 = tl * AT_R, valid = min(AT_R, ns - r0);
             if (tl >= 2) { at_bar_sync(EMPTY + b); flush(b); }
             float v[(AT_R + 2) / 3];
 #pragma unroll

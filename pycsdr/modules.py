@@ -19,6 +19,7 @@ receives the result bytes, and the selector output is materialised only when som
 """
 import ctypes as C
 import logging
+import math
 import os
 import threading
 import weakref
@@ -616,6 +617,30 @@ class WfmDeemphasis(_Stage):
         self.tau = float(tau)
 
 
+class AudioResampler(_Stage):
+    """AudioResampler(inputRate, outputRate): the client-audio Converter's rate change (csdr/chain/clientaudio.py:16), fused
+    with the Limit and Convert behind it into the channel's audio tail (owrx_chan_set_audio_resampler).  Spec-defined: the
+    reference's libsamplerate is not reproduced (DESIGN.md)."""
+    IN = Format.FLOAT
+    OUT = Format.FLOAT
+
+    def __init__(self, inputRate, outputRate):
+        super().__init__()
+        self.inputRate = int(inputRate)
+        self.outputRate = int(outputRate)
+
+
+def _resampler_ok(in_rate, out_rate):
+    """the library's limit on AudioResampler(in, out): positive rates and at most 65536 prototype taps (owrx_b200.h)"""
+    if in_rate <= 0 or out_rate <= 0:
+        return False
+    g = math.gcd(in_rate, out_rate)
+    L = out_rate // g
+    df = 0.1 * min(in_rate, out_rate) / (L * in_rate)
+    K = math.ceil(((96.0 - 7.95) / (14.36 * df) + 1.0) / L)
+    return L * K <= 65536
+
+
 class Agc(_Stage):
     def __init__(self, format=Format.FLOAT):
         super().__init__()
@@ -726,11 +751,6 @@ class AdpcmEncoder(_Unfused):
     def __init__(self, sync=False):
         super().__init__(sync=sync)
         self.sync = bool(sync)
-
-
-class AudioResampler(_Unfused):
-    IN = Format.FLOAT
-    OUT = Format.FLOAT
 
 
 class NoiseFilter(_Unfused):
@@ -1090,9 +1110,19 @@ class _ChannelPlan:
             d["demod"], used = "none", 0
         else:
             return None
-        # client audio tail (csdr/chain/clientaudio.py:6-35): Convert(FLOAT, SHORT) [+ AdpcmEncoder(sync=True)]
+        # client audio tail (csdr/chain/clientaudio.py:6-35): [AudioResampler + Limit] Convert(FLOAT, SHORT)
+        # [+ AdpcmEncoder(sync=True)]
         after = rest[used:]
         d["audio_fmt"] = "f32"
+        d["resampler"] = None
+        if after and d["demod"] != "none" and isinstance(after[0], AudioResampler):
+            rs = after[0]
+            if len(after) < 3 or not isinstance(after[1], Limit) or not _resampler_ok(rs.inputRate, rs.outputRate):
+                return None
+            d["resampler"] = (rs.inputRate, rs.outputRate)
+            d["resampler_stages"] = (after[0], after[1])
+            after = after[2:]
+            used += 2
         if after and d["demod"] != "none":
             cv = after[0]
             if not (isinstance(cv, Convert) and cv.IN is Format.FLOAT and cv.OUT is Format.SHORT):
@@ -1211,7 +1241,7 @@ class _SourceRunner(threading.Thread):
             sp.wfm_tau = d["wfm_de"].tau
         key = (sp.decimation, sp.transition, sp.cutoff, sp.fraction, sp.bp_transition, sp.squelch_length, sp.deemph_rate,
                sp.wfm, sp.wfm_decimation, sp.wfm_audio_rate, sp.wfm_tau, d["demod"], d["audio_fmt"],
-               tuple(id(m) for m in d["stages"]))
+               tuple(id(m) for m in d["stages"] if m not in d.get("resampler_stages", ())))
         if self.bank is None:
             h = C.c_void_p()
             N.check(N.lib.owrx_bank_create(0, 1.0, C.byref(h)))     # rates are carried by the explicit specs
@@ -1249,6 +1279,11 @@ class _SourceRunner(threading.Thread):
         if st["level"] != level:
             N.check(N.lib.owrx_chan_set_squelch_level(self.bank, cid, level))
             st["level"] = level
+        # the resampler follows its chain through the setter (a new one starts from empty history)
+        if st.get("resampler") != d["resampler"]:
+            rin, rout = d["resampler"] or (0, 0)
+            N.check(N.lib.owrx_chan_set_audio_resampler(self.bank, cid, rin, rout))
+            st["resampler"] = d["resampler"]
         # the multiplex tap follows its consumers through the setter: no rebuild of the channel when RDS comes or goes
         mpx = d.get("mpx")
         if st.get("mpx") != mpx:
