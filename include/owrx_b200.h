@@ -282,7 +282,8 @@ int owrx_bank_drain(owrx_bank_t* bank);
  * owrx_bank_process_device before _end, which waits for the copies and fills the queues exactly as owrx_bank_drain would
  * have.  One drain in flight at a time (_begin before the previous _end is OWRX_E_INVALID); _end without _begin is a
  * no-op.  When S-meter power reports (OWRX_OUT_POWER) or a client-audio format are enabled, _begin drains synchronously.
- * The multiplex tap (owrx_chan_set_mpx) goes asynchronously like the other outputs. */
+ * The multiplex tap (owrx_chan_set_mpx) goes asynchronously like the other outputs.  Audio, demod and IF follow the tap's
+ * rule: a channel id handed out again between _begin and _end never receives samples of the client that held it before. */
 int owrx_bank_drain_begin(owrx_bank_t* bank);
 int owrx_bank_drain_end(owrx_bank_t* bank);
 /* samples of audio produced per channel by the last owrx_bank_process_device call */

@@ -166,8 +166,8 @@ bool design_audio_resampler(int in_rate, int out_rate, int* L, int* M, int* K, s
 // rows of `slots * width` floats; rows [0, fill) hold absolute indices [abs_end - fill, abs_end).
 struct StageBuf {
     float* d[2] = {nullptr, nullptr};
-    // split-phase drain (owrx_bank_drain_begin): recorded after the transpose that read buffer b; the next writer of that
-    // buffer waits for it.  Created on first use; an event that was never recorded does not block.
+    // recorded by the split-phase drain (owrx_bank_drain_begin, through drain_enqueue) after the transpose that read buffer b;
+    // the next writer of that buffer waits for it.  Created on first use; an event that was never recorded does not block.
     cudaEvent_t drained[2] = {nullptr, nullptr};
     int cur = 0, width = 1, slots = 0;
     size_t hist = 0, cap_rows = 0, fill = 0;
@@ -331,10 +331,12 @@ struct Group {
     float2* d_partial = nullptr; size_t partial_cap = 0;
     unsigned char* d_gate = nullptr; float* d_power = nullptr; float* d_dcmean = nullptr; float* d_dcprev = nullptr;
     size_t blocks_cap = 0;
-    long long sq_block_abs = 0;                      // absolute squelch block counter (for report interval)
+    long long sq_block_abs = 0;                      // squelch blocks processed so far (S-meter report interval)
+    long long sq_block_first = 0;                    // sq_block_abs at the start of this feed
     // last run
     size_t last_audio = 0, last_demod = 0, last_if = 0, last_blocks = 0;
     size_t dr_audio = 0, dr_demod = 0, dr_if = 0, dr_blocks = 0;    // of those, already copied to the host queues
+    bool dr_final = false;                           // the feed's client-audio bytes and multiplex tap are in the queues
     size_t pass_audio = 0;                           // audio rows produced by the last tail pass
     size_t feed_blocks = 0;                          // squelch blocks processed so far in this feed
     size_t pend_rows = 0;                            // FirDecimate rows appended to s1 since the last tail pass
@@ -382,6 +384,63 @@ struct Group {
     cudaEvent_t mpx_drained[2] = {nullptr, nullptr};
 };
 
+// ---------------------------------------------------------------- output drain
+// Every path that moves outputs to the host queues (the host feed per chunk and at its end, deferred drain, owrx_bank_drain,
+// owrx_bank_drain_begin / _end) takes the same three steps: drain_items lists what is to move, one item per (group, output);
+// drain_enqueue stages the list on a stream; drain_deliver pushes the staged bytes into the queues once the copies have landed.
+enum DrainKind { DRAIN_AUDIO, DRAIN_DEMOD, DRAIN_IF, DRAIN_POWER, DRAIN_BYTES, DRAIN_MPX };
+
+// the client a slot (DRAIN_MPX: a run) belongs to when the drain is listed; delivery skips it once that client has left
+struct DrainTo {
+    int chan;
+    unsigned long long gen;
+    int fmt;                     // DRAIN_BYTES: the client-audio format; DRAIN_MPX: the tap format
+    size_t n;                    // DRAIN_BYTES: S16 samples of the slot; DRAIN_MPX: the run's first byte in the item
+};
+
+struct DrainItem {
+    DrainKind kind;
+    Group* g = nullptr;          // read by drain_enqueue only (the client-audio and tap scratch, the events it records)
+    const float* src = nullptr;  // AUDIO / DEMOD / IF: the first row to move; POWER: the first block
+    StageBuf* buf = nullptr;     // AUDIO / DEMOD / IF: the buffer src lies in
+    size_t n = 0;                // rows of `slots` elements of `width` floats (POWER: blocks; BYTES: int16 rows; MPX: rows per run)
+    int slots = 0, width = 1;
+    size_t cap = 0;              // BYTES: ADPCM bytes per slot; MPX: rows per run of the gather region
+    long long phase = 0;         // POWER: absolute squelch block of block 0
+    size_t bytes = 0, off = 0;   // size and offset in the staging (drain_enqueue)
+    std::vector<DrainTo> to;     // per slot (MPX: per run)
+    bool transposed() const { return kind == DRAIN_AUDIO || kind == DRAIN_DEMOD || kind == DRAIN_IF; }
+};
+
+// page-locked host staging and device transpose scratch of a drain; grows while no drain is in flight on it
+struct DrainStage {
+    unsigned char* h = nullptr;
+    unsigned char* d = nullptr;
+    size_t h_cap = 0, d_cap = 0;
+
+    int reserve(size_t h_bytes, size_t d_bytes)
+    {
+        if (h_bytes > h_cap) {
+            if (h) cudaFreeHost(h);
+            h = nullptr; h_cap = 0;
+            OWRX_CUDA(cudaMallocHost((void**)&h, h_bytes));
+            h_cap = h_bytes;
+        }
+        if (d_bytes > d_cap) {
+            cudaFree(d); d = nullptr; d_cap = 0;
+            OWRX_CUDA(cudaMalloc((void**)&d, d_bytes));
+            d_cap = d_bytes;
+        }
+        return OWRX_OK;
+    }
+    void release()
+    {
+        if (h) cudaFreeHost(h);
+        cudaFree(d);
+        h = nullptr; d = nullptr; h_cap = d_cap = 0;
+    }
+};
+
 }  // namespace
 
 struct owrx_bank {
@@ -398,17 +457,10 @@ struct owrx_bank {
     float2* d_iq[2] = {nullptr, nullptr};
     int iq_cur = 0;
     size_t iq_cap = 0, iq_fill = 0;
-    // pinned staging + device transpose scratch for the output drain
-    float* h_stage = nullptr; size_t h_stage_cap = 0;
-    float* d_xpose = nullptr; size_t d_xpose_cap = 0;
-    // split-phase drain of the device path (owrx_bank_drain_begin / _end): its own staging, so a synchronous drain in between
-    // cannot clobber it; one item per (group, output) that is in flight
-    struct AsyncDrainItem { int which, width; size_t n, off; std::vector<int> chans; };
-    struct AsyncMpxItem { size_t n, off; int nf; std::vector<MpxRun> runs; };     // off: floats into h_adrain
-    float* h_adrain = nullptr; size_t h_adrain_cap = 0;
-    float* d_adrain = nullptr; size_t d_adrain_cap = 0;
-    std::vector<AsyncDrainItem> adrain_items;
-    std::vector<AsyncMpxItem> adrain_mpx;
+    // staging of the synchronous drains, and of the split-phase drain (owrx_bank_drain_begin / _end): a synchronous drain
+    // between _begin and _end must not clobber the copies in flight; adrain_items is the list they deliver
+    DrainStage stage, adrain_stage;
+    std::vector<DrainItem> adrain_items;
     bool adrain_pending = false;
     cudaEvent_t adrain_done = nullptr;                         // the D2H copies have landed
     owrx_bank_stats_t stats{};
@@ -1282,16 +1334,15 @@ int group_tail(owrx_bank* bank, Group* g, cudaStream_t st)
         OWRX_LAUNCH_CHECK();
         bank->stats.kernel_launches++;
     }
-    const size_t if_row0 = g->s3.fill;
     g->s3.appended(n2);
     g->last_if += n2;
-    (void)if_row0;
 
     // ---- Squelch over whole blocks
     const size_t pending = (size_t)(g->s3.abs_end - g->sq_abs);
     const size_t nb = pending / (size_t)g->sq_len;
     const size_t n4 = nb * (size_t)g->sq_len;
     g->last_blocks += nb;
+    g->sq_block_abs += (long long)nb;
     if (nb) {
         if (g->feed_blocks + nb > g->blocks_cap) return fail(OWRX_E_STATE, "squelch scratch under-provisioned");
         // per-block scratch of this pass sits behind the blocks of earlier passes of the same feed
@@ -1546,6 +1597,8 @@ int group_begin_feed(owrx_bank* bank, Group* g, size_t rows, cudaStream_t st_fir
     g->rs_rows = 0;
     g->last_audio = g->last_demod = g->last_if = g->last_blocks = 0;
     g->dr_audio = g->dr_demod = g->dr_if = g->dr_blocks = 0;
+    g->dr_final = false;
+    g->sq_block_first = g->sq_block_abs;
     g->pass_audio = 0; g->feed_blocks = 0; g->tail_ran = false;
     const bool grow = g->s1.fill + rows > g->s1.cap_rows || (g->has_frac && g->s2.fill + low > g->s2.cap_rows) ||
                       g->s3.fill + low > g->s3.cap_rows || g->f1.fill + low > g->f1.cap_rows || low > g->f2.cap_rows ||
@@ -1604,113 +1657,180 @@ Chan* get_chan(owrx_bank* bank, int chan)
     return bank->chans[(size_t)chan].get();
 }
 
-int ensure_stage(owrx_bank* bank, size_t floats)
-{
-    if (floats <= bank->h_stage_cap) return OWRX_OK;
-    if (bank->h_stage) cudaFreeHost(bank->h_stage);
-    bank->h_stage = nullptr; bank->h_stage_cap = 0;
-    OWRX_CUDA(cudaMallocHost((void**)&bank->h_stage, floats * sizeof(float)));
-    bank->h_stage_cap = floats;
-    return OWRX_OK;
-}
+// DRAIN_BYTES staging of n int16 rows and `cap` ADPCM bytes per slot: [int16 rows][ADPCM bytes per slot][byte count per slot]
+size_t tail_bytes_at(size_t n, size_t slots) { return (n * slots * sizeof(int16_t) + 15) / 16 * 16; }
+size_t tail_counts_at(size_t n, size_t slots, size_t cap) { return tail_bytes_at(n, slots) + (cap * slots + 15) / 16 * 16; }
 
-// rows [n][slots] of `width`-float elements -> channel-major [slots][n] on the device, one D2H copy, then
-// one contiguous append per channel
-int drain_to_queues(owrx_bank* bank, Group* g, const float* dev_rows, size_t n, int width, int which, cudaStream_t ds)
+// Lists what group g has that is not in the host queues yet: rows [dr_*, last_*) of its audio, demod, IF and S-meter power (as
+// out_mask enables them) and, once the feed is complete (`final`), its client-audio bytes and multiplex tap.  Every item
+// names, per slot, the client it belongs to now.  Marks the listed outputs delivered.
+void drain_items(const owrx_bank* bank, Group* g, bool final, std::vector<DrainItem>& items)
 {
-    if (!n) return OWRX_OK;
-    const size_t floats = n * (size_t)g->slots * width;
-    int rc = ensure_stage(bank, floats);
-    if (rc != OWRX_OK) return rc;
-    if (floats > bank->d_xpose_cap) {
-        cudaFree(bank->d_xpose); bank->d_xpose = nullptr; bank->d_xpose_cap = 0;
-        OWRX_CUDA(cudaMalloc((void**)&bank->d_xpose, floats * sizeof(float)));
-        bank->d_xpose_cap = floats;
-    }
-    const dim3 grid((unsigned)((g->slots + 31) / 32), (unsigned)((n + 31) / 32));
-    if (width == 1) transpose_kernel<float><<<grid, dim3(32, 8), 0, ds>>>(dev_rows, g->slots, n, bank->d_xpose);
-    else transpose_kernel<float2><<<grid, dim3(32, 8), 0, ds>>>(reinterpret_cast<const float2*>(dev_rows), g->slots, n,
-                                                                         reinterpret_cast<float2*>(bank->d_xpose));
-    OWRX_LAUNCH_CHECK();
-    OWRX_CUDA(cudaMemcpyAsync(bank->h_stage, bank->d_xpose, floats * sizeof(float), cudaMemcpyDeviceToHost, ds));
-    OWRX_CUDA(cudaStreamSynchronize(ds));
-    for (int s = 0; s < g->slots; s++) {
+    const int S = g->slots;
+    std::vector<DrainTo> to((size_t)S, DrainTo{-1, 0, 0, 0});
+    for (int s = 0; s < S; s++) {
         const int cid = g->slot_chan[(size_t)s];
-        if (cid < 0) continue;
-        Chan* ch = bank->chans[(size_t)cid].get();
-        FQ& q = which == 0 ? ch->q_audio : (which == 1 ? ch->q_demod : (which == 2 ? ch->q_if : ch->q_power));
-        q.push(bank->h_stage + (size_t)s * n * width, n * width);
+        if (cid >= 0) to[(size_t)s] = DrainTo{cid, bank->chans[(size_t)cid]->gen, bank->chans[(size_t)cid]->audio_fmt, 0};
     }
-    return OWRX_OK;
-}
-
-// client audio tail -> per-channel byte queues (int16 LE samples, or the ADPCM stream)
-int drain_tail(owrx_bank* bank, Group* g)
-{
-    // rows of the int16 scratch: the feed's audio rows, or more when a resampler produced more
-    const size_t n = g->last_audio, S = (size_t)g->slots, rows = std::max(n, g->rs_rows);
-    const size_t s16_floats = (rows * S * sizeof(int16_t) + 3) / 4, byte_floats = ((size_t)g->tail_cap * S + 3) / 4;
-    int rc = ensure_stage(bank, s16_floats + byte_floats + S);
-    if (rc != OWRX_OK) return rc;
-    int16_t* h16 = reinterpret_cast<int16_t*>(bank->h_stage);
-    unsigned char* hb = reinterpret_cast<unsigned char*>(bank->h_stage + s16_floats);
-    int* hc = reinterpret_cast<int*>(bank->h_stage + s16_floats + byte_floats);
-    OWRX_CUDA(cudaMemcpyAsync(h16, g->d_tail_s16, rows * S * sizeof(int16_t), cudaMemcpyDeviceToHost, bank->stream));
-    OWRX_CUDA(cudaMemcpyAsync(hb, g->d_tail_bytes, (size_t)g->tail_cap * S, cudaMemcpyDeviceToHost, bank->stream));
-    OWRX_CUDA(cudaMemcpyAsync(hc, g->d_tail_count, S * sizeof(int), cudaMemcpyDeviceToHost, bank->stream));
-    OWRX_CUDA(cudaStreamSynchronize(bank->stream));
-    for (size_t s = 0; s < S; s++) {
-        const int cid = g->slot_chan[s];
-        if (cid < 0) continue;
-        Chan* ch = bank->chans[(size_t)cid].get();
-        if (ch->audio_fmt == OWRX_AUDIO_S16) {
+    auto add = [&](DrainKind kind, size_t n, size_t bytes) -> DrainItem& {
+        items.push_back(DrainItem{kind});
+        DrainItem& it = items.back();
+        it.g = g; it.n = n; it.slots = S; it.bytes = (bytes + 15) / 16 * 16; it.to = to;
+        return it;
+    };
+    auto rows = [&](DrainKind kind, int bit, StageBuf& b, int width, size_t last, size_t& dr) {
+        if ((bank->out_mask & bit) && last > dr) {
+            DrainItem& it = add(kind, last - dr, (last - dr) * (size_t)S * width * sizeof(float));
+            it.src = b.rows(b.fill - last + dr); it.buf = &b; it.width = width;
+        }
+        dr = last;
+    };
+    rows(DRAIN_AUDIO, OWRX_OUT_AUDIO, g->f3, 1, g->last_audio, g->dr_audio);
+    rows(DRAIN_DEMOD, OWRX_OUT_DEMOD, g->f2, 1, g->last_demod, g->dr_demod);
+    rows(DRAIN_IF, OWRX_OUT_IF, g->s3, 2, g->last_if, g->dr_if);
+    if ((bank->out_mask & OWRX_OUT_POWER) && g->last_blocks > g->dr_blocks) {
+        DrainItem& it = add(DRAIN_POWER, g->last_blocks - g->dr_blocks, (g->last_blocks - g->dr_blocks) * (size_t)S * sizeof(float));
+        it.src = g->d_power + g->dr_blocks * (size_t)S;
+        it.phase = g->sq_block_first + (long long)g->dr_blocks;
+    }
+    g->dr_blocks = g->last_blocks;
+    if (!final || g->dr_final) return;
+    g->dr_final = true;
+    if (g->any_tail && g->tail_ran && g->last_audio) {
+        // rows of the int16 scratch: the feed's audio rows, or more when a resampler produced more
+        const size_t n = std::max(g->last_audio, g->rs_rows);
+        DrainItem& it = add(DRAIN_BYTES, n, tail_counts_at(n, S, g->tail_cap) + (size_t)S * sizeof(int));
+        it.cap = (size_t)g->tail_cap;
+        for (int s = 0; s < S; s++) {
             // a resampled slot's count follows from its (L, M, origin), like the kernels' (the same RsCfg)
-            const RsCfg& c = g->h_rs[s];
-            const size_t ns = c.L ? std::min(rows, (size_t)(rs_outputs(c, g->f3.abs_end) - rs_outputs(c, g->audio_af))) : n;
-            const size_t o = ch->q_bytes.size();
-            ch->q_bytes.resize(o + ns * 2);
-            int16_t* dst = reinterpret_cast<int16_t*>(ch->q_bytes.data() + o);
-            for (size_t i = 0; i < ns; i++) dst[i] = h16[i * S + s];
-        } else if (ch->audio_fmt == OWRX_AUDIO_ADPCM) {
-            ch->q_bytes.insert(ch->q_bytes.end(), hb + s * (size_t)g->tail_cap, hb + s * (size_t)g->tail_cap + hc[s]);
+            const RsCfg& c = g->h_rs[(size_t)s];
+            it.to[(size_t)s].n = c.L ? std::min(it.n, (size_t)(rs_outputs(c, g->f3.abs_end) - rs_outputs(c, g->audio_af))) : g->last_audio;
         }
     }
-    return OWRX_OK;
-}
-
-// multiplex tap: the D2H of a block's runs, packed as [F32 runs][S16 runs] of n rows each (at most two copies)
-int enqueue_mpx_copy(const Group* g, unsigned char* host, cudaStream_t ds)
-{
-    const size_t n = g->mpx_rows, nf = (size_t)g->mpx_nf, ns = (size_t)g->mpx_ns, cap = g->mpx_cap;
-    const unsigned char* d = g->d_mpx[g->cur];
-    if (nf) OWRX_CUDA(cudaMemcpy2DAsync(host, n * 4, d, cap * 4, n * 4, nf, cudaMemcpyDeviceToHost, ds));
-    if (ns) OWRX_CUDA(cudaMemcpy2DAsync(host + nf * n * 4, n * 2, d + nf * cap * 4, cap * 2, n * 2, ns, cudaMemcpyDeviceToHost, ds));
-    return OWRX_OK;
-}
-
-size_t mpx_packed_bytes(const Group* g) { return g->mpx_rows * (4 * (size_t)g->mpx_nf + 2 * (size_t)g->mpx_ns); }
-
-// packed runs -> per-channel queues; a run goes only to the client it was gathered for, in the format it was gathered in
-void deliver_mpx(owrx_bank* bank, const std::vector<MpxRun>& runs, size_t nf, size_t n, const unsigned char* host)
-{
-    for (const MpxRun& r : runs) {
-        if (r.chan < 0 || (size_t)r.chan >= bank->chans.size()) continue;
-        Chan* ch = bank->chans[(size_t)r.chan].get();
-        if (!ch || ch->gen != r.gen || ch->mpx_fmt != r.fmt) continue;
-        const unsigned char* src = r.fmt == OWRX_MPX_F32 ? host + (size_t)r.run * n * 4 : host + nf * n * 4 + (size_t)r.run * n * 2;
-        ch->q_mpx.insert(ch->q_mpx.end(), src, src + n * (r.fmt == OWRX_MPX_F32 ? 4 : 2));
+    if (g->mpx_rows && !g->mpx_runs.empty()) {
+        // packed as [F32 runs][S16 runs] of mpx_rows each; a run goes to the client it was gathered for, in its format
+        DrainItem& it = add(DRAIN_MPX, g->mpx_rows, g->mpx_rows * (4 * (size_t)g->mpx_nf + 2 * (size_t)g->mpx_ns));
+        it.cap = g->mpx_cap;
+        it.to.clear();
+        const size_t f32 = (size_t)g->mpx_nf * it.n * 4;
+        for (const MpxRun& r : g->mpx_runs)
+            it.to.push_back(DrainTo{r.chan, r.gen, r.fmt, r.fmt == OWRX_MPX_F32 ? (size_t)r.run * it.n * 4 : f32 + (size_t)r.run * it.n * 2});
     }
 }
 
-int drain_mpx(owrx_bank* bank, Group* g, cudaStream_t ds)
+// Stages `items` on `st`: one transpose per row output ([n][slots] rows -> [slots][n], so that a slot's samples are one
+// contiguous run), then the D2H copies.  `split`: a split-phase drain, whose copies outlive the call; the next writer of a
+// source buffer waits for the transpose that read it (StageBuf::drained), the next gather into a tap region for its copy.
+int drain_enqueue(owrx_bank* bank, std::vector<DrainItem>& items, DrainStage& stage, cudaStream_t st, bool split)
 {
-    if (!g->mpx_rows || g->mpx_runs.empty()) return OWRX_OK;
-    int rc = ensure_stage(bank, (mpx_packed_bytes(g) + 3) / 4);
+    // the transposed items first, so that one copy moves them all
+    size_t xp = 0;
+    for (DrainItem& it : items) if (it.transposed()) { it.off = xp; xp += it.bytes; }
+    size_t total = xp;
+    for (DrainItem& it : items) if (!it.transposed()) { it.off = total; total += it.bytes; }
+    if (!total) return OWRX_OK;
+    int rc = stage.reserve(total, xp);
     if (rc != OWRX_OK) return rc;
-    unsigned char* h = reinterpret_cast<unsigned char*>(bank->h_stage);
-    if ((rc = enqueue_mpx_copy(g, h, ds)) != OWRX_OK) return rc;
-    OWRX_CUDA(cudaStreamSynchronize(ds));
-    deliver_mpx(bank, g->mpx_runs, (size_t)g->mpx_nf, g->mpx_rows, h);
+    for (DrainItem& it : items) {
+        Group* g = it.g;
+        unsigned char* h = stage.h + it.off;
+        const size_t S = (size_t)it.slots;
+        if (it.transposed()) {
+            const dim3 grid((unsigned)((S + 31) / 32), (unsigned)((it.n + 31) / 32));
+            if (it.width == 1) transpose_kernel<float><<<grid, dim3(32, 8), 0, st>>>(it.src, it.slots, it.n, reinterpret_cast<float*>(stage.d + it.off));
+            else transpose_kernel<float2><<<grid, dim3(32, 8), 0, st>>>(reinterpret_cast<const float2*>(it.src), it.slots, it.n,
+                                                                         reinterpret_cast<float2*>(stage.d + it.off));
+            OWRX_LAUNCH_CHECK();
+            bank->stats.kernel_launches++;
+            if (split && (rc = it.buf->mark_drained(st)) != OWRX_OK) return rc;
+        } else if (it.kind == DRAIN_POWER) {
+            OWRX_CUDA(cudaMemcpyAsync(h, it.src, it.n * S * sizeof(float), cudaMemcpyDeviceToHost, st));
+        } else if (it.kind == DRAIN_BYTES) {
+            OWRX_CUDA(cudaMemcpyAsync(h, g->d_tail_s16, it.n * S * sizeof(int16_t), cudaMemcpyDeviceToHost, st));
+            OWRX_CUDA(cudaMemcpyAsync(h + tail_bytes_at(it.n, S), g->d_tail_bytes, it.cap * S, cudaMemcpyDeviceToHost, st));
+            OWRX_CUDA(cudaMemcpyAsync(h + tail_counts_at(it.n, S, it.cap), g->d_tail_count, S * sizeof(int), cudaMemcpyDeviceToHost, st));
+        } else {
+            // the tap's runs, at most two copies
+            const size_t n = it.n, nf = (size_t)g->mpx_nf, ns = (size_t)g->mpx_ns;
+            const unsigned char* d = g->d_mpx[g->cur];
+            if (nf) OWRX_CUDA(cudaMemcpy2DAsync(h, n * 4, d, it.cap * 4, n * 4, nf, cudaMemcpyDeviceToHost, st));
+            if (ns) OWRX_CUDA(cudaMemcpy2DAsync(h + nf * n * 4, n * 2, d + nf * it.cap * 4, it.cap * 2, n * 2, ns, cudaMemcpyDeviceToHost, st));
+            if (split) {
+                if (!g->mpx_drained[g->cur]) OWRX_CUDA(cudaEventCreateWithFlags(&g->mpx_drained[g->cur], cudaEventDisableTiming));
+                OWRX_CUDA(cudaEventRecord(g->mpx_drained[g->cur], st));
+            }
+        }
+    }
+    if (xp) OWRX_CUDA(cudaMemcpyAsync(stage.h, stage.d, xp, cudaMemcpyDeviceToHost, st));
+    return OWRX_OK;
+}
+
+// Pushes staged items into the per-channel queues.  A slot whose client has left, or whose id now belongs to a later client,
+// gets nothing; nor does a tap run whose client has changed its tap format since.
+void drain_deliver(owrx_bank* bank, const std::vector<DrainItem>& items, const unsigned char* stage)
+{
+    for (const DrainItem& it : items) {
+        const unsigned char* h = stage + it.off;
+        const float* f = reinterpret_cast<const float*>(h);
+        for (size_t k = 0; k < it.to.size(); k++) {
+            const DrainTo& t = it.to[k];
+            Chan* ch = t.chan >= 0 && (size_t)t.chan < bank->chans.size() ? bank->chans[(size_t)t.chan].get() : nullptr;
+            if (!ch || ch->gen != t.gen) continue;
+            switch (it.kind) {
+            case DRAIN_AUDIO: case DRAIN_DEMOD: case DRAIN_IF: {
+                FQ& q = it.kind == DRAIN_AUDIO ? ch->q_audio : it.kind == DRAIN_DEMOD ? ch->q_demod : ch->q_if;
+                q.push(f + k * it.n * it.width, it.n * it.width);
+                break;
+            }
+            case DRAIN_POWER:
+                // reportInterval = measurementsPerSec / readingsPerSec = 4 (selector.py:108-109,126)
+                for (size_t b = 0; b < it.n; b++)
+                    if ((it.phase + (long long)b) % 4 == 0) ch->q_power.push_back(f[b * it.slots + k]);
+                break;
+            case DRAIN_BYTES:
+                if (t.fmt == OWRX_AUDIO_S16) {
+                    const int16_t* h16 = reinterpret_cast<const int16_t*>(h);
+                    const size_t o = ch->q_bytes.size();
+                    ch->q_bytes.resize(o + t.n * 2);
+                    int16_t* dst = reinterpret_cast<int16_t*>(ch->q_bytes.data() + o);
+                    for (size_t i = 0; i < t.n; i++) dst[i] = h16[i * it.slots + k];
+                } else if (t.fmt == OWRX_AUDIO_ADPCM) {
+                    const unsigned char* hb = h + tail_bytes_at(it.n, it.slots) + k * it.cap;
+                    ch->q_bytes.insert(ch->q_bytes.end(), hb, hb + reinterpret_cast<const int*>(h + tail_counts_at(it.n, it.slots, it.cap))[k]);
+                }
+                break;
+            case DRAIN_MPX:
+                if (ch->mpx_fmt == t.fmt) ch->q_mpx.insert(ch->q_mpx.end(), h + t.n, h + t.n + it.n * (t.fmt == OWRX_MPX_F32 ? 4 : 2));
+                break;
+            }
+        }
+    }
+}
+
+// enqueue, wait, deliver with the synchronous staging on `st` (which already waits for the work that wrote the outputs)
+int drain_now(owrx_bank* bank, std::vector<DrainItem>& items, cudaStream_t st)
+{
+    int rc = drain_enqueue(bank, items, bank->stage, st, false);
+    if (rc != OWRX_OK) return rc;
+    OWRX_CUDA(cudaStreamSynchronize(st));
+    drain_deliver(bank, items, bank->stage.h);
+    return OWRX_OK;
+}
+
+// every group's outputs of the feed or device block, complete
+int drain_final(owrx_bank* bank, cudaStream_t st)
+{
+    std::vector<DrainItem> items;
+    for (auto& g : bank->groups) if (g) drain_items(bank, g.get(), true, items);
+    return drain_now(bank, items, st);
+}
+
+// `st` waits for everything owrx_bank_process_device has issued, on all three of its streams
+int wait_device_path(owrx_bank* bank, cudaStream_t st)
+{
+    OWRX_CUDA(cudaStreamWaitEvent(st, bank->dev_done, 0));
+    OWRX_CUDA(cudaStreamWaitEvent(st, bank->tail_done[0], 0));
+    OWRX_CUDA(cudaStreamWaitEvent(st, bank->tail_done[1], 0));
     return OWRX_OK;
 }
 
@@ -1779,14 +1899,14 @@ void owrx_bank_destroy(owrx_bank_t* bank)
     for (auto& g : bank->groups) if (g) group_release(g.get());
     reap_groups(bank, true);
     if (bank->ctl_stream) cudaStreamDestroy(bank->ctl_stream);
-    cudaFree(bank->d_iq[0]); cudaFree(bank->d_iq[1]); cudaFree(bank->d_xpose); cudaFree(bank->d_raw);
+    cudaFree(bank->d_iq[0]); cudaFree(bank->d_iq[1]); cudaFree(bank->d_raw);
     for (cudaEvent_t e : bank->chunk_events) cudaEventDestroy(e);
     for (cudaEvent_t e : bank->fir_events) cudaEventDestroy(e);
     for (cudaEvent_t e : bank->drain_events) cudaEventDestroy(e);
     if (bank->drain_stream) cudaStreamDestroy(bank->drain_stream);
     if (bank->adrain_done) cudaEventDestroy(bank->adrain_done);
-    cudaFree(bank->d_adrain);
-    if (bank->h_adrain) cudaFreeHost(bank->h_adrain);
+    bank->stage.release();
+    bank->adrain_stage.release();
     if (bank->fir_done) cudaEventDestroy(bank->fir_done);
     if (bank->dev_done) cudaEventDestroy(bank->dev_done);
     if (bank->tail_done[0]) cudaEventDestroy(bank->tail_done[0]);
@@ -1796,7 +1916,6 @@ void owrx_bank_destroy(owrx_bank_t* bank)
     if (bank->serial_stream) cudaStreamDestroy(bank->serial_stream);
     if (bank->ptail_done[0]) cudaEventDestroy(bank->ptail_done[0]);
     if (bank->ptail_done[1]) cudaEventDestroy(bank->ptail_done[1]);
-    if (bank->h_stage) cudaFreeHost(bank->h_stage);
     if (bank->ev0) cudaEventDestroy(bank->ev0);
     if (bank->ev1) cudaEventDestroy(bank->ev1);
     for (auto& pe : bank->prof_events) { cudaEventDestroy(pe.first); cudaEventDestroy(pe.second); }
@@ -2137,58 +2256,12 @@ int owrx_bank_set_outputs(owrx_bank_t* bank, int mask)
     return OWRX_OK;
 }
 
-// host <- device for one group: the rows of this feed that are not in the host queues yet, up to the given counts
-// (a snapshot taken when a chunk's kernels were issued; `ds` already waits for that chunk).  `final` also moves the
-// client-audio-tail bytes and closes the feed's S-meter phase.
-struct DrainMark { size_t audio, demod, if_, blocks; };
-static int group_drain(owrx_bank* bank, Group* g, cudaStream_t ds, const DrainMark& upto, bool final)
-{
-    int rc;
-    if ((bank->out_mask & OWRX_OUT_AUDIO) && upto.audio > g->dr_audio &&
-        (rc = drain_to_queues(bank, g, g->f3.rows(g->f3.fill - g->last_audio + g->dr_audio), upto.audio - g->dr_audio, 1, 0, ds)))
-        return rc;
-    g->dr_audio = std::max(g->dr_audio, upto.audio);
-    if (final && g->any_tail && g->tail_ran && g->last_audio && (rc = drain_tail(bank, g)) != OWRX_OK) return rc;
-    if (final && (rc = drain_mpx(bank, g, ds)) != OWRX_OK) return rc;
-    if ((bank->out_mask & OWRX_OUT_DEMOD) && upto.demod > g->dr_demod &&
-        (rc = drain_to_queues(bank, g, g->f2.rows(g->f2.fill - g->last_demod + g->dr_demod), upto.demod - g->dr_demod, 1, 1, ds)))
-        return rc;
-    g->dr_demod = std::max(g->dr_demod, upto.demod);
-    if ((bank->out_mask & OWRX_OUT_IF) && upto.if_ > g->dr_if &&
-        (rc = drain_to_queues(bank, g, g->s3.rows(g->s3.fill - g->last_if + g->dr_if), upto.if_ - g->dr_if, 2, 2, ds)))
-        return rc;
-    g->dr_if = std::max(g->dr_if, upto.if_);
-    if ((bank->out_mask & OWRX_OUT_POWER) && upto.blocks > g->dr_blocks) {
-        // reportInterval = measurementsPerSec / readingsPerSec = 4 (selector.py:108-109,126)
-        const size_t b0 = g->dr_blocks, nb = upto.blocks - b0;
-        if ((rc = ensure_stage(bank, nb * (size_t)g->slots)) != OWRX_OK) return rc;
-        OWRX_CUDA(cudaMemcpyAsync(bank->h_stage, g->d_power + b0 * (size_t)g->slots, nb * (size_t)g->slots * sizeof(float),
-                                  cudaMemcpyDeviceToHost, ds));
-        OWRX_CUDA(cudaStreamSynchronize(ds));
-        for (size_t b = 0; b < nb; b++) {
-            if (((g->sq_block_abs + (long long)(b0 + b)) % 4) != 0) continue;
-            for (int s = 0; s < g->slots; s++) {
-                const int cid = g->slot_chan[(size_t)s];
-                if (cid >= 0) bank->chans[(size_t)cid]->q_power.push_back(bank->h_stage[b * (size_t)g->slots + s]);
-            }
-        }
-    }
-    g->dr_blocks = std::max(g->dr_blocks, upto.blocks);
-    if (final) g->sq_block_abs += (long long)g->last_blocks;
-    return OWRX_OK;
-}
-
 // deferred-drain mode: move the last outputs of the previous feed into the host queues (waits for that feed's kernels)
 static int finish_pending(owrx_bank* bank)
 {
     if (!bank->pending_final) return OWRX_OK;
-    int rc;
-    for (auto& gp : bank->groups) {
-        Group* g = gp.get();
-        if (g && (rc = group_drain(bank, g, bank->stream, DrainMark{g->last_audio, g->last_demod, g->last_if, g->last_blocks}, true)) != OWRX_OK)
-            return rc;
-    }
-    OWRX_CUDA(cudaStreamSynchronize(bank->stream));
+    int rc = drain_final(bank, bank->stream);
+    if (rc != OWRX_OK) return rc;
     bank->pending_final = false;
     return OWRX_OK;
 }
@@ -2297,7 +2370,7 @@ int owrx_bank_feed_fmt(owrx_bank_t* bank, const void* iq_raw, size_t n_samples, 
         OWRX_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
         bank->drain_events.push_back(e);
     }
-    std::vector<std::vector<DrainMark>> marks(n_chunks);
+    std::vector<DrainItem> chunk_items;               // outputs of the previous chunk, drained while the GPU works on the next
     while (bank->fir_events.size() < n_chunks) {
         cudaEvent_t e;
         OWRX_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -2330,17 +2403,17 @@ int owrx_bank_feed_fmt(owrx_bank_t* bank, const void* iq_raw, size_t n_samples, 
             // outputs of chunk c are complete once `tails` gets here; while the GPU works on chunk c+1 the host copies the
             // outputs of chunk c-1 into the per-channel queues (drain stream: waits for that chunk only)
             OWRX_CUDA(cudaEventRecord(bank->drain_events[c], tails));
-            marks[c].clear();
-            for (auto& gp : bank->groups) {
-                Group* g = gp.get();
-                marks[c].push_back(g ? DrainMark{g->last_audio, g->last_demod, g->last_if, g->last_blocks} : DrainMark{0, 0, 0, 0});
-            }
             // (deferred drain: the host does not wait inside a feed at all — every output of the block moves at the start of
             // the next feed, so that feed's uploads queue right behind this one's and PCIe never idles)
-            if (c >= 1 && !bank->deferred) {
-                OWRX_CUDA(cudaStreamWaitEvent(bank->drain_stream, bank->drain_events[c - 1], 0));
-                for (size_t gi = 0; gi < bank->groups.size(); gi++)
-                    if (bank->groups[gi] && (rc = group_drain(bank, bank->groups[gi].get(), bank->drain_stream, marks[c - 1][gi], false)) != OWRX_OK) return rc;
+            if (!bank->deferred) {
+                if (!chunk_items.empty()) {
+                    OWRX_CUDA(cudaStreamWaitEvent(bank->drain_stream, bank->drain_events[c - 1], 0));
+                    if ((rc = drain_now(bank, chunk_items, bank->drain_stream)) != OWRX_OK) return rc;
+                    chunk_items.clear();
+                }
+                // the last chunk's outputs go with the feed's final drain
+                if (c + 1 < n_chunks)
+                    for (auto& gp : bank->groups) if (gp) drain_items(bank, gp.get(), false, chunk_items);
             }
         }
     }
@@ -2369,13 +2442,8 @@ int owrx_bank_feed_fmt(owrx_bank_t* bank, const void* iq_raw, size_t n_samples, 
         return OWRX_OK;
     }
     if (trace) { cudaStreamSynchronize(st); lap("gpu done"); }
-    for (auto& gp : bank->groups) {
-        Group* g = gp.get();
-        if (g && (rc = group_drain(bank, g, st, DrainMark{g->last_audio, g->last_demod, g->last_if, g->last_blocks}, true)) != OWRX_OK) return rc;
-    }
+    if ((rc = drain_final(bank, st)) != OWRX_OK) return rc;
     lap("drained");
-    OWRX_CUDA(cudaStreamSynchronize(st));
-    lap("end");
     float ms = 0.f;
     if (cudaEventElapsedTime(&ms, bank->ev0, bank->ev1) == cudaSuccess) bank->stats.device_ms += ms;
     return OWRX_OK;
@@ -2458,7 +2526,6 @@ int owrx_bank_process_device(owrx_bank_t* bank, const void* iq_dev, size_t n_sam
         Group* g = gp.get();
         if (!g) continue;
         if ((rc = group_tail(bank, g, sb)) != OWRX_OK) return rc;
-        g->sq_block_abs += (long long)g->last_blocks;
     }
     if ((rc = prof_mark(bank, OWRX_PROF_TAIL, sb, false)) != OWRX_OK) return rc;
     // three-deep pipeline: FirDecimate of block i+2 (sa) | parallel low-rate stages of block i+1 (sb) | the sample-serial
@@ -2488,45 +2555,17 @@ int owrx_bank_drain(owrx_bank_t* bank)
     std::lock_guard<std::mutex> lk(bank->mu);
     if (bank->pending_final) { cudaSetDevice(bank->device); int rcp = finish_pending(bank); if (rcp != OWRX_OK) return rcp; }
     OWRX_CUDA(cudaSetDevice(bank->device));
-    cudaStream_t st = bank->stream;
-    OWRX_CUDA(cudaStreamWaitEvent(st, bank->dev_done, 0));
-    OWRX_CUDA(cudaStreamWaitEvent(st, bank->tail_done[0], 0));
-    OWRX_CUDA(cudaStreamWaitEvent(st, bank->tail_done[1], 0));
-    int rc;
-    for (auto& gp : bank->groups) {
-        Group* g = gp.get();
-        if (!g) continue;
-        const long long blocks = (long long)g->last_blocks;
-        g->sq_block_abs -= blocks;                   // group_drain re-adds it (power report phase)
-        if ((rc = group_drain(bank, g, st, DrainMark{g->last_audio, g->last_demod, g->last_if, g->last_blocks}, true)) != OWRX_OK) return rc;
-    }
-    OWRX_CUDA(cudaStreamSynchronize(st));
-    return OWRX_OK;
+    int rc = wait_device_path(bank, bank->stream);
+    return rc != OWRX_OK ? rc : drain_final(bank, bank->stream);
 }
 
-// Split-phase drain (streaming hosts of the device path): _begin enqueues, on the drain stream, the transposes and D2H copies of
-// what the last owrx_bank_process_device call produced, behind that block's kernels; the caller may issue the NEXT block
-// before _end, which waits for the copies and hands the samples to the per-channel queues.  The stage buffers are
-// double-buffered, so the next block does not touch what is being drained; whichever later block writes such a buffer again
-// waits for the transpose that read it (StageBuf::drained).  Outputs the asynchronous form does not cover (S-meter power reports, the client-audio
-// tail) make _begin fall back to the synchronous drain.
-static int adrain_sync_fallback(owrx_bank* bank)
-{
-    cudaStream_t st = bank->stream;
-    OWRX_CUDA(cudaStreamWaitEvent(st, bank->dev_done, 0));
-    OWRX_CUDA(cudaStreamWaitEvent(st, bank->tail_done[0], 0));
-    OWRX_CUDA(cudaStreamWaitEvent(st, bank->tail_done[1], 0));
-    int rc;
-    for (auto& gp : bank->groups) {
-        Group* g = gp.get();
-        if (!g) continue;
-        g->sq_block_abs -= (long long)g->last_blocks;
-        if ((rc = group_drain(bank, g, st, DrainMark{g->last_audio, g->last_demod, g->last_if, g->last_blocks}, true)) != OWRX_OK) return rc;
-    }
-    OWRX_CUDA(cudaStreamSynchronize(st));
-    return OWRX_OK;
-}
-
+// Split-phase drain (streaming hosts of the device path): _begin enqueues, on the drain stream and with staging of its own, the
+// transposes and D2H copies of what the last owrx_bank_process_device call produced, behind that block's kernels; the caller
+// may issue the NEXT block before _end, which waits for the copies and hands the samples to the per-channel queues.  The stage
+// buffers are double-buffered, so the next block does not touch what is being drained; whichever later block writes such a
+// buffer again waits for the transpose that read it (StageBuf::drained), and the next gather into a tap region for its copy
+// (Group::mpx_drained).  S-meter power reports and client-audio bytes are read from scratch the next block overwrites: with
+// either enabled, _begin completes the drain at once.
 int owrx_bank_drain_begin(owrx_bank_t* bank)
 {
     if (!bank) return fail(OWRX_E_INVALID, "NULL bank");
@@ -2535,78 +2574,21 @@ int owrx_bank_drain_begin(owrx_bank_t* bank)
     OWRX_CUDA(cudaSetDevice(bank->device));
     if (bank->pending_final) { int rcp = finish_pending(bank); if (rcp != OWRX_OK) return rcp; }
     if (bank->calls == 0) return OWRX_OK;
-    bool fallback = (bank->out_mask & OWRX_OUT_POWER) != 0;
-    for (auto& gp : bank->groups) if (gp && gp->any_tail && gp->tail_ran && gp->last_audio) fallback = true;
-    if (fallback) return adrain_sync_fallback(bank);
-    // ---- what is to move: one item per (group, output)
-    bank->adrain_items.clear();
-    size_t total = 0;
-    struct Src { const float* rows; int slots; StageBuf* buf; };
-    std::vector<Src> srcs;
-    for (auto& gp : bank->groups) {
-        Group* g = gp.get();
-        if (!g) continue;
-        const struct { int bit; int which; int width; size_t n; const float* rows; StageBuf* buf; } outs[3] = {
-            {OWRX_OUT_AUDIO, 0, 1, g->last_audio, g->last_audio ? g->f3.rows(g->f3.fill - g->last_audio) : nullptr, &g->f3},
-            {OWRX_OUT_DEMOD, 1, 1, g->last_demod, g->last_demod ? g->f2.rows(g->f2.fill - g->last_demod) : nullptr, &g->f2},
-            {OWRX_OUT_IF, 2, 2, g->last_if, g->last_if ? g->s3.rows(g->s3.fill - g->last_if) : nullptr, &g->s3}};
-        for (const auto& o : outs) {
-            if (!(bank->out_mask & o.bit) || !o.n) continue;
-            owrx_bank::AsyncDrainItem it;
-            it.which = o.which; it.width = o.width; it.n = o.n; it.off = total;
-            it.chans.assign(g->slot_chan.begin(), g->slot_chan.end());
-            total += o.n * (size_t)g->slots * o.width;
-            bank->adrain_items.push_back(std::move(it));
-            srcs.push_back(Src{o.rows, g->slots, o.buf});
-        }
+    std::vector<DrainItem> items;
+    for (auto& g : bank->groups) if (g) drain_items(bank, g.get(), true, items);
+    bool now = (bank->out_mask & OWRX_OUT_POWER) != 0;
+    for (const DrainItem& it : items) if (it.kind == DRAIN_BYTES) now = true;
+    int rc;
+    if (now) {
+        if ((rc = wait_device_path(bank, bank->stream)) != OWRX_OK) return rc;
+        return drain_now(bank, items, bank->stream);
     }
-    // the multiplex tap's packed runs land behind the transposed outputs in the same page-locked staging
-    const size_t total_xpose = total;
-    bank->adrain_mpx.clear();
-    std::vector<Group*> mpx_groups;
-    for (auto& gp : bank->groups) {
-        Group* g = gp.get();
-        if (!g || !g->mpx_rows || g->mpx_runs.empty()) continue;
-        bank->adrain_mpx.push_back(owrx_bank::AsyncMpxItem{g->mpx_rows, total, g->mpx_nf, g->mpx_runs});
-        mpx_groups.push_back(g);
-        total += (mpx_packed_bytes(g) + 3) / 4;
-    }
-    if (bank->adrain_items.empty() && bank->adrain_mpx.empty()) return OWRX_OK;
-    if (total > bank->h_adrain_cap) {
-        // (the previous drain has been ended: nothing is in flight on these buffers)
-        OWRX_CUDA(cudaStreamSynchronize(bank->drain_stream));
-        if (bank->h_adrain) cudaFreeHost(bank->h_adrain);
-        cudaFree(bank->d_adrain);
-        bank->h_adrain = nullptr; bank->d_adrain = nullptr; bank->h_adrain_cap = bank->d_adrain_cap = 0;
-        OWRX_CUDA(cudaMallocHost((void**)&bank->h_adrain, total * sizeof(float)));
-        OWRX_CUDA(cudaMalloc((void**)&bank->d_adrain, total * sizeof(float)));
-        bank->h_adrain_cap = bank->d_adrain_cap = total;
-    }
+    if (items.empty()) return OWRX_OK;
     cudaStream_t ds = bank->drain_stream;
-    OWRX_CUDA(cudaStreamWaitEvent(ds, bank->dev_done, 0));
-    OWRX_CUDA(cudaStreamWaitEvent(ds, bank->tail_done[0], 0));
-    OWRX_CUDA(cudaStreamWaitEvent(ds, bank->tail_done[1], 0));
-    for (size_t i = 0; i < bank->adrain_items.size(); i++) {
-        const auto& it = bank->adrain_items[i];
-        const dim3 grid((unsigned)((srcs[i].slots + 31) / 32), (unsigned)((it.n + 31) / 32));
-        if (it.width == 1) transpose_kernel<float><<<grid, dim3(32, 8), 0, ds>>>(srcs[i].rows, srcs[i].slots, it.n, bank->d_adrain + it.off);
-        else transpose_kernel<float2><<<grid, dim3(32, 8), 0, ds>>>(reinterpret_cast<const float2*>(srcs[i].rows), srcs[i].slots, it.n,
-                                                                     reinterpret_cast<float2*>(bank->d_adrain + it.off));
-        OWRX_LAUNCH_CHECK();
-        bank->stats.kernel_launches++;
-        int rcm = srcs[i].buf->mark_drained(ds);                      // the next writer of THIS buffer waits for the transpose
-        if (rcm != OWRX_OK) return rcm;
-    }
-    if (total_xpose) OWRX_CUDA(cudaMemcpyAsync(bank->h_adrain, bank->d_adrain, total_xpose * sizeof(float), cudaMemcpyDeviceToHost, ds));
-    for (size_t i = 0; i < mpx_groups.size(); i++) {
-        Group* g = mpx_groups[i];
-        int rcm = enqueue_mpx_copy(g, reinterpret_cast<unsigned char*>(bank->h_adrain + bank->adrain_mpx[i].off), ds);
-        if (rcm != OWRX_OK) return rcm;
-        // the next gather into this parity's region waits for the copy
-        if (!g->mpx_drained[g->cur]) OWRX_CUDA(cudaEventCreateWithFlags(&g->mpx_drained[g->cur], cudaEventDisableTiming));
-        OWRX_CUDA(cudaEventRecord(g->mpx_drained[g->cur], ds));
-    }
+    if ((rc = wait_device_path(bank, ds)) != OWRX_OK || (rc = drain_enqueue(bank, items, bank->adrain_stage, ds, true)) != OWRX_OK)
+        return rc;
     OWRX_CUDA(cudaEventRecord(bank->adrain_done, ds));
+    bank->adrain_items = std::move(items);
     bank->adrain_pending = true;
     return OWRX_OK;
 }
@@ -2619,20 +2601,8 @@ int owrx_bank_drain_end(owrx_bank_t* bank)
     OWRX_CUDA(cudaSetDevice(bank->device));
     OWRX_CUDA(cudaEventSynchronize(bank->adrain_done));
     bank->adrain_pending = false;
-    for (const auto& it : bank->adrain_items) {
-        for (size_t s = 0; s < it.chans.size(); s++) {
-            const int cid = it.chans[s];
-            if (cid < 0 || (size_t)cid >= bank->chans.size() || !bank->chans[(size_t)cid]) continue;   // the client left in between
-            Chan* ch = bank->chans[(size_t)cid].get();
-            FQ& q = it.which == 0 ? ch->q_audio : (it.which == 1 ? ch->q_demod : ch->q_if);
-            q.push(bank->h_adrain + it.off + s * it.n * (size_t)it.width, it.n * (size_t)it.width);
-        }
-    }
+    drain_deliver(bank, bank->adrain_items, bank->adrain_stage.h);
     bank->adrain_items.clear();
-    // (the tap's runs carry their client's generation: a channel id reused since _begin gets nothing of the old client)
-    for (const auto& it : bank->adrain_mpx)
-        deliver_mpx(bank, it.runs, (size_t)it.nf, it.n, reinterpret_cast<const unsigned char*>(bank->h_adrain + it.off));
-    bank->adrain_mpx.clear();
     return OWRX_OK;
 }
 
