@@ -253,11 +253,27 @@ int owrx_bank_set_outputs(owrx_bank_t* bank, int mask);
  * (owrx_bank_feed*, deferred drain, owrx_bank_drain, owrx_bank_drain_begin / _end) queues the samples, in order;
  * owrx_chan_read_mpx pops up to cap_bytes of whole samples.  A channel id handed out again never receives samples of the
  * client that held it before. */
-#define OWRX_MPX_OFF 0
+#define OWRX_MPX_OFF 0   /* tap formats: the multiplex tap and the audio tap below use this one set of codes */
 #define OWRX_MPX_F32 1
 #define OWRX_MPX_S16 2
 int owrx_chan_set_mpx(owrx_bank_t* bank, int chan, int format);
 int owrx_chan_read_mpx(owrx_bank_t* bank, int chan, void* out, size_t cap_bytes, size_t* n_bytes);
+/* Demodulated-audio tap.  The reference's secondary demodulators (the digital-mode decoders: FT8 and the other WSJT modes, JS8,
+ * packet, ...) read the Buffer the primary demodulator's last stage writes (Agc, or WfmDeemphasis for WFM), beside the
+ * client-audio Converter; a WSJT-style decoder reads it through Convert(Format.FLOAT, Format.SHORT).  owrx_chan_set_audio_tap
+ * delivers that signal per channel, at the DEMODULATOR rate (before any client-audio resampler, whatever the client-audio
+ * format and whether OWRX_OUT_AUDIO is set; squelch-closed blocks come out as zeros, as the audio does), in the tap formats:
+ *   OWRX_MPX_F32  float32, the samples owrx_chan_read_audio pops
+ *   OWRX_MPX_S16  the same after Convert(FLOAT, SHORT): int16 little-endian, x * 32767 truncated toward zero, clamped to
+ *                 [-32768, 32767]
+ * OWRX_E_INVALID for a channel without a demodulator (OWRX_DEMOD_NONE); re-moding a channel to none turns the tap off, a
+ * change between demodulators keeps it.  Like every setter it takes effect at the next block boundary; a format change
+ * discards queued samples of the old format.  Every drain path (owrx_bank_feed*, deferred drain, owrx_bank_drain,
+ * owrx_bank_drain_begin / _end) queues the samples, in order; the split-phase drain delivers them asynchronously, like the
+ * multiplex tap.  owrx_chan_read_audio_tap pops up to cap_bytes of whole samples.  A channel id handed out again never
+ * receives samples of the client that held it before. */
+int owrx_chan_set_audio_tap(owrx_bank_t* bank, int chan, int format);
+int owrx_chan_read_audio_tap(owrx_bank_t* bank, int chan, void* out, size_t cap_bytes, size_t* n_bytes);
 
 /* Device-resident batch path (bench / embedding): process one wideband block that already lives
  * in device memory; outputs stay on the device and are NOT queued for the host.
@@ -282,7 +298,7 @@ int owrx_bank_drain(owrx_bank_t* bank);
  * owrx_bank_process_device before _end, which waits for the copies and fills the queues exactly as owrx_bank_drain would
  * have.  One drain in flight at a time (_begin before the previous _end is OWRX_E_INVALID); _end without _begin is a
  * no-op.  When S-meter power reports (OWRX_OUT_POWER) or a client-audio format are enabled, _begin drains synchronously.
- * The multiplex tap (owrx_chan_set_mpx) goes asynchronously like the other outputs.  Audio, demod and IF follow the tap's
+ * The multiplex and audio taps (owrx_chan_set_mpx, owrx_chan_set_audio_tap) go asynchronously like the other outputs.  Audio, demod and IF follow the tap's
  * rule: a channel id handed out again between _begin and _end never receives samples of the client that held it before. */
 int owrx_bank_drain_begin(owrx_bank_t* bank);
 int owrx_bank_drain_end(owrx_bank_t* bank);
@@ -315,7 +331,8 @@ int owrx_bank_profile_read(owrx_bank_t* bank, double* k3_ms, uint64_t* k3_launch
 #define OWRX_PROF_TAIL        4   /* every parallel stage between FirDecimate and the Agc (one bracket per block)  */
 #define OWRX_PROF_AGC         5   /* agc_kernel: the sample-serial Agc                                        */
 #define OWRX_PROF_RESAMPLE    6   /* audio_resample_kernel: the client-audio resampler                        */
-#define OWRX_PROF_KINDS       7
+#define OWRX_PROF_TAP         7   /* tap_gather_kernel: the multiplex and audio taps' gathers                 */
+#define OWRX_PROF_KINDS       8
 int owrx_bank_profile_read_ex(owrx_bank_t* bank, double* ms, uint64_t* launches, int reset);
 
 /* How Shift + FirDecimate (csdr/chain/selector.py:29,95) is evaluated.  All forms compute the same sums

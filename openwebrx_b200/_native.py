@@ -18,7 +18,7 @@ OUT_AUDIO, OUT_DEMOD, OUT_IF, OUT_POWER = 1, 2, 4, 8
 IQ_CF32, IQ_CS16, IQ_CU8 = 0, 1, 2
 IQ_FORMATS = {"cf32": IQ_CF32, "cs16": IQ_CS16, "cu8": IQ_CU8}
 AUDIO_F32, AUDIO_S16, AUDIO_ADPCM = 0, 1, 2
-MPX_OFF, MPX_F32, MPX_S16 = 0, 1, 2
+MPX_OFF, MPX_F32, MPX_S16 = 0, 1, 2          # tap formats: the multiplex tap and the audio tap
 
 
 class ChanSpec(C.Structure):
@@ -95,6 +95,8 @@ SIGNATURES = {
     "owrx_chan_set_audio_resampler": (_i, [_vp, _i, _i, _i]),
     "owrx_chan_set_mpx": (_i, [_vp, _i, _i]),
     "owrx_chan_read_mpx": (_i, [_vp, _i, _vp, _sz, _psz]),
+    "owrx_chan_set_audio_tap": (_i, [_vp, _i, _i]),
+    "owrx_chan_read_audio_tap": (_i, [_vp, _i, _vp, _sz, _psz]),
     "owrx_bank_process_device": (_i, [_vp, _vp, _sz, _vp]),
     "owrx_bank_set_pipelined": (_i, [_vp, _i]),
     "owrx_bank_join": (_i, [_vp, _vp]),
@@ -112,7 +114,7 @@ SIGNATURES = {
     "owrx_bank_set_fir_mode": (_i, [_vp, _i]),
     "owrx_bank_fir_form": (_i, [_vp]),
 }
-PROF_KINDS = ("k3_direct", "fc_forward", "fc_contract", "fc_inverse", "tail", "agc", "resample")
+PROF_KINDS = ("k3_direct", "fc_forward", "fc_contract", "fc_inverse", "tail", "agc", "resample", "tap")
 FIR_MODES = {"auto": 0, "direct": 1, "fastconv": 2, "fastconv_tc": 3}
 
 for _name, (_res, _args) in SIGNATURES.items():

@@ -33,6 +33,7 @@ class Channel:
         self.frequencyOffset = 0
         self.bandpassCutoffs = [None, None]
         self._mpx = "off"
+        self._atap = "off"
 
     def setFrequencyOffset(self, offset):            # csdr/chain/selector.py:132-140
         self.frequencyOffset = offset
@@ -55,6 +56,8 @@ class Channel:
         N.check(N.lib.owrx_chan_set_demod(self.bank._h, self.id, k, float(audio_rate), float(tau), prof))
         if k != N.DEMOD_WFM:
             self._mpx = "off"                        # the library turns the tap off with the WFm chain
+        if k == N.DEMOD_NONE:
+            self._atap = "off"                       # ... and the audio tap with the demodulator
 
     def _read(self, fn, width=1):
         chunks = []
@@ -111,12 +114,29 @@ class Channel:
 
     def read_mpx(self):
         """queued multiplex samples: np.float32 ("f32") or np.int16 ("s16")"""
-        dtype = np.int16 if self._mpx == "s16" else np.float32
+        return self._read_tap(N.lib.owrx_chan_read_mpx, self._mpx)
+
+    def set_audio_tap(self, fmt):
+        """demodulated-audio tap (what a secondary demodulator reads beside the client-audio Converter), at the demodulator
+        rate: "off" | "f32" | "s16" (after Convert(FLOAT, SHORT)).  ValueError for an unknown format or a channel without a
+        demodulator."""
+        codes = {"off": N.MPX_OFF, "f32": N.MPX_F32, "s16": N.MPX_S16}
+        if fmt not in codes:
+            raise ValueError("unknown audio tap format %r (off | f32 | s16)" % (fmt,))
+        N.check(N.lib.owrx_chan_set_audio_tap(self.bank._h, self.id, codes[fmt]))
+        self._atap = fmt
+
+    def read_audio_tap(self):
+        """queued audio-tap samples: np.float32 ("f32") or np.int16 ("s16")"""
+        return self._read_tap(N.lib.owrx_chan_read_audio_tap, self._atap)
+
+    def _read_tap(self, fn, fmt):
+        dtype = np.int16 if fmt == "s16" else np.float32
         chunks = []
         buf = np.empty(1 << 18, np.uint8)
         while True:
             n = C.c_size_t()
-            N.check(N.lib.owrx_chan_read_mpx(self.bank._h, self.id, buf.ctypes.data_as(C.c_void_p), buf.size, C.byref(n)))
+            N.check(fn(self.bank._h, self.id, buf.ctypes.data_as(C.c_void_p), buf.size, C.byref(n)))
             if n.value == 0:
                 break
             chunks.append(buf[:n.value].copy())

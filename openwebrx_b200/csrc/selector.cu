@@ -272,18 +272,87 @@ struct Chan {
     float agc_initial = 1.0f;
     int audio_fmt = OWRX_AUDIO_F32;
     int mpx_fmt = OWRX_MPX_OFF;
+    int atap_fmt = OWRX_MPX_OFF;           // owrx_chan_set_audio_tap
     int rs_in = 0, rs_out = 0;             // owrx_chan_set_audio_resampler: 0 = none
     bool rs_dirty = false;                 // the resampler (re)starts at the next block boundary (apply_pending)
     unsigned long long gen = 0;            // bank-unique: tells this client from a later one that gets the same id
     FQ q_audio, q_demod, q_if, q_power;
-    std::vector<unsigned char> q_bytes, q_mpx;
+    std::vector<unsigned char> q_bytes, q_mpx, q_atap;
     size_t last_audio = 0;
 };
 
-// one tapped channel of a block (owrx_chan_set_mpx): where its run sits in the staging region and whom it belongs to
-struct MpxRun {
+// one tapped channel of a block (owrx_chan_set_mpx / _audio_tap): where its run sits in the staging region and whom it belongs to
+struct TapRun {
     int chan, fmt, run;
     unsigned long long gen;
+};
+
+// A per-channel tap gathered by tap_gather_kernel: the tapped slots of the block being issued (rebuilt at every block
+// boundary) and a staging region per block parity of `cap` rows per run; the split-phase drain's copy of a region is awaited
+// through `drained` before the region is written again
+struct TapStage {
+    std::vector<TapRun> runs;
+    int nf = 0, ns = 0;
+    unsigned char* d[2] = {nullptr, nullptr};
+    size_t cap = 0, bytes = 0;
+    size_t rows = 0;                                 // rows gathered in this feed
+    cudaEvent_t drained[2] = {nullptr, nullptr};
+
+    // the block's layout: F32 runs, then S16 runs, in slot order; returns the slot's run
+    void clear() { runs.clear(); nf = ns = 0; }
+    int add(int chan, int fmt, unsigned long long gen)
+    {
+        const int run = fmt == OWRX_MPX_F32 ? nf++ : (fmt == OWRX_MPX_S16 ? ns++ : 0);
+        if (fmt != OWRX_MPX_OFF) runs.push_back(TapRun{chan, fmt, run, gen});
+        return run;
+    }
+    // start of a feed: room for `low` new rows per run (the layout is this block's)
+    int provision(size_t low)
+    {
+        rows = 0;
+        if (runs.empty()) return OWRX_OK;
+        const size_t c = std::max(cap, (low + 7) / 8 * 8);
+        const size_t b = c * (4 * (size_t)nf + 2 * (size_t)ns);
+        if (c != cap || b > bytes) {
+            OWRX_CUDA(cudaDeviceSynchronize());
+            for (int k = 0; k < 2; k++) { cudaFree(d[k]); d[k] = nullptr; }
+            cap = bytes = 0;
+            for (int k = 0; k < 2; k++) OWRX_CUDA(cudaMalloc((void**)&d[k], b));
+            cap = c; bytes = b;
+        }
+        return OWRX_OK;
+    }
+    // new rows [in, in + n) of every tapped slot -> staging region `cur`, on `st`
+    template <typename Sel>
+    int gather(owrx_bank_stats_t& stats, const float* in, int slots, size_t n, Sel sel, int cur, cudaStream_t st)
+    {
+        if (rows + n > cap) return fail(OWRX_E_STATE, "tap staging under-provisioned");
+        if (drained[cur]) OWRX_CUDA(cudaStreamWaitEvent(st, drained[cur], 0));
+        const long long r0 = (long long)rows;
+        const long long tiles = (r0 + (long long)n + MG_R - 1) / MG_R - r0 / MG_R;
+        tap_gather_kernel<<<dim3((unsigned)(slots / 32), (unsigned)std::min<long long>(tiles, 65535)), 256, 0, st>>>(
+            in, slots, (int)n, sel, r0, (long long)cap, nf, d[cur]);
+        OWRX_LAUNCH_CHECK();
+        stats.kernel_launches++;
+        rows += n;
+        return OWRX_OK;
+    }
+    // the split-phase drain's copy of region `cur` has been enqueued on `st`
+    int mark_drained(int cur, cudaStream_t st)
+    {
+        if (!drained[cur]) OWRX_CUDA(cudaEventCreateWithFlags(&drained[cur], cudaEventDisableTiming));
+        OWRX_CUDA(cudaEventRecord(drained[cur], st));
+        return OWRX_OK;
+    }
+    void release()
+    {
+        for (int k = 0; k < 2; k++) {
+            cudaFree(d[k]); d[k] = nullptr;
+            if (drained[k]) cudaEventDestroy(drained[k]);
+            drained[k] = nullptr;
+        }
+        cap = bytes = 0;
+    }
 };
 
 struct Group {
@@ -373,42 +442,40 @@ struct Group {
     void* d_fc_tabp = nullptr; void* d_fc_Fp = nullptr; size_t fc_blocks_cap_tc = 0;
     std::vector<double> fc_tabp_rate;
     std::vector<float> fc_taps;                      // h[t] rounded to float (same values K3 uses)
-    // WFM multiplex tap (mpx_gather_kernel): the tapped slots of the block being issued (rebuilt at every block boundary) and
-    // a staging region per block parity of mpx_cap rows per run; the split-phase drain's copy of a region is awaited through
-    // mpx_drained before the region is written again
-    std::vector<MpxRun> mpx_runs;
-    int mpx_nf = 0, mpx_ns = 0;
-    unsigned char* d_mpx[2] = {nullptr, nullptr};
-    size_t mpx_cap = 0, mpx_bytes = 0;
-    size_t mpx_rows = 0;                             // rows gathered in this feed
-    cudaEvent_t mpx_drained[2] = {nullptr, nullptr};
+    // taps (tap_gather_kernel): the WFM multiplex tap of f1 (ChanCfg::mpx / mpx_run), and the demodulated-audio tap of f3,
+    // whose (format, run) per slot is a per-parity table of its own
+    TapStage mpx, atap;
+    std::vector<TapFmt> h_atap;
+    TapFmt* d_atap2[2] = {nullptr, nullptr};
+    TapFmt* d_atap = nullptr;                        // = d_atap2[cur]
 };
 
 // ---------------------------------------------------------------- output drain
 // Every path that moves outputs to the host queues (the host feed per chunk and at its end, deferred drain, owrx_bank_drain,
 // owrx_bank_drain_begin / _end) takes the same three steps: drain_items lists what is to move, one item per (group, output);
 // drain_enqueue stages the list on a stream; drain_deliver pushes the staged bytes into the queues once the copies have landed.
-enum DrainKind { DRAIN_AUDIO, DRAIN_DEMOD, DRAIN_IF, DRAIN_POWER, DRAIN_BYTES, DRAIN_MPX };
+enum DrainKind { DRAIN_AUDIO, DRAIN_DEMOD, DRAIN_IF, DRAIN_POWER, DRAIN_BYTES, DRAIN_MPX, DRAIN_ATAP };
 
-// the client a slot (DRAIN_MPX: a run) belongs to when the drain is listed; delivery skips it once that client has left
+// the client a slot (DRAIN_MPX / _ATAP: a run) belongs to when the drain is listed; delivery skips it once that client has left
 struct DrainTo {
     int chan;
     unsigned long long gen;
-    int fmt;                     // DRAIN_BYTES: the client-audio format; DRAIN_MPX: the tap format
-    size_t n;                    // DRAIN_BYTES: S16 samples of the slot; DRAIN_MPX: the run's first byte in the item
+    int fmt;                     // DRAIN_BYTES: the client-audio format; DRAIN_MPX / _ATAP: the tap format
+    size_t n;                    // DRAIN_BYTES: S16 samples of the slot; DRAIN_MPX / _ATAP: the run's first byte in the item
 };
 
 struct DrainItem {
     DrainKind kind;
-    Group* g = nullptr;          // read by drain_enqueue only (the client-audio and tap scratch, the events it records)
+    Group* g = nullptr;          // read by drain_enqueue only (the client-audio scratch, the parity of the tap regions)
+    TapStage* tap = nullptr;     // MPX / ATAP: the staging the runs are copied from (drain_enqueue only)
     const float* src = nullptr;  // AUDIO / DEMOD / IF: the first row to move; POWER: the first block
     StageBuf* buf = nullptr;     // AUDIO / DEMOD / IF: the buffer src lies in
-    size_t n = 0;                // rows of `slots` elements of `width` floats (POWER: blocks; BYTES: int16 rows; MPX: rows per run)
+    size_t n = 0;                // rows of `slots` elements of `width` floats (POWER: blocks; BYTES: int16 rows; taps: rows per run)
     int slots = 0, width = 1;
-    size_t cap = 0;              // BYTES: ADPCM bytes per slot; MPX: rows per run of the gather region
+    size_t cap = 0;              // BYTES: ADPCM bytes per slot; taps: rows per run of the gather region
     long long phase = 0;         // POWER: absolute squelch block of block 0
     size_t bytes = 0, off = 0;   // size and offset in the staging (drain_enqueue)
-    std::vector<DrainTo> to;     // per slot (MPX: per run)
+    std::vector<DrainTo> to;     // per slot (taps: per run)
     bool transposed() const { return kind == DRAIN_AUDIO || kind == DRAIN_DEMOD || kind == DRAIN_IF; }
 };
 
@@ -477,6 +544,7 @@ struct owrx_bank {
     std::vector<std::pair<cudaEvent_t, cudaEvent_t>> prof_events;
     std::vector<int> prof_tags;
     size_t prof_used = 0;
+    std::vector<size_t> prof_open;                   // brackets begun and not ended yet, innermost last (a tap gather inside the tail's)
     double prof_ms[OWRX_PROF_KINDS] = {};
     uint64_t prof_launches[OWRX_PROF_KINDS] = {};
     int fir_mode = OWRX_FIR_AUTO, bp_mode = OWRX_FIR_AUTO;
@@ -530,10 +598,8 @@ void group_release(Group* g)
     cudaFree(g->d_fc_h); cudaFree(g->d_fc_tab); cudaFree(g->d_fc_F); cudaFree(g->d_fc_Z); cudaFree(g->d_fc_slots); cudaFree(g->d_fc_rates);
     cudaFree(g->d_fc_scale);
     cudaFree(g->d_fc_tabp); cudaFree(g->d_fc_Fp);
-    for (int k = 0; k < 2; k++) {
-        cudaFree(g->d_mpx[k]);
-        if (g->mpx_drained[k]) cudaEventDestroy(g->mpx_drained[k]);
-    }
+    g->mpx.release(); g->atap.release();
+    cudaFree(g->d_atap2[0]); cudaFree(g->d_atap2[1]);
     g->s1.release(); g->s2.release(); g->s3.release(); g->f1.release(); g->f1p.release(); g->f1b.release(); g->f2.release(); g->f3.release();
 }
 
@@ -638,11 +704,13 @@ int group_create(owrx_bank* bank, const owrx_chan_spec_t& sp, int* index)
         (rc = dev_alloc(&g->d_cfg2[1], S)) || (rc = dev_alloc(&g->d_state, S)) || (rc = dev_alloc(&g->d_tail_mode2[0], S)) ||
         (rc = dev_alloc(&g->d_tail_mode2[1], S)) || (rc = dev_alloc(&g->d_tail, S)) || (rc = dev_alloc(&g->d_tail_count, S)) ||
         (rc = dev_alloc(&g->d_rs_cfg2[0], S)) || (rc = dev_alloc(&g->d_rs_cfg2[1], S)) ||
-        (rc = dev_alloc(&g->d_stash, S)))
+        (rc = dev_alloc(&g->d_atap2[0], S)) || (rc = dev_alloc(&g->d_atap2[1], S)) || (rc = dev_alloc(&g->d_stash, S)))
         return rc;
     g->d_cfg = g->d_cfg2[0]; g->d_bp_en = g->d_bp_en2[0]; g->d_tail_mode = g->d_tail_mode2[0]; g->d_rs_cfg = g->d_rs_cfg2[0];
+    g->d_atap = g->d_atap2[0];
     g->h_tail_mode.assign(S, 0);
     g->h_rs.assign(S, RsCfg{});
+    g->h_atap.assign(S, TapFmt{OWRX_MPX_OFF, 0});
     g->h_rate.assign(S, 0.0); g->h_phase.assign(S, 0.0); g->h_w.assign(S, make_float2(1.f, 0.f));
     g->h_bp_en.assign(S, 0);
     ChanCfg idle{}; idle.kind = OWRX_DEMOD_NONE; idle.agc_ref = 0.8f; idle.agc_max = 1.f; idle.agc_thr = 0.8f;
@@ -780,10 +848,10 @@ int group_grow(owrx_bank* bank, Group* g)
         (rc = regrow(&g->d_cfg2[1], 1)) || (rc = regrow(&g->d_state, 1)) || (rc = regrow(&g->d_tail_mode2[0], 1)) ||
         (rc = regrow(&g->d_tail_mode2[1], 1)) || (rc = regrow(&g->d_tail, 1)) || (rc = regrow(&g->d_tail_count, 1)) ||
         (rc = regrow(&g->d_rs_cfg2[0], 1)) || (rc = regrow(&g->d_rs_cfg2[1], 1)) ||
-        (rc = regrow(&g->d_stash, 1)))
+        (rc = regrow(&g->d_atap2[0], 1)) || (rc = regrow(&g->d_atap2[1], 1)) || (rc = regrow(&g->d_stash, 1)))
         return rc;
     g->d_cfg = g->d_cfg2[g->cur]; g->d_bp_en = g->d_bp_en2[g->cur]; g->d_tail_mode = g->d_tail_mode2[g->cur];
-    g->d_rs_cfg = g->d_rs_cfg2[g->cur];
+    g->d_rs_cfg = g->d_rs_cfg2[g->cur]; g->d_atap = g->d_atap2[g->cur];
     cudaFree(g->d_tail_s16); cudaFree(g->d_tail_bytes); cudaFree(g->d_rs);
     g->d_tail_s16 = nullptr; g->d_tail_bytes = nullptr; g->d_rs = nullptr; g->tail_rows_cap = 0; g->tail_cap = 0;
     auto regrow_buf = [&](StageBuf& b) -> int {
@@ -820,6 +888,7 @@ int group_grow(owrx_bank* bank, Group* g)
     g->h_bp_en.resize((size_t)ns, 0);
     g->h_tail_mode.resize((size_t)ns, 0);
     g->h_rs.resize((size_t)ns, RsCfg{});
+    g->h_atap.resize((size_t)ns, TapFmt{OWRX_MPX_OFF, 0});
     ChanCfg idle{}; idle.kind = OWRX_DEMOD_NONE; idle.agc_ref = 0.8f; idle.agc_max = 1.f; idle.agc_thr = 0.8f;
     g->h_cfg.resize((size_t)ns, idle);
     g->cfg_stale[0] = g->cfg_stale[1] = true;
@@ -962,21 +1031,26 @@ int apply_pending(owrx_bank* bank, Group* g, cudaStream_t st_fir, cudaStream_t s
         }
         g->bp_pending = false;
     }
-    if (g->wfm) {
-        // multiplex tap layout of this block: F32 runs, then S16 runs, in slot order (ChanCfg::mpx / mpx_run)
-        g->mpx_runs.clear();
-        g->mpx_nf = g->mpx_ns = 0;
-        for (int s = 0; s < S; s++) {
-            const int cid = g->slot_chan[(size_t)s];
-            const Chan* ch = cid >= 0 ? bank->chans[(size_t)cid].get() : nullptr;
+    // tap layouts of this block (ChanCfg::mpx / mpx_run for the multiplex tap, h_atap for the audio tap)
+    g->mpx.clear(); g->atap.clear();
+    for (int s = 0; s < S; s++) {
+        const int cid = g->slot_chan[(size_t)s];
+        const Chan* ch = cid >= 0 ? bank->chans[(size_t)cid].get() : nullptr;
+        if (g->wfm) {
             const int fmt = ch ? ch->mpx_fmt : OWRX_MPX_OFF;
-            const int run = fmt == OWRX_MPX_F32 ? g->mpx_nf++ : (fmt == OWRX_MPX_S16 ? g->mpx_ns++ : 0);
+            const int run = g->mpx.add(cid, fmt, ch ? ch->gen : 0);
             ChanCfg& c = g->h_cfg[(size_t)s];
             if (c.mpx != fmt || c.mpx_run != run) {
                 c.mpx = fmt; c.mpx_run = run;
                 g->cfg_stale[0] = g->cfg_stale[1] = true;
             }
-            if (fmt != OWRX_MPX_OFF) g->mpx_runs.push_back(MpxRun{cid, fmt, run, ch->gen});
+        }
+        const int fmt = ch ? ch->atap_fmt : OWRX_MPX_OFF;
+        const int run = g->atap.add(cid, fmt, ch ? ch->gen : 0);
+        TapFmt& a = g->h_atap[(size_t)s];
+        if (a.fmt != fmt || a.run != run) {
+            a = TapFmt{fmt, run};
+            g->cfg_stale[0] = g->cfg_stale[1] = true;
         }
     }
     if (g->rs_pending) {
@@ -1010,12 +1084,13 @@ int apply_pending(owrx_bank* bank, Group* g, cudaStream_t st_fir, cudaStream_t s
     g->f3.hist = rs_hist;                            // kept by the next roll (K - 1 rows back from a pass's first output)
     // per-slot tables of this block's parity: a block still in flight on the other streams keeps reading the other copy
     g->d_cfg = g->d_cfg2[g->cur]; g->d_bp_en = g->d_bp_en2[g->cur]; g->d_tail_mode = g->d_tail_mode2[g->cur];
-    g->d_rs_cfg = g->d_rs_cfg2[g->cur];
+    g->d_rs_cfg = g->d_rs_cfg2[g->cur]; g->d_atap = g->d_atap2[g->cur];
     if (g->cfg_stale[g->cur]) {
         OWRX_CUDA(cudaMemcpyAsync(g->d_cfg, g->h_cfg.data(), (size_t)S * sizeof(ChanCfg), cudaMemcpyHostToDevice, st_tail));
         OWRX_CUDA(cudaMemcpyAsync(g->d_bp_en, g->h_bp_en.data(), (size_t)S * sizeof(int), cudaMemcpyHostToDevice, st_tail));
         OWRX_CUDA(cudaMemcpyAsync(g->d_tail_mode, g->h_tail_mode.data(), (size_t)S * sizeof(int), cudaMemcpyHostToDevice, st_tail));
         OWRX_CUDA(cudaMemcpyAsync(g->d_rs_cfg, g->h_rs.data(), (size_t)S * sizeof(RsCfg), cudaMemcpyHostToDevice, st_tail));
+        OWRX_CUDA(cudaMemcpyAsync(g->d_atap, g->h_atap.data(), (size_t)S * sizeof(TapFmt), cudaMemcpyHostToDevice, st_tail));
         g->cfg_stale[g->cur] = false;
     }
     g->any_tail = false;
@@ -1041,9 +1116,10 @@ int prof_mark(owrx_bank* bank, int tag, cudaStream_t st, bool begin)
         }
         bank->prof_tags[bank->prof_used] = tag;
         OWRX_CUDA(cudaEventRecord(bank->prof_events[bank->prof_used].first, st));
+        bank->prof_open.push_back(bank->prof_used++);
     } else {
-        OWRX_CUDA(cudaEventRecord(bank->prof_events[bank->prof_used].second, st));
-        bank->prof_used++;
+        OWRX_CUDA(cudaEventRecord(bank->prof_events[bank->prof_open.back()].second, st));
+        bank->prof_open.pop_back();
     }
     return OWRX_OK;
 }
@@ -1398,17 +1474,11 @@ int group_tail(owrx_bank* bank, Group* g, cudaStream_t st)
         const long long f1_first = g->f1.abs_end;
         g->f1.appended(n4);
         g->sq_abs += (long long)n4;
-        if (g->wfm && !g->mpx_runs.empty()) {
+        if (g->wfm && !g->mpx.runs.empty()) {
             // ---- multiplex tap: the tapped slots' new f1 rows -> their staging runs (on the stream that owns f1, before it rolls)
-            if (g->mpx_rows + n4 > g->mpx_cap) return fail(OWRX_E_STATE, "multiplex tap staging under-provisioned");
-            if (g->mpx_drained[g->cur]) OWRX_CUDA(cudaStreamWaitEvent(st, g->mpx_drained[g->cur], 0));
-            const long long r0 = (long long)g->mpx_rows;
-            const long long tiles = (r0 + (long long)n4 + MG_R - 1) / MG_R - r0 / MG_R;
-            mpx_gather_kernel<<<dim3((unsigned)(S / 32), (unsigned)std::min<long long>(tiles, 65535)), 256, 0, st>>>(
-                g->f1.row_abs(f1_first), S, (int)n4, g->d_cfg, r0, (long long)g->mpx_cap, g->mpx_nf, g->d_mpx[g->cur]);
-            OWRX_LAUNCH_CHECK();
-            bank->stats.kernel_launches++;
-            g->mpx_rows += n4;
+            if ((rc = prof_mark(bank, OWRX_PROF_TAP, st, true)) != OWRX_OK) return rc;
+            if ((rc = g->mpx.gather(bank->stats, g->f1.row_abs(f1_first), S, n4, MpxTapSel{g->d_cfg}, g->cur, st)) != OWRX_OK) return rc;
+            if ((rc = prof_mark(bank, OWRX_PROF_TAP, st, false)) != OWRX_OK) return rc;
         }
 
         size_t n_audio = 0;
@@ -1517,6 +1587,13 @@ int group_tail_serial(owrx_bank* bank, Group* g, cudaStream_t st)
             if ((rc = prof_mark(bank, OWRX_PROF_AGC, st, false)) != OWRX_OK) return rc;
             bank->stats.kernel_launches++;
             g->f3.appended(n_audio);
+            if (!g->atap.runs.empty()) {
+                // ---- audio tap: the tapped slots' new f3 rows -> their staging runs (on the stream that writes f3, before it rolls)
+                if ((rc = prof_mark(bank, OWRX_PROF_TAP, st, true)) != OWRX_OK) return rc;
+                if ((rc = g->atap.gather(bank->stats, g->f3.rows(g->f3.fill - n_audio), S, n_audio, AudioTapSel{g->d_atap}, g->cur, st)) != OWRX_OK)
+                    return rc;
+                if ((rc = prof_mark(bank, OWRX_PROF_TAP, st, false)) != OWRX_OK) return rc;
+            }
             if (g->any_tail) {
                 // ---- client audio tail: [AudioResampler + Limit] Convert(FLOAT, SHORT) [+ AdpcmEncoder(sync=True)]; appends
                 // behind earlier passes.  a0: absolute audio row of this pass's first row; the feed's rows start at audio_af.
@@ -1635,19 +1712,8 @@ int group_begin_feed(owrx_bank* bank, Group* g, size_t rows, cudaStream_t st_fir
         }
         OWRX_CUDA(cudaMemsetAsync(g->d_tail_count, 0, (size_t)S * sizeof(int), st_serial));
     }
-    g->mpx_rows = 0;
-    if (!g->mpx_runs.empty()) {
-        // the multiplex staging follows the tap layout apply_pending has just rebuilt; f1 appends at most `low` rows per feed
-        const size_t cap = std::max(g->mpx_cap, (low + 7) / 8 * 8);
-        const size_t bytes = cap * (4 * (size_t)g->mpx_nf + 2 * (size_t)g->mpx_ns);
-        if (cap != g->mpx_cap || bytes > g->mpx_bytes) {
-            OWRX_CUDA(cudaDeviceSynchronize());
-            for (int k = 0; k < 2; k++) { cudaFree(g->d_mpx[k]); g->d_mpx[k] = nullptr; }
-            g->mpx_cap = g->mpx_bytes = 0;
-            for (int k = 0; k < 2; k++) OWRX_CUDA(cudaMalloc((void**)&g->d_mpx[k], bytes));
-            g->mpx_cap = cap; g->mpx_bytes = bytes;
-        }
-    }
+    // the tap staging follows the layouts apply_pending has just rebuilt; f1 and f3 append at most `low` rows per feed
+    if ((rc = g->mpx.provision(low)) != OWRX_OK || (rc = g->atap.provision(low)) != OWRX_OK) return rc;
     return OWRX_OK;
 }
 
@@ -1707,13 +1773,16 @@ void drain_items(const owrx_bank* bank, Group* g, bool final, std::vector<DrainI
             it.to[(size_t)s].n = c.L ? std::min(it.n, (size_t)(rs_outputs(c, g->f3.abs_end) - rs_outputs(c, g->audio_af))) : g->last_audio;
         }
     }
-    if (g->mpx_rows && !g->mpx_runs.empty()) {
-        // packed as [F32 runs][S16 runs] of mpx_rows each; a run goes to the client it was gathered for, in its format
-        DrainItem& it = add(DRAIN_MPX, g->mpx_rows, g->mpx_rows * (4 * (size_t)g->mpx_nf + 2 * (size_t)g->mpx_ns));
-        it.cap = g->mpx_cap;
+    for (DrainKind kind : {DRAIN_MPX, DRAIN_ATAP}) {
+        TapStage& tap = kind == DRAIN_MPX ? g->mpx : g->atap;
+        if (!tap.rows || tap.runs.empty()) continue;
+        // packed as [F32 runs][S16 runs] of tap.rows each; a run goes to the client it was gathered for, in its format
+        DrainItem& it = add(kind, tap.rows, tap.rows * (4 * (size_t)tap.nf + 2 * (size_t)tap.ns));
+        it.tap = &tap;
+        it.cap = tap.cap;
         it.to.clear();
-        const size_t f32 = (size_t)g->mpx_nf * it.n * 4;
-        for (const MpxRun& r : g->mpx_runs)
+        const size_t f32 = (size_t)tap.nf * it.n * 4;
+        for (const TapRun& r : tap.runs)
             it.to.push_back(DrainTo{r.chan, r.gen, r.fmt, r.fmt == OWRX_MPX_F32 ? (size_t)r.run * it.n * 4 : f32 + (size_t)r.run * it.n * 2});
     }
 }
@@ -1750,15 +1819,12 @@ int drain_enqueue(owrx_bank* bank, std::vector<DrainItem>& items, DrainStage& st
             OWRX_CUDA(cudaMemcpyAsync(h + tail_bytes_at(it.n, S), g->d_tail_bytes, it.cap * S, cudaMemcpyDeviceToHost, st));
             OWRX_CUDA(cudaMemcpyAsync(h + tail_counts_at(it.n, S, it.cap), g->d_tail_count, S * sizeof(int), cudaMemcpyDeviceToHost, st));
         } else {
-            // the tap's runs, at most two copies
-            const size_t n = it.n, nf = (size_t)g->mpx_nf, ns = (size_t)g->mpx_ns;
-            const unsigned char* d = g->d_mpx[g->cur];
+            // a tap's runs, at most two copies
+            const size_t n = it.n, nf = (size_t)it.tap->nf, ns = (size_t)it.tap->ns;
+            const unsigned char* d = it.tap->d[g->cur];
             if (nf) OWRX_CUDA(cudaMemcpy2DAsync(h, n * 4, d, it.cap * 4, n * 4, nf, cudaMemcpyDeviceToHost, st));
             if (ns) OWRX_CUDA(cudaMemcpy2DAsync(h + nf * n * 4, n * 2, d + nf * it.cap * 4, it.cap * 2, n * 2, ns, cudaMemcpyDeviceToHost, st));
-            if (split) {
-                if (!g->mpx_drained[g->cur]) OWRX_CUDA(cudaEventCreateWithFlags(&g->mpx_drained[g->cur], cudaEventDisableTiming));
-                OWRX_CUDA(cudaEventRecord(g->mpx_drained[g->cur], st));
-            }
+            if (split && (rc = it.tap->mark_drained(g->cur, st)) != OWRX_OK) return rc;
         }
     }
     if (xp) OWRX_CUDA(cudaMemcpyAsync(stage.h, stage.d, xp, cudaMemcpyDeviceToHost, st));
@@ -1799,9 +1865,12 @@ void drain_deliver(owrx_bank* bank, const std::vector<DrainItem>& items, const u
                     ch->q_bytes.insert(ch->q_bytes.end(), hb, hb + reinterpret_cast<const int*>(h + tail_counts_at(it.n, it.slots, it.cap))[k]);
                 }
                 break;
-            case DRAIN_MPX:
-                if (ch->mpx_fmt == t.fmt) ch->q_mpx.insert(ch->q_mpx.end(), h + t.n, h + t.n + it.n * (t.fmt == OWRX_MPX_F32 ? 4 : 2));
+            case DRAIN_MPX: case DRAIN_ATAP: {
+                const bool mpx = it.kind == DRAIN_MPX;
+                std::vector<unsigned char>& q = mpx ? ch->q_mpx : ch->q_atap;
+                if ((mpx ? ch->mpx_fmt : ch->atap_fmt) == t.fmt) q.insert(q.end(), h + t.n, h + t.n + it.n * (t.fmt == OWRX_MPX_F32 ? 4 : 2));
                 break;
+            }
             }
         }
     }
@@ -2067,6 +2136,7 @@ int owrx_chan_set_demod(owrx_bank_t* bank, int chan, int kind, double audio_rate
     const bool wfm = kind == OWRX_DEMOD_WFM;
     if (wfm && !(audio_rate > 0.0 && tau > 0.0)) return fail(OWRX_E_INVALID, "WFM needs audio_rate and tau");
     if (!wfm) { ch->mpx_fmt = OWRX_MPX_OFF; ch->q_mpx.clear(); }          // the multiplex tap is a WFm chain's
+    if (kind == OWRX_DEMOD_NONE) { ch->atap_fmt = OWRX_MPX_OFF; ch->q_atap.clear(); }   // no demodulator: no audio to tap
     if (kind == OWRX_DEMOD_NONE && ch->rs_in) {                           // no audio: nothing to resample
         ch->rs_in = ch->rs_out = 0;
         ch->rs_dirty = true; g->rs_pending = true;
@@ -2214,18 +2284,50 @@ int owrx_chan_set_mpx(owrx_bank_t* bank, int chan, int format)
     return OWRX_OK;
 }
 
+// pops whole samples of a tap queue in format `fmt`
+static void pop_tap(std::vector<unsigned char>& q, int fmt, void* out, size_t cap_bytes, size_t* n_bytes)
+{
+    const size_t unit = fmt == OWRX_MPX_S16 ? 2 : 4;
+    size_t take = std::min(cap_bytes, q.size());
+    take -= take % unit;
+    memcpy(out, q.data(), take);
+    q.erase(q.begin(), q.begin() + (ptrdiff_t)take);
+    *n_bytes = take;
+}
+
 int owrx_chan_read_mpx(owrx_bank_t* bank, int chan, void* out, size_t cap_bytes, size_t* n_bytes)
 {
     if (!bank || !out || !n_bytes) return fail(OWRX_E_INVALID, "bad argument");
     std::lock_guard<std::mutex> lk(bank->mu);
     Chan* ch = get_chan(bank, chan);
     if (!ch) return fail(OWRX_E_INVALID, "no such channel %d", chan);
-    const size_t unit = ch->mpx_fmt == OWRX_MPX_S16 ? 2 : 4;
-    size_t take = std::min(cap_bytes, ch->q_mpx.size());
-    take -= take % unit;
-    memcpy(out, ch->q_mpx.data(), take);
-    ch->q_mpx.erase(ch->q_mpx.begin(), ch->q_mpx.begin() + (ptrdiff_t)take);
-    *n_bytes = take;
+    pop_tap(ch->q_mpx, ch->mpx_fmt, out, cap_bytes, n_bytes);
+    return OWRX_OK;
+}
+
+int owrx_chan_set_audio_tap(owrx_bank_t* bank, int chan, int format)
+{
+    if (!bank) return fail(OWRX_E_INVALID, "NULL bank");
+    if (format != OWRX_MPX_OFF && format != OWRX_MPX_F32 && format != OWRX_MPX_S16) return fail(OWRX_E_INVALID, "unknown audio tap format %d", format);
+    std::lock_guard<std::mutex> lk(bank->mu);
+    Chan* ch = get_chan(bank, chan);
+    if (!ch) return fail(OWRX_E_INVALID, "no such channel %d", chan);
+    if (format != OWRX_MPX_OFF && ch->cfg.kind == OWRX_DEMOD_NONE) return fail(OWRX_E_INVALID, "channel %d has no demodulator: it has no audio to tap", chan);
+    if (bank->pending_final) { cudaSetDevice(bank->device); int rcp = finish_pending(bank); if (rcp != OWRX_OK) return rcp; }
+    if (format != ch->atap_fmt) {
+        ch->q_atap.clear();
+        ch->atap_fmt = format;                       // the group's tap layout is rebuilt at the next block boundary
+    }
+    return OWRX_OK;
+}
+
+int owrx_chan_read_audio_tap(owrx_bank_t* bank, int chan, void* out, size_t cap_bytes, size_t* n_bytes)
+{
+    if (!bank || !out || !n_bytes) return fail(OWRX_E_INVALID, "bad argument");
+    std::lock_guard<std::mutex> lk(bank->mu);
+    Chan* ch = get_chan(bank, chan);
+    if (!ch) return fail(OWRX_E_INVALID, "no such channel %d", chan);
+    pop_tap(ch->q_atap, ch->atap_fmt, out, cap_bytes, n_bytes);
     return OWRX_OK;
 }
 
@@ -2564,7 +2666,7 @@ int owrx_bank_drain(owrx_bank_t* bank)
 // may issue the NEXT block before _end, which waits for the copies and hands the samples to the per-channel queues.  The stage
 // buffers are double-buffered, so the next block does not touch what is being drained; whichever later block writes such a
 // buffer again waits for the transpose that read it (StageBuf::drained), and the next gather into a tap region for its copy
-// (Group::mpx_drained).  S-meter power reports and client-audio bytes are read from scratch the next block overwrites: with
+// (TapStage::drained).  S-meter power reports and client-audio bytes are read from scratch the next block overwrites: with
 // either enabled, _begin completes the drain at once.
 int owrx_bank_drain_begin(owrx_bank_t* bank)
 {

@@ -220,7 +220,7 @@ struct ChanCfg {
     int agc_hang_time;
     int active;
     float agc_thr;      // largest float a with fl(a / agc_ref) <= 1: "err > 1" <=> abs(v)*gain > agc_thr, exactly
-    int mpx;            // WFM multiplex tap: OWRX_MPX_OFF / _F32 / _S16 (mpx_gather_kernel)
+    int mpx;            // WFM multiplex tap: OWRX_MPX_OFF / _F32 / _S16 (tap_gather_kernel)
     int mpx_run;        // index of this slot's run among the group's tapped slots of the same format
 };
 
@@ -1284,8 +1284,14 @@ audio_tail_kernel(const float* __restrict__ in, int slots, int n, const int* __r
 }
 
 // ------------------------------------------------------------------------------------------------
-// WFM multiplex tap (csdr/chain/analog.py:62,73-76): the WFm chain writes its Limit output into a tap buffer that the audio
-// path and the RDS path (Convert(FLOAT, SHORT) -> redsea) both read.  Here that signal is f1, channel-minor at the IF rate.
+// Per-channel taps: a second reader of a Buffer that the fused chain keeps on the device.  One gather kernel serves both:
+//  - the WFM multiplex tap (csdr/chain/analog.py:62,73-76): the WFm chain writes its Limit output into a tap buffer that the
+//    audio path and the RDS path (Convert(FLOAT, SHORT) -> redsea) both read.  Here that signal is f1, channel-minor at the IF
+//    rate; a slot's (format, run) is ChanCfg::mpx / mpx_run (MpxTapSel).
+//  - the demodulated-audio tap: the Buffer the last demodulator stage writes (Agc, or WfmDeemphasis for WFM), which a
+//    secondary demodulator (Convert(FLOAT, SHORT) -> a digital-mode decoder) reads beside the client-audio Converter.  Here
+//    that signal is f3 at the demodulator rate; a slot's (format, run) comes from a per-parity table beside ChanCfg
+//    (AudioTapSel), so that ChanCfg, which the Agc loads whole, keeps its layout.
 // The kernel copies the new rows of the tapped slots only, one contiguous run per channel in a staging region, so the D2H
 // moves just the tapped bytes (C5: 128 slots; copying all of f1 would be 512 B per IF sample):
 //   F32 runs first, run k at byte k * cap * 4;  then S16 runs, run k at byte n_f32 * cap * 4 + k * cap * 2
@@ -1296,14 +1302,28 @@ audio_tail_kernel(const float* __restrict__ in, int slots, int n, const int* __r
 // S16 is Convert(FLOAT, SHORT) exactly as the client audio tail does it (SURVEY A.12).
 // ------------------------------------------------------------------------------------------------
 constexpr int MG_R = 128;
+struct TapFmt {
+    int fmt;            // OWRX_MPX_OFF / _F32 / _S16
+    int run;            // index of this slot's run among the group's tapped slots of the same format
+};
+struct MpxTapSel {
+    const ChanCfg* __restrict__ cfg;
+    __device__ __forceinline__ TapFmt operator()(int s) const { return TapFmt{cfg[s].mpx, cfg[s].mpx_run}; }
+};
+struct AudioTapSel {
+    const TapFmt* __restrict__ tab;
+    __device__ __forceinline__ TapFmt operator()(int s) const { return tab[s]; }
+};
+
+template <typename Sel>
 __global__ void __launch_bounds__(256)
-mpx_gather_kernel(const float* __restrict__ in, int slots, int n, const ChanCfg* __restrict__ cfg, long long r0, long long cap,
-                  int n_f32, unsigned char* __restrict__ out)
+tap_gather_kernel(const float* __restrict__ in, int slots, int n, Sel sel, long long r0, long long cap, int n_f32,
+                  unsigned char* __restrict__ out)
 {
     __shared__ float tile[MG_R][33];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     const int s0 = blockIdx.x * 32, s = s0 + lane;
-    const unsigned tapped = __ballot_sync(0xffffffffu, s < slots && cfg[s].mpx != 0);
+    const unsigned tapped = __ballot_sync(0xffffffffu, s < slots && sel(s).fmt != OWRX_MPX_OFF);
     if (!tapped) return;                                         // the same ballot in every warp: the whole CTA leaves
     const long long t_first = r0 / MG_R, t_end = (r0 + n + MG_R - 1) / MG_R;
     for (long long t = t_first + blockIdx.y; t < t_end; t += gridDim.y) {
@@ -1315,10 +1335,10 @@ mpx_gather_kernel(const float* __restrict__ in, int slots, int n, const ChanCfg*
         __syncthreads();
         for (int l = w; l < 32; l += 8) {
             if (!((tapped >> l) & 1u)) continue;
-            const ChanCfg c = cfg[s0 + l];
-            if (c.mpx == OWRX_MPX_F32) {
+            const TapFmt c = sel(s0 + l);
+            if (c.fmt == OWRX_MPX_F32) {
                 const long long d = d0 + 4 * lane;
-                float* o = reinterpret_cast<float*>(out + (size_t)c.mpx_run * cap * 4) + d;
+                float* o = reinterpret_cast<float*>(out + (size_t)c.run * cap * 4) + d;
                 // rows 4*lane + k sit 4*lane banks apart: each group of 8 lanes starts at another k (rot), so the 32 lanes of a read
                 // hit 32 different banks; the selects put the values back in row order
                 const int rot = lane >> 3;
@@ -1339,7 +1359,7 @@ mpx_gather_kernel(const float* __restrict__ in, int slots, int n, const ChanCfg*
                 }
             } else if (lane < 16) {
                 const long long d = d0 + 8 * lane;
-                int16_t* o = reinterpret_cast<int16_t*>(out + (size_t)n_f32 * cap * 4 + (size_t)c.mpx_run * cap * 2) + d;
+                int16_t* o = reinterpret_cast<int16_t*>(out + (size_t)n_f32 * cap * 4 + (size_t)c.run * cap * 2) + d;
                 // the same bank rotation over 8 rows (lanes 0, 4, 8, 12 share banks without it); each converted sample goes straight
                 // to its 16-bit place in the two 64-bit halves of the 16-byte store
                 const int rot = 2 * (lane >> 2);

@@ -18,6 +18,7 @@ receives the result bytes, and the selector output is materialised only when som
 (e.g. the secondary FFT on ClientDemodulatorChain.selectorBuffer, owrx/dsp.py:49,220-225).
 """
 import ctypes as C
+import itertools
 import logging
 import math
 import os
@@ -104,6 +105,7 @@ class _Graph:
 
 
 _GRAPH = _Graph()
+_STAGE_SEQ = itertools.count()
 
 
 # ================================================================================================
@@ -372,6 +374,7 @@ class _Stage(Module):
         self._writer = None
         self._stopped = False
         self._lock = threading.Lock()
+        self._seq = next(_STAGE_SEQ)          # construction order: the walk's tie-break
         _GRAPH.modules.add(self)
 
     def getInputFormat(self):
@@ -934,6 +937,22 @@ for _n in ("Lowpass", "Downmix", "Throttle", "SnrSquelch", "SmartSquelch", "Timi
 # ================================================================================================
 # chain discovery and fused plans
 # ================================================================================================
+def _float_to_short(m):
+    return isinstance(m, Convert) and m.IN is Format.FLOAT and m.OUT is Format.SHORT
+
+
+def _walk_rank(m):
+    """preference of a reader as the stage that continues a chain (_walk)"""
+    if not isinstance(m, _Unfused):
+        return 3
+    if _float_to_short(m):
+        w = m._writer
+        if isinstance(w, Buffer) and isinstance(_GRAPH.consumer_of(w), AdpcmEncoder):
+            return 2
+        return 1
+    return 0
+
+
 def _walk(head):
     """the list of stages from `head` downstream through virtual Buffers, and the Buffers between them"""
     chain, links = [head], []
@@ -945,15 +964,15 @@ def _walk(head):
         # the stage that continues THIS chain: a Buffer can have further readers that start chains of their own (the secondary
         # FFT and the SecondarySelector on ClientDemodulatorChain.selectorBuffer, owrx/dsp.py:49,188-225) — those are heads
         # A fused stage goes before an unfused one: the WFm chain's tap buffer is read by the FractionalDecimator AND by the
-        # RDS path's Convert(FLOAT, SHORT) (csdr/chain/analog.py:62,73-76); the chain goes on through the former.
-        nxt = None
-        for m in list(_GRAPH.modules):
-            r = m._reader
-            if r is not None and r._buffer is w and not m._stopped and not r._stopped and not m.HEAD:
-                if nxt is None or (isinstance(nxt, _Unfused) and not isinstance(m, _Unfused)):
-                    nxt = m
-        if nxt is None:
+        # RDS path's Convert(FLOAT, SHORT) (csdr/chain/analog.py:62,73-76); the chain goes on through the former.  On the
+        # demodulator's audio Buffer a secondary demodulator's Convert(FLOAT, SHORT) sits beside the client-audio Converter: the
+        # chain goes on through the AudioResampler (fused), else a Convert(FLOAT, SHORT) feeding an AdpcmEncoder, else any
+        # Convert(FLOAT, SHORT); ties go to the older stage, so the choice never depends on the set's iteration order.
+        cands = [m for m in list(_GRAPH.modules)
+                 if m._reader is not None and m._reader._buffer is w and not m._stopped and not m._reader._stopped and not m.HEAD]
+        if not cands:
             break
+        nxt = min(cands, key=lambda m: (-_walk_rank(m), m._seq))
         links.append(w)
         chain.append(nxt)
         cur = nxt
@@ -1032,7 +1051,7 @@ class _WaterfallPlan:
 _DEMODS = ("nfm", "am", "ssb", "wfm", "none")
 
 
-_MPX_WARNED = set()      # ids of tap Buffers whose float reader has been reported as not served
+_TAP_WARNED = set()      # ids of tap Buffers whose float reader has been reported as not served
 
 
 class _ChannelPlan:
@@ -1043,26 +1062,27 @@ class _ChannelPlan:
         self.spec_key = None
 
     @staticmethod
-    def _mpx_tap(limit, frac):
-        """the WFm chain's multiplex tap (csdr/chain/analog.py:62,73-76): the Limit writes into a Buffer of its own that the
-        audio path's FractionalDecimator reads; any other reader of it is a tap consumer.  A Convert(FLOAT, SHORT) reader (the
-        RDS path) is fused: ("s16", the Convert's writer).  Any other reader gets the float samples in the tap Buffer itself:
-        ("f32", that Buffer).  With both kinds of reader only the Convert is served (logged once).  (None, None) without a
-        consumer."""
-        tap = limit._writer
+    def _tap(writer_stage, nxt, what):
+        """a tap of a Buffer inside a fused chain: `writer_stage` writes it, `nxt` (the chain's next stage) reads it, and any other
+        reader is a tap consumer.  The WFm chain's multiplex tap (csdr/chain/analog.py:62,73-76: the Limit's Buffer, read by the
+        audio path's FractionalDecimator and by the RDS path) and the demodulator's audio Buffer (read by the client-audio
+        Converter and by a secondary demodulator) follow the same rules.  A Convert(FLOAT, SHORT) reader is fused: ("s16", the
+        Convert's writer).  Any other reader gets the float samples in the Buffer itself: ("f32", that Buffer).  With both kinds
+        of reader only the Convert is served (logged once).  (None, None) without a consumer."""
+        tap = writer_stage._writer
         if not isinstance(tap, Buffer):
             return None, None
         for m in list(_GRAPH.modules):
             r = m._reader
-            if (m is not frac and isinstance(m, Convert) and r is not None and r._buffer is tap and not m._stopped and not r._stopped
-                    and m.IN is Format.FLOAT and m.OUT is Format.SHORT and isinstance(m._writer, Buffer)):
-                if tap._extra_readers(frac._reader) and id(tap) not in _MPX_WARNED:
-                    # one tap per channel: the bank delivers one format, and the int16 samples of the RDS path win
-                    _MPX_WARNED.add(id(tap))
-                    logger.warning("pycsdr-b200: the WFM tap buffer has a float reader beside Convert(FLOAT, SHORT); only the "
-                                   "Convert is served, the float reader receives nothing")
+            if (m is not nxt and _float_to_short(m) and r is not None and r._buffer is tap and not m._stopped and not r._stopped
+                    and isinstance(m._writer, Buffer)):
+                if tap._extra_readers(nxt._reader) and id(tap) not in _TAP_WARNED:
+                    # one tap per channel: the bank delivers one format, and the int16 samples of the Convert win
+                    _TAP_WARNED.add(id(tap))
+                    logger.warning("pycsdr-b200: the %s has a float reader beside Convert(FLOAT, SHORT); only the "
+                                   "Convert is served, the float reader receives nothing", what)
                 return "s16", m._writer
-        if tap._extra_readers(frac._reader):
+        if tap._extra_readers(nxt._reader):
             return "f32", tap
         return None, None
 
@@ -1105,7 +1125,7 @@ class _ChannelPlan:
             d["demod"], d["agc"], used = "ssb", rest[1], 2
         elif kinds[:4] == [FmDemod, Limit, FractionalDecimator, WfmDeemphasis] and rest[2].format is Format.FLOAT:
             d["demod"], d["wfm_frac"], d["wfm_de"], used = "wfm", rest[2], rest[3], 4
-            d["mpx"], d["mpx_writer"] = _ChannelPlan._mpx_tap(rest[1], rest[2])
+            d["mpx"], d["mpx_writer"] = _ChannelPlan._tap(rest[1], rest[2], "WFM tap buffer")
         elif not rest:
             d["demod"], used = "none", 0
         else:
@@ -1115,6 +1135,11 @@ class _ChannelPlan:
         after = rest[used:]
         d["audio_fmt"] = "f32"
         d["resampler"] = None
+        # a second reader of the demodulator's audio Buffer (a secondary demodulator: Convert(FLOAT, SHORT) -> decoder) is
+        # served by the audio tap when the chain goes on past that Buffer; with float client audio the Buffer is materialised
+        d["atap"], d["atap_writer"] = None, None
+        if after and d["demod"] != "none":
+            d["atap"], d["atap_writer"] = _ChannelPlan._tap(rest[used - 1], after[0], "demodulator's audio buffer")
         if after and d["demod"] != "none" and isinstance(after[0], AudioResampler):
             rs = after[0]
             if len(after) < 3 or not isinstance(after[1], Limit) or not _resampler_ok(rs.inputRate, rs.outputRate):
@@ -1290,6 +1315,12 @@ class _SourceRunner(threading.Thread):
             N.check(N.lib.owrx_chan_set_mpx(self.bank, cid, {None: N.MPX_OFF, "f32": N.MPX_F32, "s16": N.MPX_S16}[mpx]))
             st["mpx"] = mpx
         st["mpx_writer"] = d.get("mpx_writer")
+        # so does the audio tap: no rebuild when a secondary demodulator comes or goes
+        atap = d.get("atap")
+        if st.get("atap") != atap:
+            N.check(N.lib.owrx_chan_set_audio_tap(self.bank, cid, {None: N.MPX_OFF, "f32": N.MPX_F32, "s16": N.MPX_S16}[atap]))
+            st["atap"] = atap
+        st["atap_writer"] = d.get("atap_writer")
         st["demod"] = d["demod"]
         st["tail_writer"] = d["tail"]._writer
         st["power_writer"] = sq.powerWriter if sq is not None else None
@@ -1407,6 +1438,10 @@ class _SourceRunner(threading.Thread):
                     bm = self._drain_bytes(N, cid, N.lib.owrx_chan_read_mpx)
                     if bm:
                         st["mpx_writer"].write(bm)
+                if st.get("atap_writer") is not None:
+                    ba = self._drain_bytes(N, cid, N.lib.owrx_chan_read_audio_tap)
+                    if ba:
+                        st["atap_writer"].write(ba)
             if st.get("power_writer") is not None:
                 bp = self._drain(N, N.lib.owrx_chan_read_power, cid, 1)
                 if bp:
