@@ -313,6 +313,48 @@ def agc(x, profile=0, initial_gain=1.0, max_gain=65535.0):
     return y
 
 
+class AgcStream:
+    """The Agc as a stream: process() carries gain and hang counter from call to call, and the setters change a live
+    instance the way the channel bank's control calls do (Agc.setProfile / setInitialGain / setMaxGain on the running
+    module).  A new demodulator means a new Agc: build a fresh instance with that kind's defaults."""
+
+    def __init__(self, profile=0, initial_gain=1.0, max_gain=65535.0):
+        self._a = Agc()
+        lib().oc_agc_init(C.byref(self._a), int(profile), float(initial_gain), float(max_gain))
+
+    def set_profile(self, profile):
+        """decay and hang time of the profile; gain and hang counter run on"""
+        fresh = Agc()
+        lib().oc_agc_init(C.byref(fresh), int(profile), 1.0, 1.0)
+        self._a.decay, self._a.hang_time = fresh.decay, fresh.hang_time
+
+    def set_initial_gain(self, gain):
+        if gain > 0:
+            self._a.gain = gain
+
+    def set_max_gain(self, gain):
+        if gain > 0:
+            self._a.max_gain = gain
+
+    @property
+    def gain(self):
+        return self._a.gain
+
+    @property
+    def hang(self):
+        return self._a.hang_counter
+
+    @property
+    def max_gain(self):
+        return self._a.max_gain
+
+    def process(self, x):
+        x = np.ascontiguousarray(x, np.float32)
+        y = np.empty_like(x)
+        lib().oc_agc_process(C.byref(self._a), _p(x), len(x), _p(y))
+        return y
+
+
 def convert_raw_iq(raw, fmt, gain=1.0):
     """source-side Convert (+ Gain): raw int16 ("cs16") / uint8 ("cu8") interleaved I, Q -> complex64"""
     raw = np.ascontiguousarray(raw, np.int16 if fmt == "cs16" else np.uint8)
